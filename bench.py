@@ -9,7 +9,7 @@ one batch of sites: per-edge expm, upward pass (partials stored), downward
 pass + per-edge weights, Frechet contraction, (N > 1) one NCCL allreduce of
 [1 + S + S*S] doubles.  Metric: site.edge messages / s = n_sites * n_edges / t.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 `value`   : inputs resident in HBM, CUDA-event time, max over ranks.
 `e2e`     : same step through the public API with HOST buffers: H2D of the leaf
@@ -21,6 +21,8 @@ pass + per-edge weights, Frechet contraction, (N > 1) one NCCL allreduce of
             likelihood + blocked Gibbs sampler + summary) and 61-state Rao-Teh figures.
 `--impl reference`: the oracle port of the reference's CPU path (numpy/scipy,
             one process per host core) on a bounded sample of the same workload.
+`--dump-outputs DIR`: what the step behind `value` returned in its last timed step,
+            as DIR/<name>.npy (rank 0), so that two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -44,6 +46,10 @@ E2E_PACKED = os.environ.get('RT_E2E_PACKED', '1') != '0'         # 4-bit leaf co
 USE_GRAPH = os.environ.get('RT_STEP_GRAPH', '1') != '0'       # device-resident arm: replay the step as one CUDA graph
 DEV_CHUNKS = int(os.environ.get('RT_DEV_CHUNKS', '0'))     # device-resident arm: two-stream chunk overlap   # site chunks of the pipelined host-buffer call
 C2_LEAVES = 32
+# what a caller of the C2 step receives: per-site log-likelihoods and status, the site-summed
+# statistics, the per-edge weights and contractions, and the packed (allreduced) vector
+# [loglik sum, dwell, trans, root posterior sum]
+DUMP_KEYS = ('loglik', 'status', 'dwell', 'trans', 'root_post_sum', 'W', 'M_edges', 'stats')
 
 
 # ----------------------------------------------------------------------------
@@ -144,6 +150,17 @@ def c2_workload(rank, n_sites=C2_SITES):
     from raoteh_b200 import synth
     return synth.config_c2(n_sites=n_sites, seed=20260201 + 1000 * rank, n_leaves=C2_LEAVES) \
         if rank else synth.config_c2(n_sites=n_sites, n_leaves=C2_LEAVES)
+
+
+def step_outputs(r, stats):
+    """Host copies of the step's outputs (float64; the int8 site status as float32), about
+    12 MB for the 1e6 C2 sites."""
+    r = dict(r, stats=stats)
+    out = {}
+    for k in DUMP_KEYS:
+        a = r[k].detach().cpu().numpy()
+        out[k] = a if a.dtype == np.float64 else a.astype(np.float32)
+    return out
 
 
 def c2_bytes_per_site(sched, S):
@@ -376,6 +393,7 @@ def run_gpu(args):
             stats = rdist.pack_stats(ll_sum, r['dwell'], r['trans'], r['root_post_sum'])
         rdist.allreduce_stats(stats)      # the path's only collective (NCCL, 1+S+S*S+S doubles)
         state['n_levels'] = r['n_levels']
+        state['last'] = r, stats
         return r, stats
     sub = {}
 
@@ -424,6 +442,10 @@ def run_gpu(args):
         sampler.start()
     ms_plain = timed(step, args.steps, args.warmup, record=True)   # per-kernel events (roofline)
     ms = timed(step, args.steps, args.warmup) if (DEV_CHUNKS > 1 or USE_GRAPH) else ms_plain
+    if args.dump_outputs and rank == 0:
+        # copied now: the legs below reuse the engine's workspaces
+        for name, a in step_outputs(*state['last']).items():
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
     clocks = sampler.stop() if rank == 0 else None
     ms_e2e = timed(step_e2e, args.steps, args.warmup)
     ms_e2e_u8 = timed(lambda: step_e2e(False), args.steps, args.warmup) if E2E_PACKED else ms_e2e
@@ -613,7 +635,7 @@ def bench_c2_loglik(dev, cfg, sched, obs, args, peaks):
         for _ in range(3):
             mjp.log_likelihood(o, out=(ll, st))
         ts = []
-        for _ in range(max(5, args.steps)):
+        for _ in range(args.steps):
             flush.fill_(1)
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
@@ -667,7 +689,7 @@ def bench_c3(dev, args):
         mjp.log_likelihood(obs, out=(ll, st))
     torch.cuda.synchronize()
     ts = []
-    for _ in range(max(5, args.steps)):
+    for _ in range(args.steps):
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
         mjp.log_likelihood(obs, out=(ll, st))
@@ -771,7 +793,15 @@ def main():
     ap.add_argument('--c4-sweeps', type=int, default=100)
     ap.add_argument('--c5-sites', type=int, default=1_000_000)
     ap.add_argument('--no-cpu', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the arrays the timed C2 step returned in its last timed step as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs:
+        if args.impl != 'b200':
+            ap.error('--dump-outputs needs --impl b200')
+        os.makedirs(args.dump_outputs, exist_ok=True)
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
     if args.impl == 'reference':
         return run_reference(args)

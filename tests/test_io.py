@@ -6,6 +6,7 @@ import os
 import numpy as np
 import pytest
 
+from helpers import GOLDEN
 from raoteh_b200 import io as rio
 from raoteh_b200.lowering import TreeSchedule
 
@@ -69,7 +70,8 @@ def test_read_disease_data_and_tolerance_observations():
 
 @pytest.mark.reference
 def test_reference_p53_inputs_parse():
-    base = '/root/reference/examples/p53'
+    from oracle import ref_shim
+    base = os.path.join(ref_shim.REFERENCE_ROOT, 'examples', 'p53')
     with open(os.path.join(base, 'p53S.const.tree')) as f:
         T, root, leaves = rio.read_newick(f)
     assert len(T) == 49 and len(leaves) == 25 and leaves[0][1] == 'Has'
@@ -86,14 +88,12 @@ def test_reference_p53_inputs_parse():
     assert (codes[0] != 255).all()                # the human sequence has no gaps or stops
 
 
-@pytest.mark.reference
 def test_mg94_matches_reference_recipe():
-    import sys
-    from oracle import ref_shim
-    ref_shim.load_reference()
-    base = '/root/reference/examples/p53'
-    with open(os.path.join(base, 'universal.code.txt')) as f:
+    # the standard genetic code as an index / residue / codon table like the reference's
+    # examples/p53/universal.code.txt, residues in alphabetical order, the stop codons last
+    with open(os.path.join(GOLDEN, 'universal.code.txt')) as f:
         code = rio.read_genetic_code(f)
+    assert len(code) == 61
     Q, distn, s2r, r2p = rio.mg94_from_genetic_code(0.25039, 0.30126, 0.25952, 0.18883, 3.17632,
                                                     0.21925, code, target_expected_rate=1.0)
     np.testing.assert_allclose(Q.sum(axis=1), 0, atol=1e-12)
