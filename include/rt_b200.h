@@ -205,27 +205,6 @@ int rt_copy2d_async(void* dst, size_t dst_pitch, const void* src, size_t src_pit
                     size_t width_bytes, size_t height, int to_device, void* stream);
 
 /*
- * FUSED evaluation for S <= 4: upward pruning, root combine, downward pass and per-edge
- * statistics in ONE persistent kernel -- the batched form of the whole per-site chain of
- * _mjp_dense.get_expected_history_statistics (raoteh/sampler/_mjp_dense.py:410-539:
- * pyfelscore.mcy_esd_get_node_to_pmap _mcy_dense.py:286-291, _mc0_dense.get_likelihood
- * _mc0_dense.py:147-212, mc0_esd_get_node_to_distn _mc0_dense.py:381, mc0_esd_get_joint_endpoint_distn
- * _mcy_dense.py:205, accumulation :502-533) when the caller wants neither the stored partials nor
- * the node marginals.  Same arguments as rt_prune_loglik + rt_posterior_stats; the partials of a
- * site tile live in a per-CTA scratch (private workspace pool) that stays L2 resident, so HBM sees
- * the observations in and loglik / status out.  n_store = number of internal nodes.
- * Outputs: loglik[n_sites], status[n_sites]; += loglik_sum[1] (nullable), W[n_nodes][S][S],
- * root_post_sum[S] (nullable).  ctas_per_sm: 0 = as many as fit.
- * *handled = 0 (and RT_OK) when the shape is not covered (S > 4, or a program whose tables exceed
- * the shared-memory budget): the caller then runs rt_prune_loglik + rt_posterior_stats.
- */
-int rt_posterior_fused(int S, int n_nodes, int n_store, int64_t n_sites, int64_t site_stride,
-                       const int32_t* program, int n_ops, int n_slots, const double* P,
-                       const double* root_distn, int obs_kind, const void* obs, double* loglik,
-                       int8_t* status, double* loglik_sum, double* W, double* root_post_sum,
-                       int ctas_per_sm, int* handled, void* stream);
-
-/*
  * Materialised per-edge joints and all-node marginals for small batches
  * (n_sites <= 65535):  J[b][site][a][c] = D[parent(b)][a] * norm(P_b[a,:] L_b)[c],
  * D_all[b][site][c] = sum_a J[b][site][a][c].  edges: all rows of the downward
@@ -247,7 +226,9 @@ int rt_joint_distn(int S, int n_nodes, int64_t n_sites, int64_t site_stride,
  * (trajectory t = chain * n_sites + site; observations are per site:
  * site = (traj0 + t) % n_sites), n_sweeps sweeps per call, Philox4x32-10
  * keyed by (seed; traj0 + t, sweep0 + i) so results do not depend on how
- * trajectories are split over launches or GPUs.  S in {2,3,4,5,6,8}.
+ * trajectories are split over launches or GPUs.  2 <= S <= 64: S in {2,3,4,5,6,8}
+ * runs one thread per trajectory; S = 7 and 9 <= S <= 64 run the warp-per-trajectory
+ * kernel below, which has neither option of rt_raoteh_run (time_f64, sweep_count).
  *
  * Trajectory state (caller-owned device arrays, trajectory-minor):
  *   node_state uint8 [n_nodes][traj_stride]  state at every tree node
@@ -324,7 +305,7 @@ int rt_raoteh_run(const rt_raoteh_args* args, void* stream);
 /*
  * Warp-cooperative Rao-Teh kernels: one warp per (chain, site) trajectory.
  *
- * (1) Rao-Teh sweeps for 9 <= S <= 64 primary states (rt_raoteh_sweeps dispatches
+ * (1) Rao-Teh sweeps for S = 7 and 9 <= S <= 64 primary states (rt_raoteh_sweeps dispatches
  *     here; n_parts = 0): lanes own the states of the FFBS messages.
  * (2) The blocked Gibbs sampler of the compound TOLERANCE process
  *     (raoteh/sampler/_sample_tmjp_dense.py:40-171 gen_histories_v1,

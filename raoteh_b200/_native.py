@@ -43,9 +43,6 @@ EXPORTS = {
                                    c_void_p, c_void_p, c_int, c_void_p,
                                    c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                    c_void_p, c_void_p, c_void_p, c_void_p], c_int),
-    'rt_posterior_fused': ([c_int, c_int, c_int, c_int64, c_int64, c_void_p, c_int, c_int, c_void_p,
-                            c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
-                            c_int, ctypes.POINTER(c_int), c_void_p], c_int),
     'rt_copy2d_async': ([c_void_p, ctypes.c_size_t, c_void_p, ctypes.c_size_t, ctypes.c_size_t,
                          ctypes.c_size_t, c_int, c_void_p], c_int),
     'rt_raoteh_sweeps': ([c_int, c_int, c_int64, c_int64, c_int64, c_int64, c_void_p, c_int, c_int,

@@ -3,7 +3,6 @@
 #include "../../include/rt_b200.h"
 #include <stdio.h>
 #include <string.h>
-#include <stdlib.h>
 
 static thread_local char g_err[512] = "";
 
@@ -85,15 +84,12 @@ int rt_posterior_dmma_dispatch(int, int, int64_t, int64_t, const int32_t*, const
                                cudaStream_t);
 
 int rt_raoteh_dispatch(const rt_raoteh_args&, cudaStream_t);
-int rt_fused_small_dispatch(int, int, int64_t, int64_t, const int32_t*, int, int, int, int, const double*,
-                            const double*, const void*, double*, int8_t*, double*, double*, double*,
-                            int, cudaStream_t, bool*);
 
 int rt_tmjp_dispatch(const rt_tmjp_args&, cudaStream_t);
 
 extern "C" {
 
-int rt_version(void) { return 200; }
+int rt_version(void) { return 201; }
 
 int rt_release_workspace(void) {
   int dev = 0;
@@ -251,25 +247,6 @@ int rt_posterior_branch_stats(int S, int n_nodes, int64_t n_sites, int64_t site_
                           node_distn, W, root_post_sum, K, branch_out, stream);
 }
 
-int rt_posterior_fused(int S, int n_nodes, int n_store, int64_t n_sites, int64_t site_stride,
-                       const int32_t* program, int n_ops, int n_slots, const double* P,
-                       const double* root_distn, int obs_kind, const void* obs, double* loglik,
-                       int8_t* status, double* loglik_sum, double* W, double* root_post_sum,
-                       int ctas_per_sm, int* handled, void* stream) {
-  if (!program || !P || !loglik || !status || !W || !handled) return arg_error("null pointer");
-  if (obs_kind < 0 || obs_kind > 3) return arg_error("obs_kind");
-  if (site_stride < n_sites) return arg_error("site_stride < n_sites");
-  *handled = 0;
-  if (n_ops <= 0 || n_slots <= 0 || n_nodes <= 1 || n_store <= 0) return arg_error("empty program");
-  if (n_sites <= 0) { *handled = 1; return RT_OK; }
-  bool h = false;
-  int rc = rt_fused_small_dispatch(S, obs_kind, n_sites, site_stride, program, n_ops, n_slots, n_nodes,
-                                   n_store, P, root_distn, obs, loglik, status, loglik_sum, W,
-                                   root_post_sum, ctas_per_sm, (cudaStream_t)stream, &h);
-  *handled = h ? 1 : 0;
-  return rc;
-}
-
 int rt_copy2d_async(void* dst, size_t dst_pitch, const void* src, size_t src_pitch,
                     size_t width_bytes, size_t height, int to_device, void* stream) {
   if (!dst || !src) return arg_error("null pointer");
@@ -289,12 +266,9 @@ static int raoteh_run_impl(const rt_raoteh_args& R, void* stream) {
   if (R.traj_stride < R.n_traj || R.n_sites <= 0 || R.cap <= 0) return arg_error("sizes");
   if (R.n_traj <= 0) return RT_OK;
   const int S = R.S;
-  // RT_RAOTEH_FORCE_WARP=1: run the warp-per-trajectory kernel for small state spaces too (the
-  // measurement that justifies thread-per-trajectory for S <= 8: profiles/r2_raoteh_warp_vs_thread.md)
-  static const bool force_warp = [] { const char* e = getenv("RT_RAOTEH_FORCE_WARP"); return e && e[0] == '1'; }();
-  if (((S > 8 || S == 7) || (force_warp && !R.time_f64)) && S <= 64) {
+  if (S == 7 || (S >= 9 && S <= 64)) {
     if (R.time_f64) return unsupported("fp64 event times: S in {2,3,4,5,6,8} only");
-    if (R.sweep_count && !force_warp) return unsupported("sweep_count: S in {2,3,4,5,6,8} only");
+    if (R.sweep_count) return unsupported("sweep_count: S in {2,3,4,5,6,8} only");
     // warp-per-trajectory kernel (csrc/rt_tmjp.cu) on the same trajectory layout
     rt_tmjp_args A;
     memset(&A, 0, sizeof(A));

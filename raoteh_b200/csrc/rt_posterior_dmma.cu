@@ -420,6 +420,7 @@ constexpr int kLeafThreads = 64;
 constexpr int kLeafLd = 67;            // odd: lanes (rows) hit distinct banks for one column; 64 = bin, 65 = unobserved
 constexpr int kLeafGroup = 16;
 constexpr int kLeafSitesPerCta = 2048;
+static_assert(kLeafSitesPerCta % 16 == 0, "K16 needs every CTA's first code byte 16-byte aligned");
 
 template <bool V4, bool K16>
 __global__ void __launch_bounds__(kLeafThreads, 6)
@@ -553,11 +554,6 @@ down_leaf_scatter_kernel(int S, int64_t n_sites, int64_t stride, const int4* __r
   }
 }
 
-static bool leaf_scatter_enabled() {
-  static const bool on = [] { const char* e = getenv("RT_DOWN_LEAF_SCATTER"); return !e || atoi(e) != 0; }();
-  return on;
-}
-
 template <int MT>
 int run(int S, int obs_kind, int64_t n_sites, int64_t stride, const int32_t* edges_dev,
         const int32_t* level_ptr_h, int n_levels, const double* P, const double* root_distn,
@@ -572,7 +568,7 @@ int run(int S, int obs_kind, int64_t n_sites, int64_t stride, const int32_t* edg
   const size_t smem = sizeof(double) * ((size_t)SP * LDP + 2 * (size_t)kWarps * SP * kLd + 2 * SP);
   const int4* edges = reinterpret_cast<const int4*>(edges_dev);
   const unsigned gx = (unsigned)((n_sites + kTilesPerCta * kTileSites - 1) / (kTilesPerCta * kTileSites));
-  const bool scatter = obs_kind == OBS_CODES && !branch_out && leaf_scatter_enabled();
+  const bool scatter = obs_kind == OBS_CODES && !branch_out;
 #define RT_LAUNCH(OBSK)                                                                           \
   if (branch_out) {                                                                               \
     auto kern = down_dmma_kernel<MT, OBSK, true>;                                                 \
@@ -600,14 +596,10 @@ int run(int S, int obs_kind, int64_t n_sites, int64_t stride, const int32_t* edg
   if (scatter && level_ptr_h[n_levels] > 0) {
     // every coded leaf edge of the tree in one launch: its parent's marginal is final by now
     const size_t lsm = sizeof(double) * 64 * kLeafLd;
-    static const int spc = [] {
-      const char* e = getenv("RT_LEAF_SITES");
-      const int v = e ? atoi(e) : kLeafSitesPerCta;
-      return v >= kLeafGroup ? v / kLeafGroup * kLeafGroup : kLeafSitesPerCta;
-    }();
+    const int spc = kLeafSitesPerCta;
     dim3 grid((unsigned)((n_sites + spc - 1) / spc), (unsigned)level_ptr_h[n_levels]);
     const bool v4 = stride % 4 == 0 && (reinterpret_cast<uintptr_t>(node_distn) & 31) == 0;
-    const bool k16 = v4 && stride % 16 == 0 && (reinterpret_cast<uintptr_t>(obs) & 15) == 0 && spc % 16 == 0;
+    const bool k16 = v4 && stride % 16 == 0 && (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
     const uint8_t* codes = reinterpret_cast<const uint8_t*>(obs);
     if (k16)
       down_leaf_scatter_kernel<true, true><<<grid, kLeafThreads, lsm, stream>>>(

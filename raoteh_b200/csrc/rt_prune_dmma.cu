@@ -15,11 +15,12 @@
 // mbarrier "full"); a warp that is done with a buffer bumps the buffer's counter and the LAST
 // of the warps to do so re-arms the barrier and issues the copy of the edge three ahead, so
 // nobody ever blocks as a producer and warps may drift up to two edges apart.
-// The FP64 tensor pipe belongs to an SM sub-partition, which hosts warps w, w + 4, ...: they can
-// take turns for their contraction loops (a shared-memory token per sub-partition), so that one
-// warp's bookkeeping (product over children, mask, exact power-of-two rescale, stores, leaf
-// gathers) runs under another warp's DMMAs.  (Round 1 ran two 4-warp CTAs per SM in lockstep,
-// with a block barrier per edge and a one-time nanosleep offset between the CTAs.)
+// The FP64 tensor pipe belongs to an SM sub-partition, which hosts four of the 16 warps; they
+// run free, so one warp's bookkeeping (product over children, mask, exact power-of-two rescale,
+// stores, leaf gathers) runs under another warp's DMMAs.  (Round 1 ran two 4-warp CTAs per SM in
+// lockstep, with a block barrier per edge and a one-time nanosleep offset between the CTAs;
+// making the warps of a sub-partition take turns on the pipe was measured slower,
+// profiles/r2_prune_dmma_variants.md.)
 // The product over children, the observation mask, the rescale and the root combine run on the C
 // fragments in registers; a finished partial goes to the warp's private shared tile (the next B
 // operand) and, coalesced, to HBM.  A leaf message with a hard code is one column of P_c per
@@ -28,21 +29,26 @@
 // P_c is stored XOR-swizzled (column ^ 4*(row&3)) so fragment loads are bank-conflict
 // free without padding.
 #include "rt_common.cuh"
-#include <stdlib.h>
 
 namespace {
 
-// NT n-tiles (8 sites each) per warp.  2: 8 warps x 16 sites, ~250 registers, two warps per SM
-// sub-partition.  1: 16 warps x 8 sites, <= 128 registers, four warps per sub-partition (more warps
-// to cover the latency-bound bookkeeping between the DMMA phases, at 1.125 instead of 0.625
-// shared-memory fragment loads per DMMA).  RT_PRUNE_DMMA_NT selects at run time.
+// One n-tile (8 sites) per warp: 16 warps x 8 sites, <= 128 registers, four warps per SM
+// sub-partition to cover the latency-bound bookkeeping between the DMMA phases, at 1.125 shared-
+// memory fragment loads per DMMA.  (8 warps x 16 sites, ~250 registers, 0.625 loads per DMMA was
+// measured slower at C3 size, profiles/r2_prune_dmma_variants.md.)
+constexpr int kNT = 1;                        // n-tiles per warp
+constexpr int kWarps = 16;
+constexpr int kThreads = 32 * kWarps;
+constexpr int kWarpSites = 8 * kNT;
+constexpr int kLdB = kWarpSites + 4;          // B tile row stride (== 4 mod 8 -> conflict-free)
+constexpr int kFillRows = 32 / kWarpSites;    // rows of the B tile one warp fills per step
 #ifndef RT_PD_PROFILE
 #define RT_PD_PROFILE 0
 #endif
 #if RT_PD_PROFILE
 // per-phase cycle counters of the pruning kernel (debug builds only: -DRT_PD_PROFILE=1), summed
-// over warps: 0 tile loop, 1 leaf gathers, 2 B-tile fills, 3 wait for P_c, 4 wait for the pipe
-// token, 5 DMMA loop, 6 release + product, 7 store / root, 8 code staging, 9 other ops
+// over warps: 0 tile loop, 1 leaf gathers, 2 B-tile fills, 3 wait for P_c, 4 unused, 5 DMMA
+// loop, 6 release + product, 7 store / root, 8 code staging, 9 other ops
 __device__ unsigned long long g_pd_prof[16];
 #define RT_PROF_DECL long long prof_t0 = 0, prof_acc[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
 #define RT_PROF_BEGIN prof_t0 = clock64();
@@ -52,7 +58,7 @@ __device__ unsigned long long g_pd_prof[16];
 #define RT_PROF_BEGIN
 #define RT_PROF_END(k)
 #endif
-constexpr int kTileSites = 128;        // sites per CTA tile = (16 / NT) warps x 8 NT sites
+constexpr int kTileSites = kWarps * kWarpSites;   // sites per CTA tile
 constexpr int kMaxSlots = 32;
 #ifndef RT_PD_RING
 #define RT_PD_RING 3
@@ -64,9 +70,6 @@ constexpr int kMaxSlots = 32;
 // for the leaf-edge column gathers -- no gain, profiles/r2_prune_dmma_variants.md.)
 constexpr int kRing = RT_PD_RING;          // P_c buffers
 constexpr int kMaxCodeBytes = RT_PD_CODE_KB * 1024;   // shared-memory budget of the staged leaf codes (0: L1)
-// defaults chosen by measurement on B200 at C3 size (profiles/r2_prune_dmma_variants.md)
-constexpr int kDefaultNT = 1;
-constexpr int kDefaultPingpong = 0;
 
 __device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
   asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
@@ -121,8 +124,8 @@ __global__ void pack_kernel(const double* __restrict__ P, int S, int SP, int n_n
 }
 
 // MT = number of 8-row m-tiles (padded states SP = 8*MT)
-template <int MT, int OBS, bool STORE, int NT>
-__global__ void __launch_bounds__(32 * (16 / NT), 1)
+template <int MT, int OBS, bool STORE>
+__global__ void __launch_bounds__(kThreads, 1)
 prune_dmma_kernel(int S, int64_t n_sites, int64_t stride, const int4* __restrict__ program,
                   int n_ops, int n_slots, const double* __restrict__ Ppad,
                   const double* __restrict__ PT, const double* __restrict__ rowsum,
@@ -130,17 +133,10 @@ prune_dmma_kernel(int S, int64_t n_sites, int64_t stride, const int4* __restrict
                   double* __restrict__ slots_ws, double* __restrict__ partials,
                   int32_t* __restrict__ exponents, double* __restrict__ loglik,
                   int8_t* __restrict__ status, double* __restrict__ loglik_sum,
-                  int code_capacity, int pingpong) {
+                  int code_capacity) {
   constexpr int SP = 8 * MT;
   constexpr int LDP = SP;       // swizzled, no padding
   constexpr int KS = SP / 4;   // k-steps
-  constexpr int kNT = NT;
-  constexpr int kWarps = 16 / NT;
-  constexpr int kThreads = 32 * kWarps;
-  constexpr int kWarpSites = 8 * NT;
-  constexpr int kLdB = kWarpSites + 4;       // B tile row stride (== 4 mod 8 -> conflict-free)
-  constexpr int kFillRows = 32 / kWarpSites; // rows of the B tile one warp fills per step
-  constexpr int kTurns = kWarps / 4;         // warps per SM sub-partition
   extern __shared__ __align__(128) unsigned char smem_raw[];
   double* Pring = reinterpret_cast<double*>(smem_raw);            // [kRing][SP][LDP]
   double* Ball = Pring + (size_t)kRing * SP * LDP;                // [kWarps][SP][kLdB]
@@ -151,7 +147,6 @@ prune_dmma_kernel(int S, int64_t n_sites, int64_t stride, const int4* __restrict
   uint8_t* codes_s = reinterpret_cast<uint8_t*>(stg_s + ((n_ops + 3) & ~3));   // [kWarps][n_code_rows][kWarpSites]
   __shared__ __align__(8) uint64_t full_bar[kRing];
   __shared__ int done_cnt[kRing];
-  __shared__ volatile int turn_s[4];
   __shared__ int counts_s[3];      // staged edges per tile, observation rows to stage, observation rows
 
   const int tid = threadIdx.x;
@@ -159,7 +154,6 @@ prune_dmma_kernel(int S, int64_t n_sites, int64_t stride, const int4* __restrict
   const int g = lane >> 2, t = lane & 3;
   double* Bw = Ball + (size_t)warp * SP * kLdB;
   int* estk_w = estk + warp * n_slots * kWarpSites;
-  const int pair = warp & 3, my_turn = warp >> 2;     // warps w, w + 4, ... share a sub-partition
 
   // edges whose P_c goes through the TMA ring: every contraction.  A leaf with a hard code needs
   // one COLUMN of P_c per site, gathered straight from the transposed copy in L2
@@ -170,7 +164,6 @@ prune_dmma_kernel(int S, int64_t n_sites, int64_t stride, const int4* __restrict
   for (int i = tid; i < n_ops; i += kThreads) prog_s[i] = program[i];
   for (int i = tid; i < SP; i += kThreads) pi_s[i] = (i < S) ? (root_distn ? root_distn[i] : 1.0) : 0.0;
   if (tid < kRing) done_cnt[tid] = 0;
-  if (tid < 4) turn_s[tid] = 0;
   if (tid == 0) {
     for (int b = 0; b < kRing; ++b) mbar_init(&full_bar[b], 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -396,20 +389,9 @@ prune_dmma_kernel(int S, int64_t n_sites, int64_t stride, const int4* __restrict
         RT_PROF_END(2)
         RT_PROF_BEGIN
 
-        // ---- wait for P_c and (optionally) for this warp's turn on the sub-partition's tensor pipe ----
+        // ---- wait for P_c ----
         mbar_wait(&full_bar[buf], parity);
         RT_PROF_END(3)
-        RT_PROF_BEGIN
-        if (pingpong == 1) {          // strict rotation among the sub-partition's warps
-          if (lane == 0)
-            while (turn_s[pair] != my_turn) __nanosleep(20);
-          __syncwarp();
-        } else if (pingpong == 2) {   // mutex: whoever is ready takes the pipe
-          if (lane == 0)
-            while (atomicCAS(const_cast<int*>(&turn_s[pair]), 0, 1) != 0) __nanosleep(40);
-          __syncwarp();
-        }
-        RT_PROF_END(4)
         RT_PROF_BEGIN
         double msg[MT][kNT][2];
 #pragma unroll
@@ -433,10 +415,6 @@ prune_dmma_kernel(int S, int64_t n_sites, int64_t stride, const int4* __restrict
 #endif
         RT_PROF_END(5)
         RT_PROF_BEGIN
-        if (pingpong) {
-          __syncwarp();
-          if (lane == 0) turn_s[pair] = pingpong == 1 ? (my_turn + 1) % kTurns : 0;
-        }
         release(consumed);
         ++consumed;
         if (first) {
@@ -624,16 +602,14 @@ prune_dmma_kernel(int S, int64_t n_sites, int64_t stride, const int4* __restrict
   }
 }
 
-template <int MT, int OBS, bool STORE, int NT>
+template <int MT, int OBS, bool STORE>
 int launch(int S, int64_t n_sites, int64_t stride, const int4* program, int n_ops, int n_slots,
            const double* Ppad, const double* PT, const double* rowsum, const double* root_distn,
            const void* obs, double* slots_ws, double* partials, int32_t* exponents, double* loglik,
-           int8_t* status, double* loglik_sum, int pingpong, cudaStream_t stream) {
-  static_assert(NT == 1 || NT == 2, "NT");
+           int8_t* status, double* loglik_sum, cudaStream_t stream) {
   constexpr int SP = 8 * MT;
   constexpr int LDP = SP;
-  auto kern = prune_dmma_kernel<MT, OBS, STORE, NT>;
-  constexpr int kWarps = 16 / NT, kThreads = 32 * kWarps, kWarpSites = 8 * NT, kLdB = kWarpSites + 4;
+  auto kern = prune_dmma_kernel<MT, OBS, STORE>;
   size_t smem = sizeof(double) * ((size_t)kRing * SP * LDP + (size_t)kWarps * SP * kLdB + SP) +
                 sizeof(int) * (size_t)kWarps * n_slots * kWarpSites + sizeof(int4) * (size_t)n_ops +
                 sizeof(int) * (((size_t)n_ops + 3) & ~(size_t)3);
@@ -653,7 +629,7 @@ int launch(int S, int64_t n_sites, int64_t stride, const int4* program, int n_op
   const unsigned grid = (unsigned)(tiles < sms ? tiles : sms);
   kern<<<grid, kThreads, smem, stream>>>(S, n_sites, stride, program, n_ops, n_slots, Ppad, PT,
                                          rowsum, root_distn, obs, slots_ws, partials, exponents,
-                                         loglik, status, loglik_sum, (int)code_capacity, pingpong);
+                                         loglik, status, loglik_sum, (int)code_capacity);
   RT_CUDA_CHECK(cudaGetLastError());
   return RT_OK;
 }
@@ -663,12 +639,11 @@ int launch_mt(int S, int obs_kind, bool store, int64_t n_sites, int64_t stride, 
               int n_ops, int n_slots, const double* Ppad, const double* PT, const double* rowsum,
               const double* root_distn, const void* obs, double* slots_ws, double* partials,
               int32_t* exponents, double* loglik, int8_t* status, double* loglik_sum,
-              int pingpong, int nt, cudaStream_t stream) {
+              cudaStream_t stream) {
 #define RT_ARGS S, n_sites, stride, program, n_ops, n_slots, Ppad, PT, rowsum, root_distn, obs, \
-                slots_ws, partials, exponents, loglik, status, loglik_sum, pingpong, stream
-#define RT_GO(OBSK)                                                                              \
-  return nt == 1 ? (store ? launch<MT, OBSK, true, 1>(RT_ARGS) : launch<MT, OBSK, false, 1>(RT_ARGS)) \
-                 : (store ? launch<MT, OBSK, true, 2>(RT_ARGS) : launch<MT, OBSK, false, 2>(RT_ARGS))
+                slots_ws, partials, exponents, loglik, status, loglik_sum, stream
+#define RT_GO(OBSK) \
+  return store ? launch<MT, OBSK, true>(RT_ARGS) : launch<MT, OBSK, false>(RT_ARGS)
   switch (obs_kind) {
     case OBS_CODES: RT_GO(OBS_CODES);
     case OBS_MASK:  RT_GO(OBS_MASK);
@@ -697,16 +672,11 @@ int rt_prune_dmma_dispatch(int S, int obs_kind, bool store, int64_t n_sites, int
   double* PT = Ppad + n_pad;
   double* rowsum = PT + n_pad;
   double* slots_ws = store ? nullptr : rowsum + n_rs;
-  // tensor-pipe arbitration between the warps of an SM sub-partition: 0 free running, 1 strict
-  // rotation, 2 mutex; sites per warp: RT_PRUNE_DMMA_NT = 2 (16 sites, 8 warps) or 1 (8 sites, 16 warps)
-  static const int pingpong = [] { const char* e = getenv("RT_PRUNE_DMMA_PINGPONG"); return e ? atoi(e) : kDefaultPingpong; }();
-  static const int nt = [] { const char* e = getenv("RT_PRUNE_DMMA_NT"); return e ? (e[0] == '1' ? 1 : 2) : kDefaultNT; }();
   pack_kernel<<<n_nodes, 256, 0, stream>>>(P, S, SP, n_nodes, Ppad, PT, rowsum);
   const int4* prog = reinterpret_cast<const int4*>(program);
   int rc;
 #define RT_ARGS S, obs_kind, store, n_sites, stride, prog, n_ops, n_slots, Ppad, PT, rowsum, \
-                root_distn, obs, slots_ws, partials, exponents, loglik, status, loglik_sum,   \
-                pingpong, nt, stream
+                root_distn, obs, slots_ws, partials, exponents, loglik, status, loglik_sum, stream
   switch (MT) {
     case 2: rc = launch_mt<2>(RT_ARGS); break;
     case 4: rc = launch_mt<4>(RT_ARGS); break;

@@ -13,8 +13,6 @@ Reference call stacks replaced (SURVEY.md section 3):
 """
 from __future__ import annotations
 
-import os
-
 import numpy as np
 import torch
 
@@ -22,6 +20,11 @@ from . import _native
 from .lowering import TreeSchedule, MISSING
 
 OBS_CODES, OBS_MASK, OBS_DENSE, OBS_CODES4 = 0, 1, 2, 3
+
+# compute streams of the host-buffer entry point; chunks take turns: the kernels of consecutive
+# chunks are independent, so the tail wave of one chunk's kernel (a chunk is only ~1.3-1.7 waves
+# of CTAs) is filled with CTAs of the next chunks' kernels
+E2E_STREAMS = 3
 
 
 def _ptr(t):
@@ -141,16 +144,6 @@ class TreeMJP(object):
         self._serial = TreeMJP._n_made
         self._Q_stage = None
         self.events = None     # optional dict: name -> [(start, end) CUDA events]
-        # S <= 4: up + down pass as ONE persistent kernel (csrc/rt_fused_small.cu) instead of two.
-        # Off by default: measured on B200 at C2 size the fused kernel takes 1.00 ms against 0.92 ms
-        # for the two kernels (profiles/r2_fused_small.md) -- it removes the 2 GB of HBM traffic of the
-        # stored partials, but the path is latency / issue bound, not HBM bound, and one kernel
-        # has to run the up pass at the walk's lower occupancy.
-        self.fused = os.environ.get('RT_FUSED', '0') == '1'
-        self.fused_ctas_per_sm = int(os.environ.get('RT_FUSED_CTAS', '0'))
-        # S > 16: when the rate matrix is time-reversible w.r.t. the root distribution, contract
-        # the edge weights in its eigenbasis instead of exponentiating a 2S x 2S block per edge
-        self.auto_spectral_frechet = os.environ.get('RT_AUTO_SPECTRAL_FRECHET', '1') != '0'
 
     def _buf(self, name, shape, dtype, zero=False):
         """Reusable device workspace (avoids per-call allocation)."""
@@ -360,37 +353,6 @@ class TreeMJP(object):
         for cs in self._ov_streams:
             cur.wait_stream(cs)
 
-    def _posterior_fused(self, obs, out=None):
-        """S <= 4, nothing but loglik / W / root posterior wanted: the fused up + down kernel
-        (csrc/rt_fused_small.cu); None when the shape is not covered."""
-        import ctypes
-        P = self.transition_matrices()
-        prog = self._programs(obs)
-        N, stride = obs.n_sites, obs.stride
-        if out is None:
-            loglik = torch.empty(N, dtype=torch.float64, device=self.device)
-            status = torch.empty(N, dtype=torch.int8, device=self.device)
-        else:
-            loglik, status = out
-        llsum = self._buf('loglik_sum', (1,), torch.float64, zero=True)
-        W = self._buf('W', (self.sched.n, self.S, self.S), torch.float64, zero=True)
-        rps = self._buf('root_post_sum', (self.S,), torch.float64, zero=True)
-        handled = ctypes.c_int(0)
-        self._mark('fused')
-        rc = _native.lib().rt_posterior_fused(
-            self.S, self.sched.n, self.sched.n_store, N, stride, _ptr(prog['ops']), prog['n_ops'],
-            prog['n_slots'], _ptr(P), _ptr(self.root_distn), obs.kind, _ptr(obs.data), _ptr(loglik),
-            _ptr(status), _ptr(llsum), _ptr(W), _ptr(rps), int(self.fused_ctas_per_sm),
-            ctypes.byref(handled), _stream())
-        _native.check(rc, 'rt_posterior_fused')
-        if not handled.value:
-            if self.events is not None:
-                self.events['fused'].pop()
-            return None
-        self._mark('fused')
-        return dict(loglik=loglik, status=status, loglik_sum=llsum[0], partials=None, exponents=None,
-                    node_distn=None, W=W, root_post_sum=rps, n_levels=len(prog['level_ptr']) - 1)
-
     def posterior(self, obs, want_exponents=False, want_node_distn=True, overlap_chunks=0):
         """Up + down pass.  Returns loglik, status, partials, node_distn (internal
         nodes, by store index), W[n,S,S] (site-summed J/P weights), root_post_sum[S].
@@ -398,10 +360,6 @@ class TreeMJP(object):
         schedule, see _posterior_overlapped."""
         if overlap_chunks > 1 and self.S <= 8 and not want_node_distn and not want_exponents:
             return self._posterior_overlapped(obs, int(overlap_chunks))
-        if self.S <= 4 and not want_node_distn and not want_exponents and self.fused:
-            res = self._posterior_fused(obs)
-            if res is not None:
-                return res
         llsum = self._buf('loglik_sum', (1,), torch.float64, zero=True)
         up = self.log_likelihood(obs, keep_partials=True, want_exponents=want_exponents,
                                  loglik_sum=llsum)
@@ -534,9 +492,7 @@ class TreeMJP(object):
         codes_dev = self._buf('h_codes%d' % bps, (L, NB), torch.uint8)
         loglik = self._buf('h_loglik', (N,), torch.float64)
         status = self._buf('h_status', (N,), torch.int8)
-        import ctypes
-        use_fused = S <= 4 and self.fused
-        partials = None if use_fused else self._buf('partials', (self.sched.n_store, S, N), torch.float64)
+        partials = self._buf('partials', (self.sched.n_store, S, N), torch.float64)
         W = self._buf('W', (n, S, S), torch.float64, zero=True)
         rps = self._buf('root_post_sum', (S,), torch.float64, zero=True)
         llsum = self._buf('h_llsum', (1,), torch.float64, zero=True)
@@ -547,11 +503,7 @@ class TreeMJP(object):
         cur = torch.cuda.current_stream()
         if getattr(self, '_copy_streams', None) is None:
             self._copy_streams = (torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev))
-            # several compute streams (three by default), chunks take turns: the kernels of
-            # consecutive chunks are independent, so the tail wave of one chunk's kernel (a chunk
-            # is only ~1.3-1.7 waves of CTAs) is filled with CTAs of the next chunks' kernels
-            self._compute_streams = tuple(torch.cuda.Stream(device=dev)
-                                          for _ in range(int(os.environ.get('RT_E2E_STREAMS', '3'))))
+            self._compute_streams = tuple(torch.cuda.Stream(device=dev) for _ in range(E2E_STREAMS))
         s_in, s_out = self._copy_streams
         s_in.wait_stream(cur)
         s_out.wait_stream(cur)
@@ -571,31 +523,18 @@ class TreeMJP(object):
         for k, ((lo, hi), e) in enumerate(zip(bounds, ev_in)):
             cs = self._compute_streams[k % len(self._compute_streams)]
             cs.wait_event(e)
-            if use_fused:
-                handled = ctypes.c_int(0)
-                rc = lib.rt_posterior_fused(
-                    S, n, self.sched.n_store, hi - lo, N, _ptr(prog['ops']), prog['n_ops'],
-                    prog['n_slots'], _ptr(P), _ptr(self.root_distn), kind,
-                    codes_dev.data_ptr() + lo // bps, loglik.data_ptr() + 8 * lo,
-                    status.data_ptr() + lo, _ptr(llsum), _ptr(W), _ptr(rps),
-                    int(self.fused_ctas_per_sm), ctypes.byref(handled), cs.cuda_stream)
-                _native.check(rc, 'rt_posterior_fused')
-                use_fused = bool(handled.value)
-            if not use_fused:
-              if partials is None:
-                  partials = self._buf('partials', (self.sched.n_store, S, N), torch.float64)
-              rc = lib.rt_prune_loglik(
+            rc = lib.rt_prune_loglik(
                 S, n, hi - lo, N, _ptr(prog['ops']), prog['n_ops'], prog['n_slots'], _ptr(P),
                 _ptr(self.root_distn), kind, codes_dev.data_ptr() + lo // bps,
                 partials.data_ptr() + 8 * lo, None, loglik.data_ptr() + 8 * lo,
                 status.data_ptr() + lo, _ptr(llsum), cs.cuda_stream)
-              _native.check(rc, 'rt_prune_loglik')
-              rc = lib.rt_posterior_stats(
+            _native.check(rc, 'rt_prune_loglik')
+            rc = lib.rt_posterior_stats(
                 S, n, hi - lo, N, _ptr(prog['ops']), prog['n_ops'], prog['n_slots'],
                 _ptr(prog['edges']), lp.ctypes.data, len(lp) - 1, _ptr(P), _ptr(self.root_distn),
                 kind, codes_dev.data_ptr() + lo // bps, partials.data_ptr() + 8 * lo,
                 status.data_ptr() + lo, None, _ptr(W), _ptr(rps), cs.cuda_stream)
-              _native.check(rc, 'rt_posterior_stats')
+            _native.check(rc, 'rt_posterior_stats')
             done = torch.cuda.Event()
             done.record(cs)
             with torch.cuda.stream(s_out):
@@ -615,7 +554,9 @@ class TreeMJP(object):
         n, S = self.sched.n, self.S
         if getattr(self, '_spectral_D', None) is not None and self._P_valid and not self._spectral_dec[3]:
             return self._history_statistics_spectral(W)
-        if S > 16 and self.auto_spectral_frechet and self._reversible_decomposition() is not None:
+        # S > 16: when the rate matrix is time-reversible w.r.t. the root distribution, contract
+        # the edge weights in its eigenbasis instead of exponentiating a 2S x 2S block per edge
+        if S > 16 and self._reversible_decomposition() is not None:
             return self._history_statistics_spectral(W, self._reversible_decomposition())
         M = self._buf('M', (n, S, S), torch.float64)
         dwell = torch.empty(S, dtype=torch.float64, device=self.device)
@@ -698,7 +639,7 @@ class TreeMJP(object):
         cache = obs.__dict__.setdefault('_rt_graphs', {})
         prog = self._programs(obs)
         key = ('ehs', self._serial, obs.kind, obs.data.data_ptr(), obs.n_sites, obs.stride,
-               _ptr(self.root_distn), prog['ops'].data_ptr(), self.fused)
+               _ptr(self.root_distn), prog['ops'].data_ptr())
         entry = cache.get(key)
         if entry is None:
             if getattr(self, '_graph_refused', False):

@@ -509,11 +509,10 @@ def test_packed_codes4_are_bit_identical_to_uint8_codes(S, n_sites):
 
 @pytest.mark.parametrize('S,n_leaves,n_sites,kind', [(4, 32, 3001, 'codes'), (4, 32, 777, 'codes4'), (3, 9, 515, 'codes'),
                                                      (2, 6, 300, 'mask'), (4, 11, 1300, 'mask'), (4, 7, 600, 'dense')])
-def test_fused_small_kernel_matches_oracle(rt, S, n_leaves, n_sites, kind):
-    """rt_posterior_fused (S <= 4: up pass, root combine, down walk and W accumulation in one
-    persistent kernel, partials in a per-CTA scratch) against the oracle and against the two-kernel
-    path, for every observation encoding, ragged site counts, missing cells and a reducible rate
-    matrix with infeasible sites (_mjp_dense.py:410-539)."""
+def test_small_state_expectations_match_oracle(rt, S, n_leaves, n_sites, kind):
+    """The S <= 4 expectation pass (rt_prune_loglik, then rt_posterior_stats: root combine, down
+    walk and W accumulation) against the oracle, for every observation encoding, ragged site counts,
+    missing cells and a reducible rate matrix with infeasible sites (_mjp_dense.py:410-539)."""
     from raoteh_b200.lowering import TreeSchedule
     from raoteh_b200 import synth
     rng = np.random.default_rng(900 + S + n_leaves)
@@ -555,22 +554,15 @@ def test_fused_small_kernel_matches_oracle(rt, S, n_leaves, n_sites, kind):
         full[nodes] = lik.transpose(0, 2, 1)
         oobs = np_oracle.Obs('dense', S, n_sites, lik=full, has=has)
     o = np_oracle.expected_history_statistics(parent, length, Q, P, oobs, pi)
-    res = {}
-    for fused in (True, False):
-        mjp = rt.TreeMJP(sched, Q, root_distn=pi)
-        mjp.fused = fused
-        r = mjp.expected_history_statistics(obs)
-        assert (r['partials'] is None) == fused        # the fused path really ran (no stored partials)
-        res[fused] = r
-        ok = np.isfinite(o['loglik'])
-        assert ((r['status'].cpu().numpy() == 0) == ok).all()
-        # atol: an unrestricted site has likelihood 1, log-lik 0 up to one rounding
-        np.testing.assert_allclose(r['loglik'].cpu().numpy()[ok], o['loglik'][ok], rtol=RTOL, atol=1e-13)
-        np.testing.assert_allclose(float(r['loglik_sum']), o['loglik'][ok].sum(), rtol=1e-10)
-        np.testing.assert_allclose(r['dwell'].cpu().numpy(), o['dwell'], rtol=RTOL)
-        np.testing.assert_allclose(r['trans'].cpu().numpy(), o['trans'], rtol=RTOL, atol=1e-12)
-        np.testing.assert_allclose(r['root_post_sum'].cpu().numpy(), o['root_post'].sum(axis=0), rtol=RTOL)
-    np.testing.assert_allclose(res[True]['W'].cpu().numpy(), res[False]['W'].cpu().numpy(), rtol=1e-11, atol=1e-13)
+    r = rt.TreeMJP(sched, Q, root_distn=pi).expected_history_statistics(obs)
+    ok = np.isfinite(o['loglik'])
+    assert ((r['status'].cpu().numpy() == 0) == ok).all()
+    # atol: an unrestricted site has likelihood 1, log-lik 0 up to one rounding
+    np.testing.assert_allclose(r['loglik'].cpu().numpy()[ok], o['loglik'][ok], rtol=RTOL, atol=1e-13)
+    np.testing.assert_allclose(float(r['loglik_sum']), o['loglik'][ok].sum(), rtol=1e-10)
+    np.testing.assert_allclose(r['dwell'].cpu().numpy(), o['dwell'], rtol=RTOL)
+    np.testing.assert_allclose(r['trans'].cpu().numpy(), o['trans'], rtol=RTOL, atol=1e-12)
+    np.testing.assert_allclose(r['root_post_sum'].cpu().numpy(), o['root_post'].sum(axis=0), rtol=RTOL)
 
 
 @pytest.mark.parametrize('shape', ['star', 'caterpillar', 'many_tiles', 'polytomy'])

@@ -18,7 +18,9 @@ L.rt_debug_prune_profile(buf)
 mjp.log_likelihood(obs)
 L.rt_debug_prune_profile(buf)
 v = list(buf)
-names = ['total', 'leaf gather', 'B fill', 'wait P', 'wait token', 'DMMA loop', 'release+product', 'store/root', 'code staging', 'other ops', 'warps']
+names = ['total', 'leaf gather', 'B fill', 'wait P', None, 'DMMA loop', 'release+product', 'store/root', 'code staging', 'other ops', 'warps']
 tot = v[0]
 for n, x in zip(names, v):
+    if n is None:       # slot 4: unused
+        continue
     print('%-16s %14d  %5.1f%%  per warp %.0f' % (n, x, 100.0 * x / tot, x / max(1, v[10])))

@@ -15,6 +15,4 @@ timeout 300 ncu --set full --clock-control none -k regex:'down_leaf_scatter|expm
 ncu -i /tmp/${T}_c3leaf.ncu-rep --page raw --csv > gpurun_out/${T}_c3leaf_raw.csv 2>/dev/null
 timeout 300 ncu --set full --clock-control none -k regex:raoteh_kernel --launch-skip 2 -c 1 -f -o /tmp/${T}_c4 python tools/c4_one.py > gpurun_out/${T}_ncu_c4.log 2>&1
 ncu -i /tmp/${T}_c4.ncu-rep --page raw --csv > gpurun_out/${T}_c4_raw.csv 2>/dev/null
-RT_FUSED=1 timeout 300 ncu --set full --clock-control none -k regex:fused_small --launch-skip 2 -c 1 -f -o /tmp/${T}_fused python tools/fused_one.py > gpurun_out/${T}_ncu_fused.log 2>&1
-ncu -i /tmp/${T}_fused.ncu-rep --page raw --csv > gpurun_out/${T}_fused_raw.csv 2>/dev/null
 tail -n 2 gpurun_out/${T}_smoke.log gpurun_out/${T}_ncu_full.log gpurun_out/${T}_ncu_down.log; ls -la gpurun_out | tail -15

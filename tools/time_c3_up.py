@@ -1,5 +1,5 @@
 """C3 (61 states, 128 leaves, 1e5 sites): time of the DMMA pruning kernel alone (log-lik only)
-and with stored partials.  Used for the RT_PRUNE_DMMA_PHASE_DELAY sweep."""
+and with stored partials."""
 import sys, os, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch, numpy as np
@@ -24,5 +24,4 @@ def timed(fn, n=8):
 t_ll, r = timed(lambda: mjp.log_likelihood(obs))
 mjp.events = {}
 t_ex, r2 = timed(lambda: mjp.expected_history_statistics(obs), n=4)
-print(json.dumps(dict(delay=os.environ.get('RT_PRUNE_DMMA_PHASE_DELAY'), loglik_ms=t_ll, expectations_ms=t_ex,
-                      loglik_sum=float(r['loglik'].sum()))))
+print(json.dumps(dict(loglik_ms=t_ll, expectations_ms=t_ex, loglik_sum=float(r['loglik'].sum()))))
