@@ -21,18 +21,28 @@ from .lowering import TreeSchedule, MISSING
 
 OBS_CODES, OBS_MASK, OBS_DENSE, OBS_CODES4 = 0, 1, 2, 3
 
-# compute streams of the host-buffer entry point; chunks take turns: the kernels of consecutive
-# chunks are independent, so the tail wave of one chunk's kernel (a chunk is only ~1.3-1.7 waves
-# of CTAs) is filled with CTAs of the next chunks' kernels
+# compute streams of the site-chunk pipeline (TreeMJP._chunked); chunks take turns: the kernels of
+# consecutive chunks are independent, so the tail wave of one chunk's kernel (a chunk is only
+# ~1.3-1.7 waves of CTAs) is filled with CTAs of the next chunks' kernels
 E2E_STREAMS = 3
 
 
-def _ptr(t):
-    return None if t is None else t.data_ptr()
+def _ptr(t, lo=0):
+    """Device address of `t` (None: NULL), or of its site `lo` when the last axis is the site axis."""
+    return None if t is None else t.data_ptr() + lo * t.element_size()
 
 
-def _stream():
-    return torch.cuda.current_stream().cuda_stream
+def _stream(s=None):
+    return (torch.cuda.current_stream() if s is None else s).cuda_stream
+
+
+def _obs_slot(sched, nodes):
+    """Row of the observations per tree node (-1 = unobserved) for observations of `nodes`, in
+    order (None: the leaves)."""
+    nodes = sched.leaves if nodes is None else np.asarray(nodes)
+    obs_slot = np.full(sched.n, -1, dtype=np.int32)
+    obs_slot[nodes] = np.arange(len(nodes), dtype=np.int32)
+    return obs_slot
 
 
 def pack_codes4(codes):
@@ -69,28 +79,26 @@ class Observations(object):
         # site stride of the per-site arrays that go with these observations
         self.stride = int(data.shape[-1]) * (2 if kind == OBS_CODES4 else 1)
 
+    def site_ptr(self, lo):
+        """Device address of site `lo` in `data` (every encoding is site-minor; OBS_CODES4 holds
+        two sites per byte, so `lo` must be even there)."""
+        return self.data.data_ptr() + lo // 2 if self.kind == OBS_CODES4 else _ptr(self.data, lo)
+
     @classmethod
-    def from_leaf_codes(cls, sched, codes, leaf_nodes=None, device='cuda', pinned=None):
+    def from_leaf_codes(cls, sched, codes, leaf_nodes=None, device='cuda'):
         """codes: uint8 [n_leaves, n_sites] host array (numpy) or device tensor."""
-        leaf_nodes = sched.leaves if leaf_nodes is None else np.asarray(leaf_nodes)
-        obs_slot = np.full(sched.n, -1, dtype=np.int32)
-        obs_slot[leaf_nodes] = np.arange(len(leaf_nodes), dtype=np.int32)
         if isinstance(codes, np.ndarray):
             host = torch.from_numpy(np.ascontiguousarray(codes, dtype=np.uint8))
             data = host.to(device, non_blocking=False)
         else:
             data = codes.to(device=device, dtype=torch.uint8).contiguous()
-        return cls(OBS_CODES, data, obs_slot, data.shape[1])
+        return cls(OBS_CODES, data, _obs_slot(sched, leaf_nodes), data.shape[1])
 
     @classmethod
     def from_leaf_codes4(cls, sched, codes, leaf_nodes=None, device='cuda'):
         """Hard leaf codes stored two per byte (RT_OBS_CODES4, S <= 8)."""
-        leaf_nodes = sched.leaves if leaf_nodes is None else np.asarray(leaf_nodes)
-        obs_slot = np.full(sched.n, -1, dtype=np.int32)
-        obs_slot[leaf_nodes] = np.arange(len(leaf_nodes), dtype=np.int32)
-        n_sites = codes.shape[1]
         data = torch.from_numpy(pack_codes4(codes)).to(device)
-        return cls(OBS_CODES4, data, obs_slot, n_sites)
+        return cls(OBS_CODES4, data, _obs_slot(sched, leaf_nodes), codes.shape[1])
 
     @classmethod
     def from_masks(cls, sched, mask, device='cuda'):
@@ -103,10 +111,8 @@ class Observations(object):
     @classmethod
     def from_dense(cls, sched, lik, nodes, device='cuda'):
         """lik: float64 [len(nodes), S, n_sites] emission likelihoods of `nodes`."""
-        obs_slot = np.full(sched.n, -1, dtype=np.int32)
-        obs_slot[np.asarray(nodes)] = np.arange(len(nodes), dtype=np.int32)
         data = torch.from_numpy(np.ascontiguousarray(lik, dtype=np.float64)).to(device)
-        return cls(OBS_DENSE, data, obs_slot, data.shape[2])
+        return cls(OBS_DENSE, data, _obs_slot(sched, nodes), data.shape[2])
 
 
 class TreeMJP(object):
@@ -143,6 +149,11 @@ class TreeMJP(object):
         TreeMJP._n_made += 1
         self._serial = TreeMJP._n_made
         self._Q_stage = None
+        self._spectral_D = None     # stationary weights of use_spectral, None = Pade
+        self._spectral_dec = None   # (A, lam, B) behind the spectral P
+        self._rev_cache = None      # (hash of Q, (A, lam, B) or None): _reversible_decomposition
+        self._streams = None        # copy-in, copy-out and E2E_STREAMS compute streams of _chunked
+        self._graph_refused = False
         self.events = None     # optional dict: name -> [(start, end) CUDA events]
 
     def _buf(self, name, shape, dtype, zero=False):
@@ -188,18 +199,21 @@ class TreeMJP(object):
         self._spectral_D = None if D is None else np.asarray(D, dtype=np.float64)
         self._P_valid = False
 
-    def _spectral_matrices(self):
+    def _decompose(self, D, rtol):
+        """(A, lam, B) on the device, Q = A diag(lam) B (examples/p53/qtop.py:126-148), for the one
+        rate matrix; ValueError unless it is time-reversible with respect to the weights `D`."""
         from . import qtop
-        S, n = self.S, self.sched.n
+        S = self.S
+        A, lam, B = qtop.decompose_spectral_v2(qtop.symmetric_factor(self.Q_host[0], D, rtol=rtol), D)
+        dec = torch.from_numpy(np.concatenate([A.ravel(), lam, B.ravel()])).to(self.device)
+        return dec[:S * S].view(S, S), dec[S * S:S * S + S], dec[S * S + S:].view(S, S)
+
+    def _spectral_matrices(self):
         D = self._spectral_D
-        A, lam, B = qtop.decompose_spectral_v2(qtop.symmetric_factor(self.Q_host[0], D), D)
-        stage = np.concatenate([A.ravel(), lam, B.ravel()])
-        dec = torch.from_numpy(stage).to(self.device)
+        self._spectral_dec = A, lam, B = self._decompose(D, rtol=1e-9)
         off = torch.from_numpy((D == 0).astype(np.uint8)).to(self.device)
-        a, l, b = dec[:S * S], dec[S * S:S * S + S], dec[S * S + S:]
-        self._spectral_dec = (a.view(S, S), l, b.view(S, S), bool((D == 0).any()))
-        rc = _native.lib().rt_expm_spectral(_ptr(a), _ptr(l), _ptr(b), _ptr(self.length), _ptr(off),
-                                            n, S, _ptr(self._P), _stream())
+        rc = _native.lib().rt_expm_spectral(_ptr(A), _ptr(lam), _ptr(B), _ptr(self.length), _ptr(off),
+                                            self.sched.n, self.S, _ptr(self._P), _stream())
         _native.check(rc, 'rt_expm_spectral')
 
     # ---- K1 ---------------------------------------------------------------
@@ -209,7 +223,7 @@ class TreeMJP(object):
             n, S = self.sched.n, self.S
             if self._P is None:
                 self._P = torch.empty((n, S, S), dtype=torch.float64, device=self.device)
-            if getattr(self, '_spectral_D', None) is not None:
+            if self._spectral_D is not None:
                 self._spectral_matrices()
             else:
                 rc = _native.lib().rt_expm_batched(_ptr(self.Q), _ptr(self.q_index), _ptr(self.length),
@@ -242,10 +256,38 @@ class TreeMJP(object):
         return mask
 
     # ---- K2 / K3 ------------------------------------------------------------
+    def _up(self, obs, prog, lo, hi, stream, loglik, status, partials=None, exponents=None,
+            loglik_sum=None):
+        """rt_prune_loglik for the sites [lo, hi) of `obs` on `stream` (None: the current one).
+        Every per-site array is site-minor, so each pointer is its base + lo * element size.
+        P comes from transition_matrices(): a caller that forks streams computes it first."""
+        rc = _native.lib().rt_prune_loglik(
+            self.S, self.sched.n, hi - lo, obs.stride, _ptr(prog['ops']), prog['n_ops'], prog['n_slots'],
+            _ptr(self.transition_matrices()), _ptr(self.root_distn), obs.kind, obs.site_ptr(lo),
+            _ptr(partials, lo), _ptr(exponents, lo), _ptr(loglik, lo), _ptr(status, lo),
+            _ptr(loglik_sum), _stream(stream))
+        _native.check(rc, 'rt_prune_loglik')
+
+    def _down(self, obs, prog, lo, hi, stream, partials, status, node_distn, W, root_post_sum,
+              K=None, branch=None):
+        """rt_posterior_stats for the sites [lo, hi) of `obs` on `stream`, addressed as in _up;
+        rt_posterior_branch_stats when a per-edge kernel K is given (per-site output `branch`)."""
+        lp = prog['level_ptr']
+        args = (self.S, self.sched.n, hi - lo, obs.stride, _ptr(prog['ops']), prog['n_ops'],
+                prog['n_slots'], _ptr(prog['edges']), lp.ctypes.data, len(lp) - 1,
+                _ptr(self.transition_matrices()), _ptr(self.root_distn), obs.kind, obs.site_ptr(lo),
+                _ptr(partials, lo), _ptr(status, lo), _ptr(node_distn, lo), _ptr(W),
+                _ptr(root_post_sum))
+        if K is None:
+            rc = _native.lib().rt_posterior_stats(*args, _stream(stream))
+        else:
+            rc = _native.lib().rt_posterior_branch_stats(*args, _ptr(K), _ptr(branch, lo), _stream(stream))
+        _native.check(rc, 'rt_posterior_stats' if K is None else 'rt_posterior_branch_stats')
+
     def log_likelihood(self, obs, keep_partials=False, want_exponents=False, out=None,
                        loglik_sum=None):
         """Per-site log-likelihood.  Returns dict(loglik, status[, partials, exponents])."""
-        P = self.transition_matrices()
+        self.transition_matrices()          # before the 'up' event: P is not part of the up pass
         prog = self._programs(obs)
         N, stride = obs.n_sites, obs.stride
         dev = self.device
@@ -260,11 +302,7 @@ class TreeMJP(object):
             if want_exponents:
                 exponents = self._buf('exponents', (self.sched.n_store, stride), torch.int32)
         self._mark('up')
-        rc = _native.lib().rt_prune_loglik(
-            self.S, self.sched.n, N, stride, _ptr(prog['ops']), prog['n_ops'], prog['n_slots'],
-            _ptr(P), _ptr(self.root_distn), obs.kind, _ptr(obs.data), _ptr(partials),
-            _ptr(exponents), _ptr(loglik), _ptr(status), _ptr(loglik_sum), _stream())
-        _native.check(rc, 'rt_prune_loglik')
+        self._up(obs, prog, 0, N, None, loglik, status, partials, exponents, loglik_sum)
         self._mark('up')
         res = dict(loglik=loglik, status=status)
         if keep_partials:
@@ -273,135 +311,113 @@ class TreeMJP(object):
         return res
 
     # ---- K4 / K5 ------------------------------------------------------------
-    def _posterior_overlapped(self, obs, n_chunks, use_graph=True):
-        """Up + down pass for S <= 8 with the site axis cut into chunks that alternate between
-        two streams: the kernels of different chunks are independent, so the write-heavy
-        pruning kernel of one chunk runs under the issue-bound walk of another and no kernel's
-        tail wave leaves SMs idle."""
-        lib = _native.lib()
-        S, n = self.S, self.sched.n
-        N, stride = obs.n_sites, obs.stride
-        dev = self.device
+    def _chunked(self, obs, n_chunks, codes_host=None, out_loglik=None, out_status=None):
+        """Up + down pass with the site axis cut into `n_chunks` chunks (multiples of 128 sites) that
+        take turns on E2E_STREAMS compute streams.  codes_host: pinned codes in the layout of
+        obs.data; the H2D copies of all chunks are enqueued first on the copy-in stream, one event
+        per chunk, so chunk k+1 arrives under the kernels of chunk k.  out_loglik / out_status:
+        pinned arrays the chunk's log-likelihoods and status go to on the copy-out stream as soon as
+        its kernels are done; the caller joins that stream.  Sites are independent and W only
+        accumulates, so the chunks need no order among themselves.  Returns the dict of
+        `posterior`, without node marginals and exponents."""
+        S, n, N = self.S, self.sched.n, obs.n_sites
         prog = self._programs(obs)
-        P = self.transition_matrices()
-        loglik = self._buf('ov_loglik', (N,), torch.float64)
-        status = self._buf('ov_status', (N,), torch.int8)
-        partials = self._buf('partials', (self.sched.n_store, S, stride), torch.float64)
+        self.transition_matrices()          # on the current stream, before the fork
+        loglik = self._buf('h_loglik', (N,), torch.float64)
+        status = self._buf('h_status', (N,), torch.int8)
+        partials = self._buf('partials', (self.sched.n_store, S, obs.stride), torch.float64)
         W = self._buf('W', (n, S, S), torch.float64, zero=True)
         rps = self._buf('root_post_sum', (S,), torch.float64, zero=True)
-        lp = prog['level_ptr']
-        esz = {OBS_CODES: 1, OBS_MASK: 8, OBS_DENSE: 8, OBS_CODES4: 0.5}[obs.kind]
-        if getattr(self, '_ov_streams', None) is None:
-            self._ov_streams = (torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev))
-            self._ov_graphs = {}
-        res = dict(loglik=loglik, status=status, partials=partials, exponents=None, node_distn=None,
-                   W=W, root_post_sum=rps, n_levels=len(lp) - 1)
-        # the chunk schedule is launch-bound on the host (2 launches per chunk), so it is
-        # captured once per (observations, chunking) into a CUDA graph and replayed.  The graphs
-        # live ON the Observations object (they bake in its data pointer, encoding and tree
-        # program), keyed by this engine's serial number and every other baked-in pointer: a new
-        # Observations never sees another one's graph even if the allocator hands it the same
-        # address, and the graphs die with the observations.
-        cache = obs.__dict__.setdefault('_rt_graphs', {})
-        key = (self._serial, obs.kind, obs.data.data_ptr(), N, stride, n_chunks, P.data_ptr(),
-               partials.data_ptr(), loglik.data_ptr(), status.data_ptr(), W.data_ptr(),
-               rps.data_ptr(), _ptr(self.root_distn), prog['ops'].data_ptr(),
-               prog['edges'].data_ptr())
-        self._ov_graphs = cache
-        g = self._ov_graphs.get(key)
-        if g is not None:
-            g.replay()
-            return res
-        if use_graph:
-            torch.cuda.synchronize()
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                self._ov_launch(obs, prog, P, partials, loglik, status, W, rps, n_chunks)
-            self._ov_graphs[key] = g
-            g.replay()
-            return res
-        self._ov_launch(obs, prog, P, partials, loglik, status, W, rps, n_chunks)
-        return res
-
-    def _ov_launch(self, obs, prog, P, partials, loglik, status, W, rps, n_chunks):
-        lib = _native.lib()
-        S, n = self.S, self.sched.n
-        N, stride = obs.n_sites, obs.stride
-        lp = prog['level_ptr']
-        esz = {OBS_CODES: 1, OBS_MASK: 8, OBS_DENSE: 8, OBS_CODES4: 0.5}[obs.kind]
+        llsum = self._buf('h_llsum', (1,), torch.float64, zero=True)
         cur = torch.cuda.current_stream()
-        chunk = _round_up((N + n_chunks - 1) // n_chunks, 256)
-        W.zero_()
-        rps.zero_()
-        for cs in self._ov_streams:
-            cs.wait_stream(cur)
-        for k, lo in enumerate(range(0, N, chunk)):
-            hi = min(N, lo + chunk)
-            cs = self._ov_streams[k % 2]
-            rc = lib.rt_prune_loglik(
-                S, n, hi - lo, stride, _ptr(prog['ops']), prog['n_ops'], prog['n_slots'], _ptr(P),
-                _ptr(self.root_distn), obs.kind, obs.data.data_ptr() + int(esz * lo),
-                partials.data_ptr() + 8 * lo, None, loglik.data_ptr() + 8 * lo,
-                status.data_ptr() + lo, None, cs.cuda_stream)
-            _native.check(rc, 'rt_prune_loglik')
-            rc = lib.rt_posterior_stats(
-                S, n, hi - lo, stride, _ptr(prog['ops']), prog['n_ops'], prog['n_slots'],
-                _ptr(prog['edges']), lp.ctypes.data, len(lp) - 1, _ptr(P), _ptr(self.root_distn),
-                obs.kind, obs.data.data_ptr() + int(esz * lo), partials.data_ptr() + 8 * lo,
-                status.data_ptr() + lo, None, _ptr(W), _ptr(rps), cs.cuda_stream)
-            _native.check(rc, 'rt_posterior_stats')
-        for cs in self._ov_streams:
+        if self._streams is None:
+            self._streams = [torch.cuda.Stream(device=self.device) for _ in range(2 + E2E_STREAMS)]
+        s_in, s_out, *compute = self._streams
+        for s in self._streams:
+            s.wait_stream(cur)
+        chunk = _round_up((N + n_chunks - 1) // n_chunks, 128)
+        bounds = [(lo, min(N, lo + chunk)) for lo in range(0, N, chunk)]
+        ev_in = []
+        if codes_host is not None:
+            base, (L, row) = obs.data.data_ptr(), obs.data.shape     # uint8 rows of `row` bytes
+            for lo, hi in bounds:
+                off = obs.site_ptr(lo) - base
+                end = obs.site_ptr(hi) - base if hi < N else row     # with an odd last site's byte
+                rc = _native.lib().rt_copy2d_async(base + off, row, codes_host.data_ptr() + off, row,
+                                                   end - off, L, 1, s_in.cuda_stream)
+                _native.check(rc, 'rt_copy2d_async')
+                e = torch.cuda.Event()
+                e.record(s_in)
+                ev_in.append(e)
+        for k, (lo, hi) in enumerate(bounds):
+            cs = compute[k % E2E_STREAMS]
+            if ev_in:
+                cs.wait_event(ev_in[k])
+            self._up(obs, prog, lo, hi, cs, loglik, status, partials, loglik_sum=llsum)
+            self._down(obs, prog, lo, hi, cs, partials, status, None, W, rps)
+            if out_loglik is not None:
+                done = torch.cuda.Event()
+                done.record(cs)
+                with torch.cuda.stream(s_out):
+                    s_out.wait_event(done)
+                    out_loglik[lo:hi].copy_(loglik[lo:hi], non_blocking=True)
+                    out_status[lo:hi].copy_(status[lo:hi], non_blocking=True)
+        for cs in compute:
             cur.wait_stream(cs)
+        return dict(loglik=loglik, status=status, loglik_sum=llsum[0], partials=partials,
+                    exponents=None, node_distn=None, W=W, root_post_sum=rps,
+                    n_levels=len(prog['level_ptr']) - 1)
 
     def posterior(self, obs, want_exponents=False, want_node_distn=True, overlap_chunks=0):
-        """Up + down pass.  Returns loglik, status, partials, node_distn (internal
+        """Up + down pass.  Returns loglik, status, loglik_sum, partials, node_distn (internal
         nodes, by store index), W[n,S,S] (site-summed J/P weights), root_post_sum[S].
-        overlap_chunks > 1 (S <= 8, no node marginals / exponents wanted): chunked two-stream
-        schedule, see _posterior_overlapped."""
+        overlap_chunks > 1 (S <= 8, no node marginals / exponents wanted): the site chunks of the
+        host-buffer pipeline, without its copies, see _chunked."""
         if overlap_chunks > 1 and self.S <= 8 and not want_node_distn and not want_exponents:
-            return self._posterior_overlapped(obs, int(overlap_chunks))
+            return self._chunked(obs, int(overlap_chunks))
         llsum = self._buf('loglik_sum', (1,), torch.float64, zero=True)
         up = self.log_likelihood(obs, keep_partials=True, want_exponents=want_exponents,
                                  loglik_sum=llsum)
         up['loglik_sum'] = llsum[0]      # sum of the finite log-likelihoods, reduced by the kernel
         prog = self._programs(obs)
-        N, stride = obs.n_sites, obs.stride
-        dev = self.device
-        P = self.transition_matrices()
         node_distn = None
         if want_node_distn or self.S > 8:
-            node_distn = self._buf('node_distn', (self.sched.n_store, self.S, stride), torch.float64)
+            node_distn = self._buf('node_distn', (self.sched.n_store, self.S, obs.stride), torch.float64)
         W = self._buf('W', (self.sched.n, self.S, self.S), torch.float64, zero=True)
         root_post_sum = self._buf('root_post_sum', (self.S,), torch.float64, zero=True)
-        lp = prog['level_ptr']
         self._mark('down')
-        rc = _native.lib().rt_posterior_stats(
-            self.S, self.sched.n, N, stride, _ptr(prog['ops']), prog['n_ops'], prog['n_slots'],
-            _ptr(prog['edges']), lp.ctypes.data, len(lp) - 1,
-            _ptr(P), _ptr(self.root_distn), obs.kind, _ptr(obs.data), _ptr(up['partials']),
-            _ptr(up['status']), _ptr(node_distn), _ptr(W), _ptr(root_post_sum), _stream())
-        _native.check(rc, 'rt_posterior_stats')
+        self._down(obs, prog, 0, obs.n_sites, None, up['partials'], up['status'], node_distn, W,
+                   root_post_sum)
         self._mark('down')
-        up.update(node_distn=node_distn, W=W, root_post_sum=root_post_sum, n_levels=len(lp) - 1)
+        up.update(node_distn=node_distn, W=W, root_post_sum=root_post_sum,
+                  n_levels=len(prog['level_ptr']) - 1)
         return up
+
+    def _edge_rates(self):
+        """Q_b for every node b: [n, S, S]."""
+        n, S = self.sched.n, self.S
+        return self.Q[0].expand(n, S, S) if self.q_index is None else self.Q[self.q_index.long()]
+
+    def _frechet(self, Q, W, M):
+        """M[b] = L(t_b Q_b^T, t_b W[b]) for every node b, Q_b = Q[q_index[b]]."""
+        rc = _native.lib().rt_frechet_contract(_ptr(Q), _ptr(self.q_index), _ptr(self.length), _ptr(W),
+                                               self.sched.n, self.S, _ptr(M), _stream())
+        _native.check(rc, 'rt_frechet_contract')
+        return M
 
     def transition_kernels(self, E=None):
         """K_b = L(t_b Q_b, t_b (E o Q_b)) for every edge: K_b[a, c] = expected number of E-type
         transitions on the branch jointly with the end state c, from the start state a
         (the Frechet-derivative form of examples/code2x3/extras.py:108-129)."""
         n, S = self.sched.n, self.S
-        Qe = self.Q[0].expand(n, S, S) if self.q_index is None else self.Q[self.q_index.long()]
         off = 1.0 - torch.eye(S, dtype=torch.float64, device=self.device)
         if E is None:
             Et = off
         else:
             Et = torch.as_tensor(np.asarray(E, dtype=np.float64), device=self.device) * off
-        C = (Qe * Et).contiguous()
-        Qt = self.Q.transpose(1, 2).contiguous()
+        C = (self._edge_rates() * Et).contiguous()
         K = torch.empty((n, S, S), dtype=torch.float64, device=self.device)
-        rc = _native.lib().rt_frechet_contract(_ptr(Qt), _ptr(self.q_index), _ptr(self.length),
-                                               _ptr(C), n, S, _ptr(K), _stream())
-        _native.check(rc, 'rt_frechet_contract')
+        self._frechet(self.Q.transpose(1, 2).contiguous(), C, K)
         K[0].zero_()
         return K
 
@@ -422,14 +438,7 @@ class TreeMJP(object):
         W = self._buf('W', (self.sched.n, self.S, self.S), torch.float64, zero=True)
         rps = self._buf('root_post_sum', (self.S,), torch.float64, zero=True)
         branch = torch.zeros((self.sched.n, stride), dtype=torch.float64, device=self.device)
-        lp = prog['level_ptr']
-        rc = _native.lib().rt_posterior_branch_stats(
-            self.S, self.sched.n, N, stride, _ptr(prog['ops']), prog['n_ops'], prog['n_slots'],
-            _ptr(prog['edges']), lp.ctypes.data, len(lp) - 1,
-            _ptr(self.transition_matrices()), _ptr(self.root_distn), obs.kind, _ptr(obs.data),
-            _ptr(up['partials']), _ptr(up['status']), _ptr(node_distn), _ptr(W), _ptr(rps),
-            _ptr(K), _ptr(branch), _stream())
-        _native.check(rc, 'rt_posterior_branch_stats')
+        self._down(obs, prog, 0, N, None, up['partials'], up['status'], node_distn, W, rps, K, branch)
         return dict(branch=branch[:, :N], loglik=up['loglik'], status=up['status'], W=W,
                     root_post_sum=rps, K=K)
 
@@ -445,13 +454,7 @@ class TreeMJP(object):
         node_distn = self._buf('node_distn', (self.sched.n_store, self.S, stride), torch.float64)
         W = self._buf('W', (self.sched.n, self.S, self.S), torch.float64, zero=True)
         root_post_sum = self._buf('root_post_sum', (self.S,), torch.float64, zero=True)
-        lp = prog['level_ptr']
-        rc = _native.lib().rt_posterior_stats(
-            self.S, self.sched.n, N, stride, _ptr(prog['ops']), prog['n_ops'], prog['n_slots'],
-            _ptr(prog['edges']), lp.ctypes.data, len(lp) - 1,
-            _ptr(self.transition_matrices()), _ptr(self.root_distn), obs.kind, _ptr(obs.data),
-            _ptr(partials), _ptr(status), _ptr(node_distn), _ptr(W), _ptr(root_post_sum), _stream())
-        _native.check(rc, 'rt_posterior_stats')
+        self._down(obs, prog, 0, N, None, partials, status, node_distn, W, root_post_sum)
         return dict(partials=partials, status=status, node_distn=node_distn, W=W,
                     root_post_sum=root_post_sum)
 
@@ -477,87 +480,27 @@ class TreeMJP(object):
         pinned memory in, per-site log-likelihoods / status into pinned `out_*`, summed
         statistics returned.  The site axis is cut into `n_chunks` chunks; the H2D copy
         of chunk k+1 and the D2H copy of chunk k-1 run on their own streams under the
-        kernels of chunk k (sites are independent, W only accumulates)."""
-        lib = _native.lib()
-        L, NB = codes_pinned.shape
+        kernels of chunk k (sites are independent, W only accumulates; see _chunked)."""
         # packed=True: codes_pinned is RT_OBS_CODES4 (pack_codes4), N = len(out_loglik) sites
-        N = int(out_loglik.shape[0]) if packed else NB
-        kind = OBS_CODES4 if packed else OBS_CODES
-        bps = 2 if packed else 1                      # sites per byte of the code rows
-        S, n = self.S, self.sched.n
-        dev = self.device
-        leaf_nodes = self.sched.leaves if leaf_nodes is None else np.asarray(leaf_nodes)
-        obs_slot = np.full(n, -1, dtype=np.int32)
-        obs_slot[leaf_nodes] = np.arange(len(leaf_nodes), dtype=np.int32)
-        codes_dev = self._buf('h_codes%d' % bps, (L, NB), torch.uint8)
-        loglik = self._buf('h_loglik', (N,), torch.float64)
-        status = self._buf('h_status', (N,), torch.int8)
-        partials = self._buf('partials', (self.sched.n_store, S, N), torch.float64)
-        W = self._buf('W', (n, S, S), torch.float64, zero=True)
-        rps = self._buf('root_post_sum', (S,), torch.float64, zero=True)
-        llsum = self._buf('h_llsum', (1,), torch.float64, zero=True)
-        obs = Observations(kind, codes_dev, obs_slot, N)
-        prog = self._programs(obs)
-        lp = prog['level_ptr']
-        P = self.transition_matrices()
-        cur = torch.cuda.current_stream()
-        if getattr(self, '_copy_streams', None) is None:
-            self._copy_streams = (torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev))
-            self._compute_streams = tuple(torch.cuda.Stream(device=dev) for _ in range(E2E_STREAMS))
-        s_in, s_out = self._copy_streams
-        s_in.wait_stream(cur)
-        s_out.wait_stream(cur)
-        for cs in self._compute_streams:
-            cs.wait_stream(cur)
-        chunk = _round_up((N + n_chunks - 1) // n_chunks, 128)
-        bounds = [(lo, min(N, lo + chunk)) for lo in range(0, N, chunk)]
-        ev_in = []
-        for lo, hi in bounds:
-            rc = lib.rt_copy2d_async(codes_dev.data_ptr() + lo // bps, NB,
-                                     codes_pinned.data_ptr() + lo // bps, NB,
-                                     (hi - lo + bps - 1) // bps, L, 1, s_in.cuda_stream)
-            _native.check(rc, 'rt_copy2d_async')
-            e = torch.cuda.Event()
-            e.record(s_in)
-            ev_in.append(e)
-        for k, ((lo, hi), e) in enumerate(zip(bounds, ev_in)):
-            cs = self._compute_streams[k % len(self._compute_streams)]
-            cs.wait_event(e)
-            rc = lib.rt_prune_loglik(
-                S, n, hi - lo, N, _ptr(prog['ops']), prog['n_ops'], prog['n_slots'], _ptr(P),
-                _ptr(self.root_distn), kind, codes_dev.data_ptr() + lo // bps,
-                partials.data_ptr() + 8 * lo, None, loglik.data_ptr() + 8 * lo,
-                status.data_ptr() + lo, _ptr(llsum), cs.cuda_stream)
-            _native.check(rc, 'rt_prune_loglik')
-            rc = lib.rt_posterior_stats(
-                S, n, hi - lo, N, _ptr(prog['ops']), prog['n_ops'], prog['n_slots'],
-                _ptr(prog['edges']), lp.ctypes.data, len(lp) - 1, _ptr(P), _ptr(self.root_distn),
-                kind, codes_dev.data_ptr() + lo // bps, partials.data_ptr() + 8 * lo,
-                status.data_ptr() + lo, None, _ptr(W), _ptr(rps), cs.cuda_stream)
-            _native.check(rc, 'rt_posterior_stats')
-            done = torch.cuda.Event()
-            done.record(cs)
-            with torch.cuda.stream(s_out):
-                s_out.wait_event(done)
-                out_loglik[lo:hi].copy_(loglik[lo:hi], non_blocking=True)
-                out_status[lo:hi].copy_(status[lo:hi], non_blocking=True)
-        for cs in self._compute_streams:
-            cur.wait_stream(cs)
-        M, dwell, trans = self.history_statistics(W)
-        cur.wait_stream(s_out)
-        return dict(loglik_sum=llsum[0], dwell=dwell, trans=trans, root_post_sum=rps, M_edges=M)
+        N = int(out_loglik.shape[0]) if packed else codes_pinned.shape[1]
+        codes_dev = self._buf('h_codes', tuple(codes_pinned.shape), torch.uint8)
+        obs = Observations(OBS_CODES4 if packed else OBS_CODES, codes_dev,
+                           _obs_slot(self.sched, leaf_nodes), N)
+        r = self._chunked(obs, n_chunks, codes_pinned, out_loglik, out_status)
+        M, dwell, trans = self.history_statistics(r['W'])
+        torch.cuda.current_stream().wait_stream(self._streams[1])    # the D2H copies
+        return dict(loglik_sum=r['loglik_sum'], dwell=dwell, trans=trans,
+                    root_post_sum=r['root_post_sum'], M_edges=M)
 
     def history_statistics(self, W):
         """(M_edges, dwell, trans) from the per-edge weights W: one Frechet contraction per edge
         and the accumulation over edges, one library call (rt_history_statistics;
-        raoteh/sampler/_mjp_dense.py:497-533)."""
+        raoteh/sampler/_mjp_dense.py:497-533), or the same contraction in an eigenbasis of the
+        rate matrix where _eigenbasis gives one."""
+        dec = self._eigenbasis()
+        if dec is not None:
+            return self._history_statistics_spectral(W, dec)
         n, S = self.sched.n, self.S
-        if getattr(self, '_spectral_D', None) is not None and self._P_valid and not self._spectral_dec[3]:
-            return self._history_statistics_spectral(W)
-        # S > 16: when the rate matrix is time-reversible w.r.t. the root distribution, contract
-        # the edge weights in its eigenbasis instead of exponentiating a 2S x 2S block per edge
-        if S > 16 and self._reversible_decomposition() is not None:
-            return self._history_statistics_spectral(W, self._reversible_decomposition())
         M = self._buf('M', (n, S, S), torch.float64)
         dwell = torch.empty(S, dtype=torch.float64, device=self.device)
         trans = torch.empty((S, S), dtype=torch.float64, device=self.device)
@@ -567,37 +510,43 @@ class TreeMJP(object):
         _native.check(rc, 'rt_history_statistics')
         return M, dwell, trans
 
+    def _eigenbasis(self):
+        """(A, lam, B) for history_statistics, or None (Pade): the use_spectral decomposition when
+        no state has zero weight; otherwise, for S > 16, the decomposition of a rate matrix that is
+        time-reversible w.r.t. the root distribution, so that the edge weights are contracted in
+        its eigenbasis instead of exponentiating a 2S x 2S block per edge."""
+        D = self._spectral_D
+        if D is not None and self._P_valid and not (D == 0).any():
+            return self._spectral_dec
+        if self.S > 16:
+            return self._reversible_decomposition()
+        return None
+
     def _reversible_decomposition(self):
         """(A, lam, B) on the device if the (single) rate matrix is time-reversible with respect to
         the root distribution and every state has positive weight, else None; cached per rate
         matrix.  Used for the Frechet contraction of large state spaces (codon models are
         reversible): the check is S^2 host work, the symmetric eigenproblem ~0.5 ms at S = 61."""
         key = hash(self.Q_host.tobytes())
-        hit = getattr(self, '_rev_cache', None)
-        if hit is not None and hit[0] == key:
-            return hit[1]
-        dec = None
-        D = self.root_distn_host
-        if D is not None and self.q_index is None and self.Q_host.shape[0] == 1 and (D > 0).all():
-            from . import qtop
-            try:
-                Sm = qtop.symmetric_factor(self.Q_host[0], D, rtol=1e-10)
-                A, lam, B = qtop.decompose_spectral_v2(Sm, D)
-                to = lambda x: torch.from_numpy(np.ascontiguousarray(x)).to(self.device)
-                dec = (to(A), to(lam), to(B), False)
-            except ValueError:
-                dec = None
-        self._rev_cache = (key, dec)
-        return dec
+        if self._rev_cache is None or self._rev_cache[0] != key:
+            dec = None
+            D = self.root_distn_host
+            if D is not None and self.q_index is None and self.Q_host.shape[0] == 1 and (D > 0).all():
+                try:
+                    dec = self._decompose(D, rtol=1e-10)
+                except ValueError:
+                    pass
+            self._rev_cache = (key, dec)
+        return self._rev_cache[1]
 
-    def _history_statistics_spectral(self, W, dec=None):
+    def _history_statistics_spectral(self, W, dec):
         """The same contraction in the eigenbasis of a time-reversible rate matrix (spectral scheme,
         use_spectral): with Q = A diag(lam) B, B = A^-1 (examples/p53/qtop.py:140-148),
             L(t Q^T, t W) = B^T [Phi(t) o (A^T (t W) B^T)] A^T,
             Phi_ij(t) = (e^{t lam_i} - e^{t lam_j}) / (t (lam_i - lam_j))   (e^{t lam_i} on the diagonal),
         four batched S x S products per edge (plain library GEMMs) instead of the Pade exponential
         of a 2S x 2S block matrix per edge: 0.3 ms instead of 4.0 ms for the 254 edges of C3."""
-        A, lam, B, _ = self._spectral_dec if dec is None else dec
+        A, lam, B = dec
         t = self.length[:, None, None]
         x = lam[None, :, None] * t                 # t lam_i
         y = lam[None, None, :] * t                 # t lam_j
@@ -619,20 +568,15 @@ class TreeMJP(object):
 
     def frechet_contract(self, W):
         """M[b] = L(t_b Q_b^T, t_b W[b]) for every node b (slot 0 -> 0)."""
-        n, S = self.sched.n, self.S
-        M = self._buf('M', (n, S, S), torch.float64)
-        rc = _native.lib().rt_frechet_contract(_ptr(self.Q), _ptr(self.q_index), _ptr(self.length),
-                                               _ptr(W), n, S, _ptr(M), _stream())
-        _native.check(rc, 'rt_frechet_contract')
-        return M
+        return self._frechet(self.Q, W, self._buf('M', (self.sched.n, self.S, self.S), torch.float64))
 
     def expected_history_statistics_graphed(self, obs):
         """expected_history_statistics for a NEW rate matrix (set_rate_matrix) replayed as one
         CUDA graph: batched expm, up pass, down walk, Frechet contraction and the packing of the
         statistics are ~13 small launches, and for a few hundred thousand sites per GPU (strong
         scaling, optimiser loops) the host cannot issue them as fast as the GPU runs them.
-        Captured once per (engine, observations) -- the graph lives on the Observations object like
-        the chunked schedule's -- and replayed afterwards; the H2D copy of the rate matrix stays
+        Captured once per (engine, observations) -- the graph lives on the Observations object --
+        and replayed afterwards; the H2D copy of the rate matrix stays
         outside (stream ordered before the replay).  Returns the same dict (static tensors, valid
         until the next call) plus 'stats' = the packed [1 + S + S*S + S] vector for the allreduce.
         Falls back to the eager path if the capture is refused."""
@@ -642,7 +586,7 @@ class TreeMJP(object):
                _ptr(self.root_distn), prog['ops'].data_ptr())
         entry = cache.get(key)
         if entry is None:
-            if getattr(self, '_graph_refused', False):
+            if self._graph_refused:
                 return self._ehs_with_stats(obs)
             self._P_valid = False
             self._ehs_with_stats(obs)                 # eager once: workspaces, pool growth
@@ -666,8 +610,7 @@ class TreeMJP(object):
 
     def _ehs_with_stats(self, obs):
         r = self.expected_history_statistics(obs)
-        ll_sum = r['loglik_sum'] if 'loglik_sum' in r else r['loglik'].sum()
-        r['stats'] = torch.cat([ll_sum.reshape(1), r['dwell'].reshape(-1), r['trans'].reshape(-1),
+        r['stats'] = torch.cat([r['loglik_sum'].reshape(1), r['dwell'].reshape(-1), r['trans'].reshape(-1),
                                 r['root_post_sum'].reshape(-1)])
         return r
 
@@ -680,10 +623,5 @@ class TreeMJP(object):
         edge, the form of examples/code2x3/extras.py:108-129)."""
         post = self.posterior(obs, want_node_distn=want_node_distn, overlap_chunks=overlap_chunks)
         M, dwell, trans = self.history_statistics(post['W'])
-        S = self.S
-        if self.q_index is None:
-            Qe = self.Q[0].expand(self.sched.n, S, S)
-        else:
-            Qe = self.Q[self.q_index.long()]
-        post.update(dwell=dwell, trans=trans, M_edges=M, Q_edges=Qe)
+        post.update(dwell=dwell, trans=trans, M_edges=M, Q_edges=self._edge_rates())
         return post

@@ -347,16 +347,20 @@ def test_c2_full_size_properties(rt):
 
 
 def test_host_buffer_pipeline_matches_resident_path(rt):
-    """The chunked host-buffer entry point (e2e path of bench.py) gives the same numbers."""
+    """The chunked host-buffer entry point (e2e path of bench.py) gives the same numbers, and so
+    does the same site-chunk pipeline on device-resident observations of every encoding
+    (expected_history_statistics(overlap_chunks=k)), for a site count that is not a multiple of
+    the 128-site chunk granule."""
     import torch
     from raoteh_b200 import synth
-    from raoteh_b200.lowering import TreeSchedule
+    from raoteh_b200.lowering import TreeSchedule, MISSING
     cfg = synth.config_c2(n_sites=10_007, n_leaves=16)
+    keys = ('loglik', 'status', 'dwell', 'trans', 'root_post_sum')
     sched = TreeSchedule(cfg['parent'], cfg['length'])
     mjp = rt.TreeMJP(sched, cfg['Q'], root_distn=cfg['pi'])
     obs = rt.Observations.from_leaf_codes(sched, cfg['codes'], cfg['leaves'])
     ref = mjp.expected_history_statistics(obs)
-    ref = {k: ref[k].clone() for k in ('loglik', 'status', 'dwell', 'trans', 'root_post_sum')}
+    ref = {k: ref[k].clone() for k in keys}
     codes_pinned = torch.from_numpy(cfg['codes']).pin_memory()
     out_ll = torch.empty(10_007, dtype=torch.float64).pin_memory()
     out_st = torch.empty(10_007, dtype=torch.int8).pin_memory()
@@ -367,6 +371,23 @@ def test_host_buffer_pipeline_matches_resident_path(rt):
     np.testing.assert_allclose(r['dwell'].cpu().numpy(), ref['dwell'].cpu().numpy(), rtol=1e-12)
     np.testing.assert_allclose(r['trans'].cpu().numpy(), ref['trans'].cpu().numpy(), rtol=1e-12)
     np.testing.assert_allclose(float(r['loglik_sum']), float(ref['loglik'].sum()), rtol=1e-12)
+
+    S, codes, leaves = cfg['S'], cfg['codes'], cfg['leaves']
+    assert (codes == MISSING).any()
+    allowed = (codes[:, None, :] == np.arange(S)[None, :, None]) | (codes == MISSING)[:, None, :]
+    mask = np.full((sched.n, codes.shape[1]), (1 << S) - 1, dtype=np.uint64)
+    mask[leaves] = (allowed.astype(np.uint64) << np.arange(S, dtype=np.uint64)[None, :, None]).sum(axis=1)
+    for obs in (obs, rt.Observations.from_leaf_codes4(sched, codes, leaves),
+                rt.Observations.from_masks(sched, mask),
+                rt.Observations.from_dense(sched, allowed.astype(np.float64), leaves)):
+        ref = mjp.expected_history_statistics(obs)
+        ref = {k: ref[k].clone() for k in keys}
+        for k in (3, 8):
+            r = mjp.expected_history_statistics(obs, overlap_chunks=k)
+            assert torch.equal(r['loglik'], ref['loglik']) and torch.equal(r['status'], ref['status'])
+            for key in ('dwell', 'trans', 'root_post_sum'):
+                np.testing.assert_allclose(r[key].cpu().numpy(), ref[key].cpu().numpy(), rtol=1e-12)
+            np.testing.assert_allclose(float(r['loglik_sum']), float(ref['loglik'].sum()), rtol=1e-12)
 
 
 @pytest.mark.parametrize('S,n_leaves,n_sites', [(4, 9, 70), (6, 6, 33), (20, 5, 37), (61, 6, 150)])
