@@ -303,6 +303,68 @@ typedef struct rt_raoteh_args {
 int rt_raoteh_run(const rt_raoteh_args* args, void* stream);
 
 /*
+ * Exact posterior draws of whole histories (stochastic mapping; Nielsen 2002, Hobolth & Stone
+ * 2009), one per trajectory, written in the trajectory layout of rt_raoteh_sweeps above, so that
+ * rt_raoteh_run can continue from them.  The law drawn is the posterior of the MJP history given
+ * the observations of the trajectory's site (site = (traj0 + t) % n_sites) -- the stationary law
+ * of the sweeps, so a chain started from a draw needs no burn-in:
+ *   node states  x_root ~ pi * L_root, then, walking the upward program backwards (parents first),
+ *                x_c ~ P_c[x_a, :] * L_c with L_c the stored partial (OP_MSG_SLOT, store index =
+ *                op field 3), the observation (OP_MSG_OBS) or ones (OP_MSG_ONES): the tree form of
+ *                _sample_mc0.resample_states (raoteh/sampler/_sample_mc0.py:20);
+ *   branch paths given (x_a, x_c, t_c), by uniformization with mu = max_s q_s, B = I + Q/mu:
+ *                Pr(N = n) ~ Pois(n; mu t_c) (B^n)[x_a, x_c], intermediate states
+ *                Pr(x_i = s) ~ B[x_{i-1}, s] (B^{N-i})[s, x_c], event times the order statistics
+ *                of N uniforms on (0, t_c); only the state changes are stored, strictly inside
+ *                (0, t_c) and strictly increasing in the stored precision.
+ * It replaces the arbitrary initial history of _sampler.get_restricted_feasible_history
+ * (raoteh/sampler/_sampler.py:563), which the sweeps must then forget.
+ *
+ * S in 2..8, observations RT_OBS_CODES or RT_OBS_MASK, fp64 event times (time_f64) except at
+ * S = 7 (whose sweeps take float times only).  Inputs: program/parent/length as for the sweeps,
+ * Q [S][S] with diagonal, P [n_nodes][S][S] = expm(t_b Q) (rt_expm_batched), partials and
+ * site_status [n_sites] from rt_prune_loglik (site_stride = their row length), root_distn nullable.
+ * The powers B^0..B^n_pow are built in a workspace, n_pow from the Poisson tail at
+ * mu * max_b t_b, at most 320: a branch with mu * t_c beyond ~200 cannot be drawn (status 3;
+ * subdivide it with degree-two nodes).
+ * Philox4x32-10 keyed by (seed; traj0 + t, k): k is the draw's index in the chain's sweep
+ * numbering (the draw uses its own substream, so a sweep with the same index draws other words);
+ * results do not depend on how trajectories are split over launches or GPUs.
+ * Outputs: the trajectory arrays; sweep_count (nullable) = k + 1 where the draw succeeded;
+ * dwell_sum [S] / trans_sum [S*S] (nullable) += the statistics of the drawn histories.
+ * status [traj_stride]: trajectories with status != 0 on entry are skipped; a trajectory whose
+ * site has status != 0 gets that status; 1 = no feasible history, 3 = more than 255 real jumps on
+ * a branch, a branch too long for the power table, or a jump time that cannot be stored,
+ * 4 = more than `cap` real jumps in the trajectory (ev_total is then 0).
+ */
+typedef struct rt_posterior_draw_args {
+  int32_t S, n_nodes, n_ops, cap, obs_kind, time_f64;
+  int64_t n_traj, traj_stride, n_sites, traj0, obs_stride, site_stride;
+  uint64_t seed;
+  int64_t k;
+  const int32_t* program;
+  const int32_t* parent;
+  const double* length;
+  const double* Q;
+  const double* P;
+  const double* root_distn;
+  const void* obs;
+  const double* partials;
+  const int8_t* site_status;
+  uint8_t* node_state;
+  void* ev_time;
+  uint8_t* ev_sb;
+  uint8_t* ev_count;
+  int32_t* ev_total;
+  int32_t* sweep_count;
+  double* dwell_sum;
+  double* trans_sum;
+  int8_t* status;
+} rt_posterior_draw_args;
+
+int rt_posterior_draw(const rt_posterior_draw_args* args, void* stream);
+
+/*
  * Warp-cooperative Rao-Teh kernels: one warp per (chain, site) trajectory.
  *
  * (1) Rao-Teh sweeps for S = 7 and 9 <= S <= 64 primary states (rt_raoteh_sweeps dispatches

@@ -103,6 +103,26 @@ class TmjpArgs(ctypes.Structure):
 EXPORTS['rt_tmjp_run'] = ([ctypes.POINTER(TmjpArgs), c_void_p], c_int)
 
 
+class PosteriorDrawArgs(ctypes.Structure):
+    """Mirror of `rt_posterior_draw_args` (include/rt_b200.h)."""
+    _fields_ = [
+        ('S', ctypes.c_int32), ('n_nodes', ctypes.c_int32), ('n_ops', ctypes.c_int32),
+        ('cap', ctypes.c_int32), ('obs_kind', ctypes.c_int32), ('time_f64', ctypes.c_int32),
+        ('n_traj', c_int64), ('traj_stride', c_int64), ('n_sites', c_int64), ('traj0', c_int64),
+        ('obs_stride', c_int64), ('site_stride', c_int64),
+        ('seed', ctypes.c_uint64), ('k', c_int64),
+        ('program', c_void_p), ('parent', c_void_p), ('length', c_void_p), ('Q', c_void_p),
+        ('P', c_void_p), ('root_distn', c_void_p), ('obs', c_void_p), ('partials', c_void_p),
+        ('site_status', c_void_p),
+        ('node_state', c_void_p), ('ev_time', c_void_p), ('ev_sb', c_void_p),
+        ('ev_count', c_void_p), ('ev_total', c_void_p), ('sweep_count', c_void_p),
+        ('dwell_sum', c_void_p), ('trans_sum', c_void_p), ('status', c_void_p),
+    ]
+
+
+EXPORTS['rt_posterior_draw'] = ([ctypes.POINTER(PosteriorDrawArgs), c_void_p], c_int)
+
+
 class NativeError(RuntimeError):
     pass
 

@@ -87,9 +87,11 @@ int rt_raoteh_dispatch(const rt_raoteh_args&, cudaStream_t);
 
 int rt_tmjp_dispatch(const rt_tmjp_args&, cudaStream_t);
 
+int rt_posterior_draw_dispatch(const rt_posterior_draw_args&, cudaStream_t);
+
 extern "C" {
 
-int rt_version(void) { return 201; }
+int rt_version(void) { return 202; }
 
 int rt_release_workspace(void) {
   int dev = 0;
@@ -319,6 +321,26 @@ int rt_raoteh_sweeps(int S, int n_nodes, int64_t n_traj, int64_t traj_stride, in
   R.ev_sb = ev_sb; R.ev_count = ev_count; R.ev_total = ev_total;
   R.dwell_sum = dwell_sum; R.trans_sum = trans_sum; R.status = status;
   return raoteh_run_impl(R, stream);
+}
+
+int rt_posterior_draw(const rt_posterior_draw_args* args, void* stream) {
+  if (!args) return arg_error("null pointer");
+  const rt_posterior_draw_args& R = *args;
+  if (!R.program || !R.parent || !R.length || !R.Q || !R.P || !R.obs || !R.partials ||
+      !R.node_state || !R.ev_time || !R.ev_sb || !R.ev_count || !R.ev_total || !R.status)
+    return arg_error("null pointer");
+  if ((R.dwell_sum == nullptr) != (R.trans_sum == nullptr)) return arg_error("dwell_sum and trans_sum go together");
+  if (R.obs_kind != 0 && R.obs_kind != 1) return arg_error("rt_posterior_draw takes codes or masks");
+  if (R.S < 2 || R.S > 8) return unsupported("rt_posterior_draw needs 2 <= S <= 8");
+  if (R.time_f64 && R.S == 7) return unsupported("fp64 event times: S in {2,3,4,5,6,8} only");
+  if (R.traj_stride < R.n_traj || R.n_sites <= 0 || R.cap <= 0) return arg_error("sizes");
+  if (R.site_stride < R.n_sites) return arg_error("site_stride < n_sites");
+  if (R.k < 0 || R.k >= INT32_MAX) return arg_error("draw index k out of range");
+  if (R.n_ops <= 0 || R.n_nodes <= 1) return arg_error("empty program");
+  if (R.n_traj <= 0) return RT_OK;
+  int rc = rt_posterior_draw_dispatch(R, (cudaStream_t)stream);
+  if (rc == RT_ERR_UNSUPPORTED) snprintf(g_err, sizeof(g_err), "unsupported: S or shared-memory budget");
+  return rc;
 }
 
 }  // extern "C"

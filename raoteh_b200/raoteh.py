@@ -16,6 +16,29 @@ from . import _native
 from .engine import OBS_CODES, OBS_MASK, _ptr, _stream
 
 
+# longest table of powers B^0..B^n of rt_posterior_draw (csrc/rt_posterior_draw.cu, kMaxPow)
+DRAW_MAX_POW = 320
+
+
+def draw_power_table_length(Q, length, eps=1e-17):
+    """n such that the Poisson tail beyond n at mu * max_b t_b (mu = max_s q_s) is below eps: the
+    length of the table of powers B^n the exact draw needs (the kernel's own rule, before its cap)."""
+    import math
+    Q = np.asarray(Q, dtype=np.float64)
+    mu = float((-np.diag(Q)).max())
+    if not mu > 0:
+        mu = 1.0
+    lam = mu * float(np.max(length[1:])) if len(length) > 1 else 0.0
+    n = int(math.ceil(lam))
+    while n < 4 * DRAW_MAX_POW:
+        r = lam / (n + 1)
+        logp = (-lam + n * math.log(lam) - math.lgamma(n + 1.0)) if lam > 0 else (0.0 if n == 0 else -math.inf)
+        if r < 1.0 and math.exp(logp) * r / (1.0 - r) < eps:
+            break
+        n += 1
+    return max(n, 2 * Q.shape[0] + 8)
+
+
 class RaoTehChains(object):
     """n_chains x n_sites trajectories of one MJP on one tree.
 
@@ -73,6 +96,9 @@ class RaoTehChains(object):
         if chain_matrix is not None:
             B, rate, self.omega = Bc, np.zeros(S), 1.0
         self.Q_host = Q
+        self._chain_matrix = chain_matrix is not None
+        self._root_distn_host = None if root_distn is None else np.asarray(root_distn, dtype=np.float64)
+        self._draw_inputs = None       # (TreeMJP, P, partials, site status) of draw_posterior
         self.B = torch.from_numpy(np.ascontiguousarray(B)).to(dev)
         self.rate = torch.from_numpy(np.ascontiguousarray(rate)).to(dev)
         self.root_distn = None if root_distn is None else torch.from_numpy(
@@ -162,6 +188,58 @@ class RaoTehChains(object):
                 self._call(int(n_sweeps), -1, stats)
                 tries += 1
         self.sweeps_done += int(n_sweeps)
+        self.check()
+
+    def draw_posterior(self, stats=True):
+        """Replace every trajectory with an independent exact draw from the posterior over histories
+        given its site's observations (rt_posterior_draw: node states top-down from the pruning
+        partials, then a path on every branch given its end states by uniformization).  The draw
+        takes sweep index k = sweeps_done, as a sweep would, so
+
+          - called instead of initialize(), the chains start at stationarity: no burn-in is needed
+            before the sweeps' statistics are unbiased;
+          - called repeatedly, it is an iid Monte Carlo sampler whose statistics accumulate in
+            dwell_sum / trans_sum (stats=True) exactly like those of sweeps.
+
+        Thread-per-trajectory kernel: 2..8 states; not for chain_matrix chains (no rate matrix)."""
+        import ctypes
+        from .engine import TreeMJP
+        if self._chain_matrix:
+            raise ValueError('draw_posterior needs a rate matrix; chain_matrix chains have none')
+        if self.S > 8:
+            raise ValueError('draw_posterior supports 2..8 states')
+        n_pow = draw_power_table_length(self.Q_host, self.sched.length)
+        if n_pow > DRAW_MAX_POW:
+            raise ValueError(
+                'a branch is too long for the exact draw: max_s q_s * length = %.0f needs B^n up to '
+                'n = %d, more than %d; subdivide long branches with degree-two nodes '
+                '(lowering.subdivide_long_branches)'
+                % (float(-np.diag(self.Q_host).min()) * float(self.sched.length.max()), n_pow, DRAW_MAX_POW))
+        if self._draw_inputs is None:
+            # P and the pruning partials depend on Q and the observations only, both fixed here
+            mjp = TreeMJP(self.sched, self.Q_host, root_distn=self._root_distn_host, device=self.device)
+            P = mjp.transition_matrices()
+            up = mjp.log_likelihood(self.obs, keep_partials=True)
+            self._draw_inputs = (mjp, P, up['partials'], up['status'])
+        mjp, P, partials, site_status = self._draw_inputs
+        self.status.zero_()
+        A = _native.PosteriorDrawArgs()
+        A.S, A.n_nodes, A.n_ops, A.cap = self.S, self.sched.n, self.n_ops, self.cap
+        A.obs_kind, A.time_f64 = self.obs.kind, 1 if self.time_dtype == 'float64' else 0
+        A.n_traj, A.traj_stride, A.n_sites, A.traj0 = self.n_traj, self.stride, self.n_sites, self.traj0
+        A.obs_stride, A.site_stride = self.obs.stride, self.obs.stride
+        A.seed, A.k = self.seed, self.sweeps_done
+        A.program, A.parent, A.length = _ptr(self.ops), _ptr(self.parent), _ptr(self.length)
+        A.Q, A.P, A.root_distn = _ptr(mjp.Q), _ptr(P), _ptr(self.root_distn)
+        A.obs, A.partials, A.site_status = _ptr(self.obs.data), _ptr(partials), _ptr(site_status)
+        A.node_state, A.ev_time, A.ev_sb = _ptr(self.node_state), _ptr(self.ev_time), _ptr(self.ev_sb)
+        A.ev_count, A.ev_total, A.sweep_count = _ptr(self.ev_count), _ptr(self.ev_total), _ptr(self.sweep_count)
+        A.dwell_sum = _ptr(self.dwell_sum) if stats else None
+        A.trans_sum = _ptr(self.trans_sum) if stats else None
+        A.status = _ptr(self.status)
+        _native.check(_native.lib().rt_posterior_draw(ctypes.byref(A), _stream()), 'rt_posterior_draw')
+        self.sweeps_done += 1
+        self.initialized = True
         self.check()
 
     def grow(self, cap):
