@@ -25,7 +25,7 @@ constexpr int kSitesPerCta = 2048;
 
 template <int S>
 __global__ void __launch_bounds__(kBlock)
-root_distn_kernel(int64_t n_sites, int64_t stride, const double* __restrict__ root_distn,
+root_distn_kernel(int64_t n_sites, int64_t stride, int64_t nd_stride, const double* __restrict__ root_distn,
                   const double* __restrict__ partials, const int8_t* __restrict__ status,
                   double* __restrict__ node_distn, double* __restrict__ root_post_sum) {
   __shared__ double red[kBlock / 32][S];
@@ -37,7 +37,7 @@ root_distn_kernel(int64_t n_sites, int64_t stride, const double* __restrict__ ro
        site += (int64_t)gridDim.x * kBlock) {
     if (status[site] != RT_SITE_OK) {
 #pragma unroll
-      for (int s = 0; s < S; ++s) node_distn[(int64_t)s * stride + site] = 0.0;
+      for (int s = 0; s < S; ++s) node_distn[(int64_t)s * nd_stride + site] = 0.0;
       continue;
     }
     double w[S];
@@ -51,7 +51,7 @@ root_distn_kernel(int64_t n_sites, int64_t stride, const double* __restrict__ ro
 #pragma unroll
     for (int s = 0; s < S; ++s) {
       const double d = w[s] * inv;
-      node_distn[(int64_t)s * stride + site] = d;
+      node_distn[(int64_t)s * nd_stride + site] = d;
       sum[s] += d;
     }
   }
@@ -70,18 +70,23 @@ root_distn_kernel(int64_t n_sites, int64_t stride, const double* __restrict__ ro
   }
 }
 
-template <int S, int OBS>
-__global__ void __launch_bounds__(kBlock, (S <= 4 ? 2 : 1))
-down_level_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ edges,
+// PACKED: RT_OBS_CODES4 leaf codes.  BR: also the per-site branch expectation of the walk's BR.
+// Node marginals are indexed with their own site stride (a workspace holds only this chunk).
+template <int S, int OBS, bool BR, bool PACKED>
+__global__ void __launch_bounds__(kBlock)
+down_level_kernel(int64_t n_sites, int64_t stride, int64_t nd_stride, const int4* __restrict__ edges,
                   const double* __restrict__ P, const void* __restrict__ obs,
                   const double* __restrict__ partials, const int8_t* __restrict__ status,
-                  double* __restrict__ node_distn, double* __restrict__ W) {
+                  double* __restrict__ node_distn, double* __restrict__ W,
+                  const double* __restrict__ Kmat, double* __restrict__ branch_out) {
   __shared__ double Ps[S * S];
+  __shared__ double Ks[BR ? S * S : 1];
   __shared__ double red[kBlock / 32][S * S];
   const int tid = threadIdx.x;
   const int4 e = edges[blockIdx.y];   // (child node, parent store, child store, child obs slot)
   const int b = e.x;
   if (tid < S * S) Ps[tid] = P[(size_t)b * S * S + tid];
+  if (BR && tid < S * S) Ks[tid] = Kmat[(size_t)b * S * S + tid];
   __syncthreads();
 
   double Wacc[S][S];
@@ -90,9 +95,9 @@ down_level_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ edge
 #pragma unroll
     for (int j = 0; j < S; ++j) Wacc[i][j] = 0.0;
 
-  const double* Dp = node_distn + (int64_t)e.y * S * stride;
+  const double* Dp = node_distn + (int64_t)e.y * S * nd_stride;
   const double* Lc = e.z >= 0 ? partials + (int64_t)e.z * S * stride : nullptr;
-  double* Dc = e.z >= 0 ? node_distn + (int64_t)e.z * S * stride : nullptr;
+  double* Dc = e.z >= 0 ? node_distn + (int64_t)e.z * S * nd_stride : nullptr;
 
   const int64_t lo = (int64_t)blockIdx.x * kSitesPerCta;
   const int64_t hi = (n_sites < lo + kSitesPerCta) ? n_sites : lo + kSitesPerCta;
@@ -113,7 +118,14 @@ down_level_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ edge
 #pragma unroll
       for (int s = 0; s < S; ++s) L[s] = 1.0;
     } else if (OBS == OBS_CODES) {
-      const int k = reinterpret_cast<const uint8_t*>(obs)[(int64_t)e.w * stride + site];
+      const uint8_t* row = reinterpret_cast<const uint8_t*>(obs);
+      int k;
+      if (PACKED) {      // nibble site & 1 of byte site >> 1, 15 = unobserved
+        k = (row[(int64_t)e.w * ((stride + 1) >> 1) + (site >> 1)] >> ((int)(site & 1) * 4)) & 15;
+        if (k == 15) k = RT_MISSING;
+      } else {
+        k = row[(int64_t)e.w * stride + site];
+      }
 #pragma unroll
       for (int s = 0; s < S; ++s) L[s] = (k == RT_MISSING || k == s) ? 1.0 : 0.0;
     } else if (OBS == OBS_MASK) {
@@ -127,23 +139,38 @@ down_level_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ edge
       for (int s = 0; s < S; ++s) L[s] = d[((int64_t)e.w * S + s) * stride + site];
     }
 #pragma unroll
-    for (int s = 0; s < S; ++s) D[s] = Dp[(int64_t)s * stride + site];
+    for (int s = 0; s < S; ++s) D[s] = Dp[(int64_t)s * nd_stride + site];
   };
 
+  // P_b is re-read from shared memory at every use from S = 7 on: kept in registers across the
+  // site loop (S * S values), it and the S x S accumulator would not fit in 255 registers
+  auto p_at = [&](int i) -> double {
+    if constexpr (S >= 7) return reinterpret_cast<volatile const double*>(Ps)[i];
+    else return Ps[i];
+  };
+  // the next site's loads are issued before the current site is computed up to S = 5; from S = 6
+  // on, their 2 S registers next to the S x S accumulator would spill
+  constexpr bool kPrefetch = S <= 5;
   double Ln[S], Dn[S];
-  bool okn;
-  load_site(lo + tid, Ln, Dn, okn);
+  bool okn = false;
+  if (kPrefetch) load_site(lo + tid, Ln, Dn, okn);
   for (int64_t site = lo + tid; site < hi; site += kBlock) {
     double L[S], D[S];
-    const bool ok = okn;
+    bool ok;
+    if (kPrefetch) {
+      ok = okn;
 #pragma unroll
-    for (int s = 0; s < S; ++s) { L[s] = Ln[s]; D[s] = Dn[s]; }
-    load_site(site + kBlock, Ln, Dn, okn);
+      for (int s = 0; s < S; ++s) { L[s] = Ln[s]; D[s] = Dn[s]; }
+      load_site(site + kBlock, Ln, Dn, okn);
+    } else {
+      load_site(site, L, D, ok);
+    }
     if (!ok) {
       if (Dc) {
 #pragma unroll
-        for (int s = 0; s < S; ++s) Dc[(int64_t)s * stride + site] = 0.0;
+        for (int s = 0; s < S; ++s) Dc[(int64_t)s * nd_stride + site] = 0.0;
       }
+      if (BR) branch_out[(int64_t)b * stride + site] = 0.0;
       continue;
     }
     double G[S];
@@ -151,7 +178,7 @@ down_level_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ edge
     for (int a = 0; a < S; ++a) {
       double m = 0.0;
 #pragma unroll
-      for (int c = 0; c < S; ++c) m = fma(Ps[a * S + c], L[c], m);
+      for (int c = 0; c < S; ++c) m = fma(p_at(a * S + c), L[c], m);
       G[a] = (D[a] > 0.0) ? D[a] / m : 0.0;
     }
     if (Dc) {
@@ -159,9 +186,20 @@ down_level_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ edge
       for (int c = 0; c < S; ++c) {
         double t = 0.0;
 #pragma unroll
-        for (int a = 0; a < S; ++a) t = fma(G[a], Ps[a * S + c], t);
-        Dc[(int64_t)c * stride + site] = t * L[c];
+        for (int a = 0; a < S; ++a) t = fma(G[a], p_at(a * S + c), t);
+        Dc[(int64_t)c * nd_stride + site] = t * L[c];
       }
+    }
+    if (BR) {
+      double x = 0.0;
+#pragma unroll
+      for (int a = 0; a < S; ++a) {
+        double kl = 0.0;
+#pragma unroll
+        for (int c = 0; c < S; ++c) kl = fma(Ks[a * S + c], L[c], kl);
+        x = fma(G[a], kl, x);
+      }
+      branch_out[(int64_t)b * stride + site] = x;
     }
 #pragma unroll
     for (int a = 0; a < S; ++a)
@@ -181,6 +219,22 @@ down_level_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ edge
     double t = 0.0;
     for (int i = 0; i < kBlock / 32; ++i) t += red[i][tid];
     if (Ps[tid] > 0.0 && t != 0.0) atomicAdd(&W[(size_t)b * S * S + tid], t);
+  }
+}
+
+template <int S, int OBS, bool BR, bool PACKED>
+void launch_levels(int64_t n_sites, int64_t stride, int64_t nd_stride, const int4* edges,
+                   const int32_t* level_ptr_h, int n_levels, const double* P, const void* obs,
+                   const double* partials, const int8_t* status, double* node_distn, double* W,
+                   const double* Kmat, double* branch_out, cudaStream_t stream) {
+  const unsigned gx = (unsigned)((n_sites + kSitesPerCta - 1) / kSitesPerCta);
+  for (int l = 0; l < n_levels; ++l) {
+    const int e0 = level_ptr_h[l], e1 = level_ptr_h[l + 1];
+    if (e1 <= e0) continue;
+    dim3 grid(gx, (unsigned)(e1 - e0));
+    down_level_kernel<S, OBS, BR, PACKED><<<grid, kBlock, 0, stream>>>(
+        n_sites, stride, nd_stride, edges + e0, P, obs, partials, status, node_distn, W, Kmat,
+        branch_out);
   }
 }
 
@@ -696,34 +750,52 @@ int run(int obs_kind, int64_t n_sites, int64_t stride, const int32_t* program, i
 #undef RT_WALK
     if (rc != RT_OK || handled) return rc;
   }
-  if (branch_out || obs_kind == 3) return RT_ERR_UNSUPPORTED;   // walk-kernel-only features
-  if (!node_distn) return RT_ERR_ARG;   // the level-synchronous kernel needs the marginals buffer
-  int64_t gr = (n_sites + kBlock - 1) / kBlock;
-  int grid_root = (int)(gr < 148 * 8 ? gr : 148 * 8);
-  root_distn_kernel<S><<<grid_root, kBlock, 0, stream>>>(n_sites, stride, root_distn, partials,
-                                                         status, node_distn, root_post_sum);
-  const int4* edges = reinterpret_cast<const int4*>(edges_dev);
-  const unsigned gx = (unsigned)((n_sites + kSitesPerCta - 1) / kSitesPerCta);
-  for (int l = 0; l < n_levels; ++l) {
-    const int e0 = level_ptr_h[l], e1 = level_ptr_h[l + 1];
-    if (e1 <= e0) continue;
-    dim3 grid(gx, (unsigned)(e1 - e0));
-    switch (obs_kind) {
-      case OBS_CODES:
-        down_level_kernel<S, OBS_CODES><<<grid, kBlock, 0, stream>>>(
-            n_sites, stride, edges + e0, P, obs, partials, status, node_distn, W);
-        break;
-      case OBS_MASK:
-        down_level_kernel<S, OBS_MASK><<<grid, kBlock, 0, stream>>>(
-            n_sites, stride, edges + e0, P, obs, partials, status, node_distn, W);
-        break;
-      case OBS_DENSE:
-        down_level_kernel<S, OBS_DENSE><<<grid, kBlock, 0, stream>>>(
-            n_sites, stride, edges + e0, P, obs, partials, status, node_distn, W);
-        break;
-      default: return RT_ERR_ARG;
-    }
+  // Level-synchronous kernels: the walk's per-node tables do not fit in shared memory.  They pass
+  // node marginals through global memory; without a caller's buffer the sites go in chunks through
+  // a workspace of kFallbackChunk sites.
+  if (obs_kind < 0 || obs_kind > 3) return RT_ERR_ARG;
+  constexpr int64_t kFallbackChunk = 1 << 16;
+  double* ws = nullptr;
+  if (!node_distn) {
+    // rows = store indices: one per internal node.  The upward program has one message per edge
+    // (n_nodes - 1) and, per internal node, one OP_STORE / OP_ROOT and at most one OP_APPLY_OBS,
+    // so n_ops - (n_nodes - 1) is at least the number of internal nodes and at most twice it
+    int64_t rows = (int64_t)n_ops - (n_nodes - 1);
+    if (rows < 1) rows = 1;
+    if (rows > n_nodes) rows = n_nodes;
+    const int64_t cs = n_sites < kFallbackChunk ? n_sites : kFallbackChunk;
+    RT_CUDA_CHECK(rt_ws_alloc((void**)&ws, sizeof(double) * (size_t)rows * S * cs, stream));
   }
+  const int4* edges = reinterpret_cast<const int4*>(edges_dev);
+  const int64_t step = ws ? kFallbackChunk : n_sites;
+  for (int64_t lo = 0; lo < n_sites; lo += step) {
+    const int64_t n = (n_sites - lo < step) ? n_sites - lo : step;
+    // every per-site array is site-minor: chunk `lo` starts at element lo of each row
+    // (RT_OBS_CODES4 holds two sites per byte, and chunks start at even sites)
+    const void* ob = obs;
+    if (obs_kind == OBS_DENSE) ob = reinterpret_cast<const double*>(obs) + lo;
+    else if (obs_kind == OBS_MASK) ob = reinterpret_cast<const unsigned long long*>(obs) + lo;
+    else if (obs_kind == OBS_CODES) ob = reinterpret_cast<const uint8_t*>(obs) + lo;
+    else ob = reinterpret_cast<const uint8_t*>(obs) + lo / 2;
+    const int64_t nd_stride = ws ? n : stride;
+    double* nd = ws ? ws : node_distn + lo;
+    double* br = branch_out ? branch_out + lo : nullptr;
+    int64_t gr = (n + kBlock - 1) / kBlock;
+    int grid_root = (int)(gr < 148 * 8 ? gr : 148 * 8);
+    root_distn_kernel<S><<<grid_root, kBlock, 0, stream>>>(n, stride, nd_stride, root_distn, partials + lo,
+                                                           status + lo, nd, root_post_sum);
+#define RT_LEVELS(OBSK, PACKED)                                                                     \
+  (br ? launch_levels<S, OBSK, true, PACKED>(n, stride, nd_stride, edges, level_ptr_h, n_levels, P, ob, \
+                                             partials + lo, status + lo, nd, W, Kmat, br, stream)     \
+      : launch_levels<S, OBSK, false, PACKED>(n, stride, nd_stride, edges, level_ptr_h, n_levels, P, ob, \
+                                              partials + lo, status + lo, nd, W, nullptr, nullptr, stream))
+    if (obs_kind == OBS_CODES) RT_LEVELS(OBS_CODES, false);
+    else if (obs_kind == 3) RT_LEVELS(OBS_CODES, true);
+    else if (obs_kind == OBS_MASK) RT_LEVELS(OBS_MASK, false);
+    else RT_LEVELS(OBS_DENSE, false);
+#undef RT_LEVELS
+  }
+  if (ws) RT_CUDA_CHECK(rt_ws_free(ws, stream));
   RT_CUDA_CHECK(cudaGetLastError());
   return RT_OK;
 }
