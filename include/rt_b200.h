@@ -176,6 +176,25 @@ int rt_posterior_stats(int S, int n_nodes, int64_t n_sites, int64_t site_stride,
                        double* node_distn, double* W, double* root_post_sum, void* stream);
 
 /*
+ * rt_posterior_stats with one weight per site: the root marginal becomes
+ *   D[root] = w_site * norm(pi * L_root),
+ * and since nothing below the root renormalises, W, root_post_sum and node_distn all carry the
+ * weight (each site contributes w_site times what rt_posterior_stats adds).  A site with weight 0
+ * contributes nothing.  site_weight: device fp64, required, entries [0, n_sites) read (indexed
+ * like status); weights are meant to be non-negative and finite.  Uses: the E-step of site-class mixtures (w = posterior probability
+ * of the class at the site) and site-pattern compression (w = number of alignment columns with
+ * the pattern).
+ */
+int rt_posterior_weighted_stats(int S, int n_nodes, int64_t n_sites, int64_t site_stride,
+                                const int32_t* program, int n_ops, int n_slots,
+                                const int32_t* edges, const int32_t* level_ptr_h, int n_levels,
+                                const double* P, const double* root_distn,
+                                int obs_kind, const void* obs,
+                                const double* partials, const int8_t* status,
+                                double* node_distn, double* W, double* root_post_sum,
+                                const double* site_weight, void* stream);
+
+/*
  * rt_posterior_stats plus, per SITE and BRANCH, the posterior expectation of a statistic
  * given by one S x S kernel per edge:
  *   branch_out[b][site] = sum_ac J_b[a,c] K_b[a,c] / P_b[a,c] = sum_ac G_b[a] K_b[a,c] L_b[c]

@@ -39,6 +39,10 @@ EXPORTS = {
                             c_void_p, c_void_p, c_int, c_void_p,
                             c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                             c_void_p, c_void_p], c_int),
+    'rt_posterior_weighted_stats': ([c_int, c_int, c_int64, c_int64, c_void_p, c_int, c_int,
+                                     c_void_p, c_void_p, c_int, c_void_p,
+                                     c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, c_void_p, c_void_p, c_void_p], c_int),
     'rt_posterior_branch_stats': ([c_int, c_int, c_int64, c_int64, c_void_p, c_int, c_int,
                                    c_void_p, c_void_p, c_int, c_void_p,
                                    c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,

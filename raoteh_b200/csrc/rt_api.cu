@@ -77,11 +77,11 @@ int rt_posterior_small_dispatch(int, int, int64_t, int64_t, const int32_t*, int,
                                 const int32_t*, const int32_t*, int,
                                 const double*, const double*, const void*, const double*,
                                 const int8_t*, double*, double*, double*, const double*, double*,
-                                cudaStream_t);
+                                const double*, cudaStream_t);
 int rt_posterior_dmma_dispatch(int, int, int64_t, int64_t, const int32_t*, const int32_t*, int,
                                const double*, const double*, const void*, const double*,
                                const int8_t*, double*, double*, double*, const double*, double*,
-                               cudaStream_t);
+                               const double*, cudaStream_t);
 
 int rt_raoteh_dispatch(const rt_raoteh_args&, cudaStream_t);
 
@@ -91,7 +91,7 @@ int rt_posterior_draw_dispatch(const rt_posterior_draw_args&, cudaStream_t);
 
 extern "C" {
 
-int rt_version(void) { return 202; }
+int rt_version(void) { return 203; }
 
 int rt_release_workspace(void) {
   int dev = 0;
@@ -199,7 +199,8 @@ static int posterior_common(int S, int n_nodes, int64_t n_sites, int64_t site_st
                             const int32_t* edges, const int32_t* level_ptr_h, int n_levels,
                             const double* P, const double* root_distn, int obs_kind, const void* obs,
                             const double* partials, const int8_t* status, double* node_distn, double* W,
-                            double* root_post_sum, const double* K, double* branch_out, void* stream) {
+                            double* root_post_sum, const double* K, double* branch_out,
+                            const double* site_weight, void* stream) {
   if (!edges || !level_ptr_h || !P || !partials || !status || !W)
     return arg_error("null pointer");
   if (!node_distn && !(S >= 2 && S <= 8 && program))
@@ -208,17 +209,18 @@ static int posterior_common(int S, int n_nodes, int64_t n_sites, int64_t site_st
   if (obs_kind == 3 && !(S >= 2 && S <= 8 && program)) return unsupported("RT_OBS_CODES4 needs 2 <= S <= 8");
   if (site_stride < n_sites) return arg_error("site_stride < n_sites");
   if ((K == nullptr) != (branch_out == nullptr)) return arg_error("K and branch_out go together");
+  if (site_weight && branch_out) return arg_error("site weights with per-branch output");
   if (n_sites <= 0) return RT_OK;
   int rc;
   if (S >= 2 && S <= 8)
     rc = rt_posterior_small_dispatch(S, obs_kind, n_sites, site_stride, program, n_ops, n_slots,
                                      n_nodes, edges, level_ptr_h, n_levels, P, root_distn, obs,
                                      partials, status, node_distn, W, root_post_sum, K, branch_out,
-                                     (cudaStream_t)stream);
+                                     site_weight, (cudaStream_t)stream);
   else if (S >= 1 && S <= 64)
     rc = rt_posterior_dmma_dispatch(S, obs_kind, n_sites, site_stride, edges, level_ptr_h,
                                     n_levels, P, root_distn, obs, partials, status, node_distn, W,
-                                    root_post_sum, K, branch_out, (cudaStream_t)stream);
+                                    root_post_sum, K, branch_out, site_weight, (cudaStream_t)stream);
   else
     return unsupported("rt_posterior_stats needs 1 <= S <= 64");
   if (rc == RT_ERR_UNSUPPORTED) snprintf(g_err, sizeof(g_err), "unsupported: shared-memory budget");
@@ -233,7 +235,20 @@ int rt_posterior_stats(int S, int n_nodes, int64_t n_sites, int64_t site_stride,
                        double* root_post_sum, void* stream) {
   return posterior_common(S, n_nodes, n_sites, site_stride, program, n_ops, n_slots, edges,
                           level_ptr_h, n_levels, P, root_distn, obs_kind, obs, partials, status,
-                          node_distn, W, root_post_sum, nullptr, nullptr, stream);
+                          node_distn, W, root_post_sum, nullptr, nullptr, nullptr, stream);
+}
+
+int rt_posterior_weighted_stats(int S, int n_nodes, int64_t n_sites, int64_t site_stride,
+                                const int32_t* program, int n_ops, int n_slots,
+                                const int32_t* edges, const int32_t* level_ptr_h, int n_levels,
+                                const double* P, const double* root_distn, int obs_kind,
+                                const void* obs, const double* partials, const int8_t* status,
+                                double* node_distn, double* W, double* root_post_sum,
+                                const double* site_weight, void* stream) {
+  if (!site_weight) return arg_error("null pointer");
+  return posterior_common(S, n_nodes, n_sites, site_stride, program, n_ops, n_slots, edges,
+                          level_ptr_h, n_levels, P, root_distn, obs_kind, obs, partials, status,
+                          node_distn, W, root_post_sum, nullptr, nullptr, site_weight, stream);
 }
 
 int rt_posterior_branch_stats(int S, int n_nodes, int64_t n_sites, int64_t site_stride,
@@ -246,7 +261,7 @@ int rt_posterior_branch_stats(int S, int n_nodes, int64_t n_sites, int64_t site_
   if (!K || !branch_out) return arg_error("null pointer");
   return posterior_common(S, n_nodes, n_sites, site_stride, program, n_ops, n_slots, edges,
                           level_ptr_h, n_levels, P, root_distn, obs_kind, obs, partials, status,
-                          node_distn, W, root_post_sum, K, branch_out, stream);
+                          node_distn, W, root_post_sum, K, branch_out, nullptr, stream);
 }
 
 int rt_copy2d_async(void* dst, size_t dst_pitch, const void* src, size_t src_pitch,

@@ -36,10 +36,13 @@ __device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double
                : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
 }
 
+// site_weight (nullable): D[root] = w_site * norm(pi o L_root); the level kernels and the leaf
+// scatter only propagate the root marginal, so W and every marginal of the site carry the weight.
 __global__ void __launch_bounds__(256)
 root_distn_generic_kernel(int S, int64_t n_sites, int64_t stride,
                           const double* __restrict__ root_distn,
                           const double* __restrict__ partials, const int8_t* __restrict__ status,
+                          const double* __restrict__ site_weight,
                           double* __restrict__ node_distn, double* __restrict__ root_post_sum) {
   extern __shared__ double rsum[];   // [S]
   for (int s = threadIdx.x; s < S; s += blockDim.x) rsum[s] = 0.0;
@@ -54,7 +57,7 @@ root_distn_generic_kernel(int S, int64_t n_sites, int64_t stride,
     double tot = 0.0;
     for (int s = 0; s < S; ++s)
       tot += in ? partials[(int64_t)s * stride + site] * (root_distn ? root_distn[s] : 1.0) : 0.0;
-    const double inv = (ok && tot > 0.0) ? 1.0 / tot : 0.0;
+    const double inv = (ok && tot > 0.0) ? (site_weight ? site_weight[site] : 1.0) / tot : 0.0;
     for (int s = 0; s < S; ++s) {
       const double d = in ? partials[(int64_t)s * stride + site] * (root_distn ? root_distn[s] : 1.0) * inv : 0.0;
       if (in) node_distn[(int64_t)s * stride + site] = d;
@@ -559,12 +562,12 @@ int run(int S, int obs_kind, int64_t n_sites, int64_t stride, const int32_t* edg
         const int32_t* level_ptr_h, int n_levels, const double* P, const double* root_distn,
         const void* obs, const double* partials, const int8_t* status, double* node_distn,
         double* W, double* root_post_sum, const double* Kmat, double* branch_out,
-        cudaStream_t stream) {
+        const double* site_weight, cudaStream_t stream) {
   constexpr int SP = 8 * MT;
   constexpr int LDP = SP + 4;
   int64_t gr = (n_sites + 255) / 256;
   root_distn_generic_kernel<<<(int)(gr < 1184 ? gr : 1184), 256, sizeof(double) * S, stream>>>(
-      S, n_sites, stride, root_distn, partials, status, node_distn, root_post_sum);
+      S, n_sites, stride, root_distn, partials, status, site_weight, node_distn, root_post_sum);
   const size_t smem = sizeof(double) * ((size_t)SP * LDP + 2 * (size_t)kWarps * SP * kLd + 2 * SP);
   const int4* edges = reinterpret_cast<const int4*>(edges_dev);
   const unsigned gx = (unsigned)((n_sites + kTilesPerCta * kTileSites - 1) / (kTilesPerCta * kTileSites));
@@ -622,10 +625,10 @@ int rt_posterior_dmma_dispatch(int S, int obs_kind, int64_t n_sites, int64_t str
                                const double* P, const double* root_distn, const void* obs,
                                const double* partials, const int8_t* status, double* node_distn,
                                double* W, double* root_post_sum, const double* Kmat,
-                               double* branch_out, cudaStream_t stream) {
+                               double* branch_out, const double* site_weight, cudaStream_t stream) {
   const int MT = (S + 15) / 16 * 2;
 #define RT_ARGS S, obs_kind, n_sites, stride, edges_dev, level_ptr_h, n_levels, P, root_distn, obs, \
-                partials, status, node_distn, W, root_post_sum, Kmat, branch_out, stream
+                partials, status, node_distn, W, root_post_sum, Kmat, branch_out, site_weight, stream
   switch (MT) {
     case 2: return run<2>(RT_ARGS);
     case 4: return run<4>(RT_ARGS);

@@ -23,11 +23,14 @@ namespace {
 constexpr int kBlock = 256;
 constexpr int kSitesPerCta = 2048;
 
+// site_weight (nullable): D[root] = w_site * norm(pi o L_root).  The level kernels below only
+// propagate the root marginal, so every marginal and W of the site then carries the weight.
 template <int S>
 __global__ void __launch_bounds__(kBlock)
 root_distn_kernel(int64_t n_sites, int64_t stride, int64_t nd_stride, const double* __restrict__ root_distn,
                   const double* __restrict__ partials, const int8_t* __restrict__ status,
-                  double* __restrict__ node_distn, double* __restrict__ root_post_sum) {
+                  const double* __restrict__ site_weight, double* __restrict__ node_distn,
+                  double* __restrict__ root_post_sum) {
   __shared__ double red[kBlock / 32][S];
   const int tid = threadIdx.x;
   double sum[S];
@@ -47,7 +50,7 @@ root_distn_kernel(int64_t n_sites, int64_t stride, int64_t nd_stride, const doub
       w[s] = partials[(int64_t)s * stride + site] * (root_distn ? root_distn[s] : 1.0);
       tot += w[s];
     }
-    const double inv = 1.0 / tot;
+    const double inv = (site_weight ? site_weight[site] : 1.0) / tot;
 #pragma unroll
     for (int s = 0; s < S; ++s) {
       const double d = w[s] * inv;
@@ -352,15 +355,22 @@ __device__ __forceinline__ double fast_rcp(double x) {
 // BR: also write, per site and branch, x = sum_ab G_a K_b[a,c] L_c -- the posterior expectation
 // of the statistic whose per-edge kernel is K (e.g. K_b = L(t_b Q, t_b (E o Q)): expected number
 // of E-type transitions on the branch, examples/code2x3/extras.py:19-132).
-template <int S, int OBS, bool BR, bool PACKED>
-__global__ void __launch_bounds__(kWalkBlock)
+// WEIGHTED: the root marginal of a site is w_site * norm(pi o L_root) (site_weight[n_sites]).
+// Nothing below the root renormalises, so W, root_post_sum and the node marginals carry the
+// weight.  site_weight is the last parameter: the WEIGHTED = false instantiations never read it
+// and keep the parameter layout of the kernel without it.  With a minimum of one CTA per SM
+// (none for the unweighted kernels, as before) ptxas gives the weighted walk the registers it
+// needs: with the default heuristic it spilled 4-20 bytes for S = 2..4, and with this none up to
+// S = 6.
+template <int S, int OBS, bool BR, bool PACKED, bool WEIGHTED>
+__global__ void __launch_bounds__(kWalkBlock, WEIGHTED ? 1 : 0)
 down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ program, int n_ops,
                  int n_slots, int n_nodes, const double* __restrict__ P,
                  const double* __restrict__ root_distn, const void* __restrict__ obs,
                  const double* __restrict__ partials, const int8_t* __restrict__ status,
                  double* __restrict__ node_distn, double* __restrict__ W,
                  double* __restrict__ root_post_sum, const double* __restrict__ Kmat,
-                 double* __restrict__ branch_out) {
+                 double* __restrict__ branch_out, const double* __restrict__ site_weight) {
   constexpr int obs_packed = PACKED ? 1 : 0;   // RT_OBS_CODES4 decoded at compile time
   constexpr int V = WalkV<S>::value;
   constexpr int NS = WalkNS<S>::value;
@@ -497,7 +507,8 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
             cur[q][s] = live[q] ? src[(int64_t)s * stride + q * kWalkBlock] * pi_s[s] : 0.0;
             tot += cur[q][s];
           }
-          const double inv = tot > 0.0 ? 1.0 / tot : 0.0;
+          const double num = WEIGHTED ? (live[q] ? site_weight[site0 + q * kWalkBlock] : 0.0) : 1.0;
+          const double inv = tot > 0.0 ? num / tot : 0.0;
 #pragma unroll
           for (int s = 0; s < S; ++s) {
             cur[q][s] *= inv;
@@ -692,14 +703,14 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
   if (root_post_sum && tid < S && rp_s[tid] != 0.0) atomicAdd(&root_post_sum[tid], rp_s[tid]);
 }
 
-template <int S, int OBS, bool BR, bool PACKED = false>
+template <int S, int OBS, bool BR, bool PACKED, bool WEIGHTED>
 int launch_walk(int64_t n_sites, int64_t stride, const int4* program, int n_ops, int n_slots,
                 int n_nodes, const double* P, const double* root_distn, const void* obs,
                 const double* partials, const int8_t* status, double* node_distn, double* W,
                 double* root_post_sum, const double* Kmat, double* branch_out,
-                cudaStream_t stream, bool* handled) {
+                const double* site_weight, cudaStream_t stream, bool* handled) {
   constexpr int NS = WalkNS<S>::value;
-  auto kern = down_walk_kernel<S, OBS, BR, PACKED>;
+  auto kern = down_walk_kernel<S, OBS, BR, PACKED, WEIGHTED>;
   const size_t smem = (sizeof(int4) + sizeof(long long)) * n_ops +
                       sizeof(double) * (2 * S + (size_t)n_nodes * ((BR ? 3 : 2) * S * S + S * (S + 1))) +
                       sizeof(double) * (size_t)n_slots * NS * S * kWalkBlock;
@@ -717,32 +728,40 @@ int launch_walk(int64_t n_sites, int64_t stride, const int4* program, int n_ops,
   if (grid > tiles) grid = tiles;
   kern<<<(unsigned)grid, kWalkBlock, smem, stream>>>(n_sites, stride, program, n_ops, n_slots,
                                                      n_nodes, P, root_distn, obs, partials, status,
-                                                     node_distn, W, root_post_sum, Kmat, branch_out);
+                                                     node_distn, W, root_post_sum, Kmat, branch_out,
+                                                     site_weight);
   RT_CUDA_CHECK(cudaGetLastError());
   *handled = true;
   return RT_OK;
 }
 
+// site_weight (nullable): weighted root marginals (see down_walk_kernel); not combined with
+// per-branch output
 template <int S>
 int run(int obs_kind, int64_t n_sites, int64_t stride, const int32_t* program, int n_ops,
         int n_slots, int n_nodes, const int32_t* edges_dev,
         const int32_t* level_ptr_h, int n_levels, const double* P, const double* root_distn,
         const void* obs, const double* partials, const int8_t* status, double* node_distn,
         double* W, double* root_post_sum, const double* Kmat, double* branch_out,
-        cudaStream_t stream) {
+        const double* site_weight, cudaStream_t stream) {
+  if (site_weight && branch_out) return RT_ERR_ARG;
   if (program && n_ops > 0) {
     bool handled = false;
     const int4* prog = reinterpret_cast<const int4*>(program);
     int rc = RT_ERR_ARG;
 #define RT_WALK(OBSK, PACKED)                                                                     \
-  rc = branch_out ? launch_walk<S, OBSK, true, PACKED>(n_sites, stride, prog, n_ops, n_slots,       \
-                                                       n_nodes, P, root_distn, obs, partials,       \
-                                                       status, node_distn, W, root_post_sum, Kmat,  \
-                                                       branch_out, stream, &handled)                \
-                  : launch_walk<S, OBSK, false, PACKED>(n_sites, stride, prog, n_ops, n_slots,      \
-                                                        n_nodes, P, root_distn, obs, partials,      \
-                                                        status, node_distn, W, root_post_sum,       \
-                                                        nullptr, nullptr, stream, &handled)
+  rc = branch_out    ? launch_walk<S, OBSK, true, PACKED, false>(                                  \
+                           n_sites, stride, prog, n_ops, n_slots, n_nodes, P, root_distn, obs,      \
+                           partials, status, node_distn, W, root_post_sum, Kmat, branch_out,        \
+                           nullptr, stream, &handled)                                               \
+       : site_weight ? launch_walk<S, OBSK, false, PACKED, true>(                                  \
+                           n_sites, stride, prog, n_ops, n_slots, n_nodes, P, root_distn, obs,      \
+                           partials, status, node_distn, W, root_post_sum, nullptr, nullptr,        \
+                           site_weight, stream, &handled)                                           \
+                     : launch_walk<S, OBSK, false, PACKED, false>(                                 \
+                           n_sites, stride, prog, n_ops, n_slots, n_nodes, P, root_distn, obs,      \
+                           partials, status, node_distn, W, root_post_sum, nullptr, nullptr,        \
+                           nullptr, stream, &handled)
     if (obs_kind == OBS_CODES) RT_WALK(OBS_CODES, false);
     else if (obs_kind == 3) RT_WALK(OBS_CODES, true);
     else if (obs_kind == OBS_MASK) RT_WALK(OBS_MASK, false);
@@ -783,7 +802,8 @@ int run(int obs_kind, int64_t n_sites, int64_t stride, const int32_t* program, i
     int64_t gr = (n + kBlock - 1) / kBlock;
     int grid_root = (int)(gr < 148 * 8 ? gr : 148 * 8);
     root_distn_kernel<S><<<grid_root, kBlock, 0, stream>>>(n, stride, nd_stride, root_distn, partials + lo,
-                                                           status + lo, nd, root_post_sum);
+                                                           status + lo, site_weight ? site_weight + lo : nullptr,
+                                                           nd, root_post_sum);
 #define RT_LEVELS(OBSK, PACKED)                                                                     \
   (br ? launch_levels<S, OBSK, true, PACKED>(n, stride, nd_stride, edges, level_ptr_h, n_levels, P, ob, \
                                              partials + lo, status + lo, nd, W, Kmat, br, stream)     \
@@ -808,10 +828,10 @@ int rt_posterior_small_dispatch(int S, int obs_kind, int64_t n_sites, int64_t st
                                 const double* P, const double* root_distn, const void* obs,
                                 const double* partials, const int8_t* status, double* node_distn,
                                 double* W, double* root_post_sum, const double* Kmat,
-                                double* branch_out, cudaStream_t stream) {
+                                double* branch_out, const double* site_weight, cudaStream_t stream) {
 #define RT_ARGS obs_kind, n_sites, stride, program, n_ops, n_slots, n_nodes, edges_dev, level_ptr_h, \
                 n_levels, P, root_distn, obs, partials, status, node_distn, W, root_post_sum, Kmat,  \
-                branch_out, stream
+                branch_out, site_weight, stream
   switch (S) {
     case 2: return run<2>(RT_ARGS);
     case 3: return run<3>(RT_ARGS);

@@ -269,20 +269,45 @@ class TreeMJP(object):
         _native.check(rc, 'rt_prune_loglik')
 
     def _down(self, obs, prog, lo, hi, stream, partials, status, node_distn, W, root_post_sum,
-              K=None, branch=None):
+              K=None, branch=None, site_weight=None):
         """rt_posterior_stats for the sites [lo, hi) of `obs` on `stream`, addressed as in _up;
-        rt_posterior_branch_stats when a per-edge kernel K is given (per-site output `branch`)."""
+        rt_posterior_branch_stats when a per-edge kernel K is given (per-site output `branch`),
+        rt_posterior_weighted_stats when per-site weights are given."""
         lp = prog['level_ptr']
         args = (self.S, self.sched.n, hi - lo, obs.stride, _ptr(prog['ops']), prog['n_ops'],
                 prog['n_slots'], _ptr(prog['edges']), lp.ctypes.data, len(lp) - 1,
                 _ptr(self.transition_matrices()), _ptr(self.root_distn), obs.kind, obs.site_ptr(lo),
                 _ptr(partials, lo), _ptr(status, lo), _ptr(node_distn, lo), _ptr(W),
                 _ptr(root_post_sum))
-        if K is None:
-            rc = _native.lib().rt_posterior_stats(*args, _stream(stream))
-        else:
+        if K is not None:
+            name = 'rt_posterior_branch_stats'
             rc = _native.lib().rt_posterior_branch_stats(*args, _ptr(K), _ptr(branch, lo), _stream(stream))
-        _native.check(rc, 'rt_posterior_stats' if K is None else 'rt_posterior_branch_stats')
+        elif site_weight is not None:
+            name = 'rt_posterior_weighted_stats'
+            rc = _native.lib().rt_posterior_weighted_stats(*args, _ptr(site_weight, lo), _stream(stream))
+        else:
+            name = 'rt_posterior_stats'
+            rc = _native.lib().rt_posterior_stats(*args, _stream(stream))
+        _native.check(rc, name)
+
+    def _check_site_weight(self, site_weight, n_sites):
+        """Shape, dtype and device of per-site weights, on the host (no device sync)."""
+        if not isinstance(site_weight, torch.Tensor):
+            raise TypeError('site_weight must be a torch tensor')
+        if site_weight.dtype != torch.float64:
+            raise ValueError('site_weight must be float64')
+        dev = self.device
+        if dev.type == 'cuda' and dev.index is None:
+            dev = torch.device('cuda', torch.cuda.current_device())
+        if site_weight.device != dev:
+            raise ValueError('site_weight must be on %s' % dev)
+        if tuple(site_weight.shape) != (n_sites,) or not site_weight.is_contiguous():
+            raise ValueError('site_weight must be a contiguous [n_sites] = [%d] tensor' % n_sites)
+
+    @staticmethod
+    def _weighted_loglik_sum(loglik, status, site_weight):
+        """sum_s w_s * loglik_s over the feasible sites."""
+        return (torch.where(status == 0, loglik, torch.zeros_like(loglik)) * site_weight).sum()
 
     def log_likelihood(self, obs, keep_partials=False, want_exponents=False, out=None,
                        loglik_sum=None):
@@ -311,7 +336,8 @@ class TreeMJP(object):
         return res
 
     # ---- K4 / K5 ------------------------------------------------------------
-    def _chunked(self, obs, n_chunks, codes_host=None, out_loglik=None, out_status=None):
+    def _chunked(self, obs, n_chunks, codes_host=None, out_loglik=None, out_status=None,
+                 site_weight=None):
         """Up + down pass with the site axis cut into `n_chunks` chunks (multiples of 128 sites) that
         take turns on E2E_STREAMS compute streams.  codes_host: pinned codes in the layout of
         obs.data; the H2D copies of all chunks are enqueued first on the copy-in stream, one event
@@ -354,7 +380,7 @@ class TreeMJP(object):
             if ev_in:
                 cs.wait_event(ev_in[k])
             self._up(obs, prog, lo, hi, cs, loglik, status, partials, loglik_sum=llsum)
-            self._down(obs, prog, lo, hi, cs, partials, status, None, W, rps)
+            self._down(obs, prog, lo, hi, cs, partials, status, None, W, rps, site_weight=site_weight)
             if out_loglik is not None:
                 done = torch.cuda.Event()
                 done.record(cs)
@@ -364,21 +390,33 @@ class TreeMJP(object):
                     out_status[lo:hi].copy_(status[lo:hi], non_blocking=True)
         for cs in compute:
             cur.wait_stream(cs)
+        if site_weight is not None:
+            llsum = self._weighted_loglik_sum(loglik, status, site_weight).reshape(1)
         return dict(loglik=loglik, status=status, loglik_sum=llsum[0], partials=partials,
                     exponents=None, node_distn=None, W=W, root_post_sum=rps,
                     n_levels=len(prog['level_ptr']) - 1)
 
-    def posterior(self, obs, want_exponents=False, want_node_distn=True, overlap_chunks=0):
+    def posterior(self, obs, want_exponents=False, want_node_distn=True, overlap_chunks=0,
+                  site_weight=None):
         """Up + down pass.  Returns loglik, status, loglik_sum, partials, node_distn (internal
         nodes, by store index), W[n,S,S] (site-summed J/P weights), root_post_sum[S].
         overlap_chunks > 1 (S <= 8, no node marginals / exponents wanted): the site chunks of the
-        host-buffer pipeline, without its copies, see _chunked."""
+        host-buffer pipeline, without its copies, see _chunked.
+        site_weight: fp64 device tensor [n_sites] of non-negative, finite weights, or None (all
+        1).  Site s then counts w_s times in W, root_post_sum and node_distn, and loglik_sum is
+        sum_s w_s loglik_s over the feasible sites; per-site loglik and status do not change.
+        Integer weights are site-pattern compression (w = columns with the pattern); class
+        posteriors give the E-step of a site-class mixture (raoteh_b200.mixture)."""
+        if site_weight is not None:
+            self._check_site_weight(site_weight, obs.n_sites)
         if overlap_chunks > 1 and self.S <= 8 and not want_node_distn and not want_exponents:
-            return self._chunked(obs, int(overlap_chunks))
+            return self._chunked(obs, int(overlap_chunks), site_weight=site_weight)
         llsum = self._buf('loglik_sum', (1,), torch.float64, zero=True)
         up = self.log_likelihood(obs, keep_partials=True, want_exponents=want_exponents,
                                  loglik_sum=llsum)
         up['loglik_sum'] = llsum[0]      # sum of the finite log-likelihoods, reduced by the kernel
+        if site_weight is not None:
+            up['loglik_sum'] = self._weighted_loglik_sum(up['loglik'], up['status'], site_weight)
         prog = self._programs(obs)
         node_distn = None
         if want_node_distn or self.S > 8:
@@ -387,7 +425,7 @@ class TreeMJP(object):
         root_post_sum = self._buf('root_post_sum', (self.S,), torch.float64, zero=True)
         self._mark('down')
         self._down(obs, prog, 0, obs.n_sites, None, up['partials'], up['status'], node_distn, W,
-                   root_post_sum)
+                   root_post_sum, site_weight=site_weight)
         self._mark('down')
         up.update(node_distn=node_distn, W=W, root_post_sum=root_post_sum,
                   n_levels=len(prog['level_ptr']) - 1)
@@ -614,14 +652,17 @@ class TreeMJP(object):
                                 r['root_post_sum'].reshape(-1)])
         return r
 
-    def expected_history_statistics(self, obs, want_node_distn=False, overlap_chunks=0):
+    def expected_history_statistics(self, obs, want_node_distn=False, overlap_chunks=0,
+                                    site_weight=None):
         """Site-summed expected dwell[S], transition counts[S,S], root posterior sum[S],
         per-site loglik, per-edge contraction matrices M_edges[n,S,S].
 
         dwell[c] = sum_b M_b[c,c]; trans[c,d] = Q_b[c,d] * M_b[c,d] summed over
         edges (raoteh/sampler/_mjp_dense.py:497-533 with one Frechet derivative per
-        edge, the form of examples/code2x3/extras.py:108-129)."""
-        post = self.posterior(obs, want_node_distn=want_node_distn, overlap_chunks=overlap_chunks)
+        edge, the form of examples/code2x3/extras.py:108-129).
+        site_weight: per-site weights of the sums, as in `posterior`."""
+        post = self.posterior(obs, want_node_distn=want_node_distn, overlap_chunks=overlap_chunks,
+                              site_weight=site_weight)
         M, dwell, trans = self.history_statistics(post['W'])
         post.update(dwell=dwell, trans=trans, M_edges=M, Q_edges=self._edge_rates())
         return post

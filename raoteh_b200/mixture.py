@@ -1,0 +1,180 @@
+"""
+Site-class mixtures of tree MJPs: among-site rate variation (discrete gamma, +G, Yang 1994), an
+invariant-sites class (+I, rate 0) and classes with their own rate matrix (codon models with
+several omega classes, the M1a/M2a/M8 family).
+
+Every site evolves under one of K classes, class k with prior weight w_k, rate matrix Q_k and
+branch lengths r_k t; the classes share the tree and the root distribution.  Per site
+
+    loglik = logsumexp_k(log w_k + loglik_k),    class_post[k] = exp(log w_k + loglik_k - loglik),
+
+and the expected statistics under the mixture are sum_s class_post[k](s) E_k[stat | s].  Each
+class is one TreeMJP on the schedule with lengths r_k t, so P, both tree passes and the Frechet
+contraction are the single-class ones; the class posterior enters the down pass as a per-site
+weight of the root marginal (rt_posterior_weighted_stats).  The classes share one workspace, so
+the device memory is that of one single-class evaluation plus [K, n_sites] per-site arrays.
+"""
+from __future__ import annotations
+
+import math
+
+import numpy as np
+import torch
+from scipy import special
+
+from .engine import TreeMJP
+from .lowering import TreeSchedule
+
+
+def discrete_gamma_rates(alpha, K, median=False):
+    """Rates of the K equal-probability categories of Gamma(alpha, rate alpha) (mean 1), Yang
+    (1994): the category boundaries are the quantiles k/K; the rate of a category is its mean
+    (K times the integral of x g(x) over the category), or with `median` its median, rescaled so
+    that the K rates have mean 1."""
+    alpha = float(alpha)
+    if not (math.isfinite(alpha) and alpha > 0):
+        raise ValueError('alpha must be positive and finite')
+    if int(K) != K or K < 1:
+        raise ValueError('K must be a positive integer')
+    K = int(K)
+    if median:
+        r = special.gammaincinv(alpha, (2.0 * np.arange(K) + 1.0) / (2.0 * K)) / alpha
+        return r * (K / r.sum())
+    # boundaries in units of the rate-1 gamma: alpha * b_k, with b_0 = 0 and b_K = inf
+    cut = np.concatenate([[0.0], special.gammaincinv(alpha, np.arange(1, K) / K), [np.inf]])
+    # int_a^b x g(x) dx = P(alpha + 1, alpha b) - P(alpha + 1, alpha a), P the regularised gamma
+    return K * np.diff(special.gammainc(alpha + 1.0, cut))
+
+
+class SiteMixtureMJP(object):
+    """K site classes on one tree.
+
+    Q: one rate matrix [S, S] shared by the K = len(rates) classes, or K matrices [K, S, S].
+    rates: per-class multipliers of the branch lengths (default all 1); rate 0 is the +I class.
+    weights: prior class probabilities (default uniform), positive, summing to 1.
+    root_distn: the root distribution of every class (None: weights of 1, as TreeMJP).
+    Per-edge rate matrices inside a class (TreeMJP's q_index) are not supported."""
+
+    def __init__(self, sched, Q, root_distn=None, rates=None, weights=None, q_index=None,
+                 device='cuda'):
+        if q_index is not None:
+            raise ValueError('per-edge rate matrices (q_index) are not supported inside mixture classes')
+        Q = np.asarray(Q, dtype=np.float64)
+        if Q.ndim == 2:
+            K = 1 if rates is None else len(rates)
+            Qs = np.broadcast_to(Q, (K,) + Q.shape)
+        elif Q.ndim == 3:
+            K = Q.shape[0]
+            Qs = Q
+        else:
+            raise ValueError('Q must be [S, S] or [K, S, S]')
+        S = Q.shape[-1]
+        if Q.shape[-2] != S or not 2 <= S <= 64:
+            raise ValueError('rate matrices must be square with 2..64 states')
+        rates = np.ones(K) if rates is None else np.asarray(rates, dtype=np.float64).ravel()
+        weights = np.full(K, 1.0 / K) if weights is None else np.asarray(weights, dtype=np.float64).ravel()
+        if len(rates) != K or len(weights) != K:
+            raise ValueError('rates and weights need one entry per class (K = %d)' % K)
+        if not (np.isfinite(rates).all() and (rates >= 0).all()):
+            raise ValueError('class rates must be finite and non-negative')
+        if not (np.isfinite(weights).all() and (weights > 0).all() and abs(weights.sum() - 1.0) <= 1e-9):
+            raise ValueError('class weights must be positive and sum to 1')
+        self.K, self.S, self.sched = K, S, sched
+        self.rates, self.weights = rates, weights
+        self.device = torch.device(device)
+        self.length = torch.from_numpy(np.asarray(sched.length, dtype=np.float64).copy()).to(self.device)
+        self.tree_length = float(np.asarray(sched.length, dtype=np.float64)[1:].sum())
+        self.classes = []
+        for k in range(K):
+            s = TreeSchedule(sched.parent, rates[k] * sched.length, sched.nodes)
+            m = TreeMJP(s, Qs[k], root_distn=root_distn, device=device)
+            if self.classes:
+                # the classes run one after the other on one stream and have the same topology:
+                # one set of workspaces (partials, W, node marginals) and of programs serves all
+                m._ws = self.classes[0]._ws
+                m._prog_cache = self.classes[0]._prog_cache
+            self.classes.append(m)
+        self.log_weights = torch.from_numpy(np.log(weights)).to(self.device)
+
+    def log_likelihood(self, obs):
+        """Per-site mixture log-likelihood.  Returns dict(loglik [N], status [N], class_post [K, N],
+        loglik_class [K, N], loglik_sum).  status is 0 where some class has status 0, else 2 where
+        some class has 2, else 1; infeasible sites have loglik -inf and class_post 0 and are left
+        out of loglik_sum."""
+        K, N, dev = self.K, obs.n_sites, self.device
+        ll_class = torch.empty((K, N), dtype=torch.float64, device=dev)
+        st_class = torch.empty((K, N), dtype=torch.int8, device=dev)
+        for k, m in enumerate(self.classes):
+            m.log_likelihood(obs, out=(ll_class[k], st_class[k]))
+        ok_class = st_class == 0
+        lw = torch.where(ok_class, self.log_weights[:, None] + ll_class,
+                         torch.full_like(ll_class, -math.inf))
+        loglik = torch.logsumexp(lw, dim=0)
+        ok = ok_class.any(dim=0)
+        loglik = torch.where(ok, loglik, torch.full_like(loglik, -math.inf))
+        class_post = torch.where(ok[None, :], torch.exp(lw - torch.where(ok, loglik, 0.0)[None, :]),
+                                 torch.zeros_like(lw))
+        two = (st_class == 2).any(dim=0)
+        status = torch.where(ok, 0, torch.where(two, 2, 1)).to(torch.int8)
+        loglik_sum = torch.where(ok, loglik, torch.zeros_like(loglik)).sum()
+        return dict(loglik=loglik, status=status, class_post=class_post, loglik_class=ll_class,
+                    loglik_sum=loglik_sum)
+
+    def expected_history_statistics(self, obs, want_node_distn=False, site_weight=None):
+        """Expected statistics under the mixture, summed over sites (each site weighted by
+        site_weight, default 1).  Returns the keys of TreeMJP's result that dist.pack_stats
+        reads -- loglik_sum (sum of w_s loglik_s over feasible sites), dwell [S], trans [S, S],
+        root_post_sum [S] -- and the per-site loglik, status, class_post; per class dwell_class
+        [K, S], trans_class [K, S, S], M_edges_class [K, n, S, S] and class_post_sum [K] (the EM
+        update of the class weights, times the total site weight); with want_node_distn the
+        mixture node marginals [n_store, S, stride].  Dwell times are in tree time (the class's
+        contraction runs on lengths r_k t and is divided by r_k; a rate-0 class dwells
+        sum_b t_b per unit of root posterior and makes no transitions)."""
+        N, S, K, n = obs.n_sites, self.S, self.K, self.sched.n
+        if site_weight is not None:
+            self.classes[0]._check_site_weight(site_weight, N)
+        mix = self.log_likelihood(obs)
+        cp = mix['class_post']
+        w = cp if site_weight is None else cp * site_weight[None, :]
+        dev = self.device
+        dwell = torch.empty((K, S), dtype=torch.float64, device=dev)
+        trans = torch.empty((K, S, S), dtype=torch.float64, device=dev)
+        M_class = torch.empty((K, n, S, S), dtype=torch.float64, device=dev)
+        rps = torch.empty((K, S), dtype=torch.float64, device=dev)
+        node_distn = None
+        for k, m in enumerate(self.classes):
+            post = m.posterior(obs, want_node_distn=want_node_distn, site_weight=w[k])
+            rps[k] = post['root_post_sum']
+            r = float(self.rates[k])
+            if r > 0:
+                M, d, t = m.history_statistics(post['W'])
+                M_class[k] = M / r
+                dwell[k] = d / r
+                trans[k] = t
+            else:
+                # P = I: W_b is diagonal and L(r t Q^T, r t W) / r -> t W as r -> 0
+                M_class[k] = self.length[:, None, None] * post['W']
+                dwell[k] = self.tree_length * post['root_post_sum']
+                trans[k].zero_()
+            if want_node_distn:
+                nd = post['node_distn']
+                node_distn = nd.clone() if node_distn is None else node_distn.add_(nd)
+        loglik_sum = (mix['loglik_sum'] if site_weight is None else
+                      TreeMJP._weighted_loglik_sum(mix['loglik'], mix['status'], site_weight))
+        return dict(loglik=mix['loglik'], status=mix['status'], class_post=cp,
+                    loglik_class=mix['loglik_class'], loglik_sum=loglik_sum,
+                    dwell=dwell.sum(dim=0), trans=trans.sum(dim=0), root_post_sum=rps.sum(dim=0),
+                    dwell_class=dwell, trans_class=trans, M_edges_class=M_class,
+                    class_post_sum=w.sum(dim=1), node_distn=node_distn)
+
+    def branch_expectations(self, obs, E=None):
+        """Per site and branch posterior expectation of the number of E-type transitions under
+        the mixture: sum_k class_post[k] * (class k's TreeMJP.branch_expectations, with K_b built
+        on the class's lengths r_k t).  Returns dict(branch [n, N], loglik, status, class_post)."""
+        mix = self.log_likelihood(obs)
+        cp = mix['class_post']
+        branch = None
+        for k, m in enumerate(self.classes):
+            b = m.branch_expectations(obs, E=E)['branch'] * cp[k][None, :]
+            branch = b if branch is None else branch.add_(b)
+        return dict(branch=branch, loglik=mix['loglik'], status=mix['status'], class_post=cp)
