@@ -16,6 +16,8 @@
 // joint J_b = G_b[:,None] * P_b * L_b[None,:] is never materialised.
 // HBM traffic per site and edge: D_parent in, L_child in, D_child out
 // (3 * S * 8 B; leaves read 1 code byte instead) -- HBM-bound.
+#include <type_traits>
+
 #include "rt_common.cuh"
 
 namespace {
@@ -251,10 +253,21 @@ void launch_levels(int64_t n_sites, int64_t stride, int64_t nd_stride, const int
 // transpose (reduce-scatter) butterfly -- V = S*S values over 32 lanes in
 // V/2 + V/4 + ... exchanges instead of V full reductions -- and then added to a per-CTA
 // accumulator in shared memory; one masked global atomicAdd per entry per CTA at the end.
+//
+// Lane frames (S = 4): lane l holds every S-vector with its states permuted by an XOR mask,
+// a parent-side vector (the node marginal `cur`, G) in frame x = (l >> 3) & 3 -- element a is
+// state a ^ x -- and a child-side vector (L, the child marginal t) in frame y = (l >> 1) & 3.
+// Entry (a, b) of G (x) L then sits in register ((a ^ x) << 2) | (b ^ y) = (4a + b) ^ z with
+// z = (l >> 1) & 15, and in every stage of the butterfly the lane keeps the lower half of its
+// registers and sends the upper half: the stages are shuffles and adds without selects (two
+// FSEL per double and per half before).  The frame costs per-lane addresses: P, K and the leaf
+// reciprocal table are read at permuted indices, stored partials at row b ^ y, node marginals
+// are written to rows a ^ x / b ^ y, and a child marginal goes to the stack at position
+// b ^ x ^ y, so that it reads back in frame x -- also the one the next op consumes, which
+// otherwise stays in registers (the round trip costs fewer instructions than 16 FSEL per site).
+// Only the S = 4 kernels without per-branch output use frames: with them, the per-branch
+// kernel needed 75 more registers (233) and lost a CTA per SM.  Elsewhere both masks are 0.
 // ---------------------------------------------------------------------------------------
-#ifndef RT_WALK_DMMA_REDUCE
-#define RT_WALK_DMMA_REDUCE 0
-#endif
 #ifndef RT_WALK_BLOCK
 #define RT_WALK_BLOCK 128
 #endif
@@ -273,7 +286,9 @@ void launch_levels(int64_t n_sites, int64_t stride, int64_t nd_stride, const int
 #endif
 constexpr int kWalkBlock = RT_WALK_BLOCK;
 
-template <int V>
+// FRAMED: the lane's values are in the lane frame described above (V = 16), so that the lane
+// keeps v[i] and sends v[i + half] in every stage; otherwise it picks the halves by its lane bit
+template <int V, bool FRAMED>
 __device__ __forceinline__ void reduce_scatter_warp(double (&v)[V], int lane) {
   // after the call: V==16 -> lane holds value (lane>>1) in v[0]; V==32 -> value `lane`;
   // V==64 -> values 2*lane, 2*lane+1 in v[0], v[1]   (all fully summed over the warp)
@@ -281,7 +296,7 @@ __device__ __forceinline__ void reduce_scatter_warp(double (&v)[V], int lane) {
 #pragma unroll
   for (int m = 16; m >= 1; m >>= 1) {
     if (len > 1) {
-      const bool up = (lane & m) != 0;
+      const bool up = !FRAMED && (lane & m) != 0;
       const int half = len / 2;
 #pragma unroll
       for (int i = 0; i < V / 2; ++i) {
@@ -300,39 +315,14 @@ __device__ __forceinline__ void reduce_scatter_warp(double (&v)[V], int lane) {
 
 template <int S> struct WalkV { static constexpr int value = (S <= 4) ? 16 : (S == 5 ? 32 : 64); };
 
-__device__ __forceinline__ void dmma884_acc(double& c0, double& c1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-               : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
-}
-
-// Cross-lane reduction of the S*S per-lane weights on the FP64 tensor pipe.  One DMMA with the
-// lane's value as the B fragment (k = lane % 4, n = lane / 4) and a row selector as the A
-// fragment (a[m][k] = [m == r]) adds, for value r of the tile, the 4 lanes of every lane group n
-// into C[r][n]; 8 DMMAs fill an 8 x 8 tile (value x lane group), two adds and two shuffles
-// finish the sum over the groups.  16 DMMA + ~14 other instructions per edge and warp for
-// S = 4, against 30 SHFL + 60 FSEL + 15 DADD for the shuffle butterfly -- but MEASURED SLOWER
-// (C2 walk 0.749 ms vs 0.640 ms): on B200 the FP64 DMMA runs at the FP64 FMA rate (37.0 vs
-// 33.5 TFLOP/s measured), so 16 DMMAs cost the FP64 pipe as much as 128 DFMAs, far more than
-// the butterfly's 15 DADDs.  Kept behind RT_WALK_DMMA_REDUCE (0) as a recorded experiment.
-template <int S, int V>
-__device__ __forceinline__ void reduce_w_dmma(const double (&w)[V], const double (&sel)[8], int lane,
-                                              double* Wc) {
-  const int g = lane >> 2, t = lane & 3;
-  constexpr int NT = (S * S + 7) / 8;
+// v[i] <- v[i ^ d] for a 2-bit lane mask d (S = 4): two select stages
+__device__ __forceinline__ void xor_permute4(double (&v)[4], int d) {
+  const bool b0 = (d & 1) != 0, b1 = (d & 2) != 0;
+  double u[4];
 #pragma unroll
-  for (int tile = 0; tile < NT; ++tile) {
-    double c0 = 0.0, c1 = 0.0;
+  for (int i = 0; i < 4; ++i) u[i] = b0 ? v[i ^ 1] : v[i];
 #pragma unroll
-    for (int r = 0; r < 8; ++r) {
-      const int i = tile * 8 + r;
-      if (i < S * S) dmma884_acc(c0, c1, sel[r], w[i]);
-    }
-    double v = c0 + c1;
-    v += __shfl_xor_sync(0xffffffffu, v, 1);
-    v += __shfl_xor_sync(0xffffffffu, v, 2);
-    const int idx = tile * 8 + g;
-    if (t == 0 && idx < S * S && v != 0.0) atomicAdd(&Wc[idx], v);
-  }
+  for (int i = 0; i < 4; ++i) v[i] = b1 ? u[i ^ 2] : u[i];
 }
 // sites per thread: more sites amortise the per-op work (program decode, P loads, the
 // cross-lane reduction of W) over more arithmetic; bounded by registers
@@ -363,7 +353,7 @@ __device__ __forceinline__ double fast_rcp(double x) {
 // needs: with the default heuristic it spilled 4-20 bytes for S = 2..4, and with this none up to
 // S = 6.
 template <int S, int OBS, bool BR, bool PACKED, bool WEIGHTED>
-__global__ void __launch_bounds__(kWalkBlock, WEIGHTED ? 1 : 0)
+__global__ void __launch_bounds__(kWalkBlock, WEIGHTED ? 1 : (S == 4 && !BR ? 4 : 0))
 down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ program, int n_ops,
                  int n_slots, int n_nodes, const double* __restrict__ P,
                  const double* __restrict__ root_distn, const void* __restrict__ obs,
@@ -414,13 +404,30 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
   }
   __syncthreads();
 
-  double sel[8];     // A-fragment row selectors of reduce_w_dmma
-#pragma unroll
-  for (int r = 0; r < 8; ++r) sel[r] = ((lane >> 2) == r) ? 1.0 : 0.0;
+  // lane frames (see the header of the walk): parent side x, child side y, W register z
+  constexpr bool kFramed = S == 4 && !BR;
+  const int fx = kFramed ? (lane >> 3) & 3 : 0;
+  const int fy = kFramed ? (lane >> 1) & 3 : 0;
+  const int fz = (fx << 2) | fy;     // P'[a][b] = P[a ^ x][b ^ y] = P[(4a + b) ^ z] for S = 4
+  const int fd = fx ^ fy;            // child frame -> parent frame
+  static_assert(!kFramed || (kWalkBlock & (kWalkBlock - 1)) == 0, "stack rows are XOR-addressed");
+  // entry i of the S x S table of node c (P_s) in the lane's frame.  Framed, a table is 128
+  // bytes, so the permuted byte offset is one XOR (LOP3) with the lane part folded into `cz`.
+  auto tab = [&](const double* t, int c, int i) -> double {
+    if constexpr (kFramed) {
+      const unsigned cz = (unsigned)c * (S * S * 8) | (unsigned)fz * 8;
+      return *reinterpret_cast<const double*>(reinterpret_cast<const char*>(t) + (cz ^ (unsigned)(i * 8)));
+    } else {
+      return t[c * S * S + i];
+    }
+  };
   const int64_t tile_sites = (int64_t)kWalkBlock * NS;
-  const int64_t tiles = (n_sites + tile_sites - 1) / tile_sites;
-  for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-    const int64_t site0 = tile * tile_sites + tid;            // site of q: site0 + q*kWalkBlock
+  // framed: a 32-bit tile index, and the thread index read again at the end, keep the kernels at
+  // 128 registers (4 CTAs per SM) without spills
+  using TileIdx = typename std::conditional<kFramed, int, int64_t>::type;
+  const TileIdx tiles = (TileIdx)((n_sites + tile_sites - 1) / tile_sites);
+  for (TileIdx tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+    const int64_t site0 = (int64_t)tile * tile_sites + tid;            // site of q: site0 + q*kWalkBlock
     // the NEXT tile's leaf-code rows: pulled into L2 a whole tile ahead (the byte loads one op ahead
     // of their use cannot hide a DRAM round trip behind a short leaf op: 9 % of the warp samples
     // sat on that load, ncu source view)
@@ -475,7 +482,7 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
         for (int q = 0; q < NS; ++q)
 #pragma unroll
           for (int s = 0; s < S; ++s)
-            Lb[q][s] = live[q] ? __ldcs(&src[(int64_t)s * stride + q * kWalkBlock]) : 0.0;
+            Lb[q][s] = live[q] ? __ldcs(&src[(int64_t)(s ^ fy) * stride + q * kWalkBlock]) : 0.0;
       } else if (ncode == OP_MSG_OBS && OBS == OBS_CODES) {
         const uint8_t* row = reinterpret_cast<const uint8_t*>(obs) + off_s[j];
 #pragma unroll
@@ -504,7 +511,7 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
           double tot = 0.0;
 #pragma unroll
           for (int s = 0; s < S; ++s) {
-            cur[q][s] = live[q] ? src[(int64_t)s * stride + q * kWalkBlock] * pi_s[s] : 0.0;
+            cur[q][s] = live[q] ? src[(int64_t)(s ^ fx) * stride + q * kWalkBlock] * pi_s[s ^ fx] : 0.0;
             tot += cur[q][s];
           }
           const double num = WEIGHTED ? (live[q] ? site_weight[site0 + q * kWalkBlock] : 0.0) : 1.0;
@@ -513,16 +520,21 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
           for (int s = 0; s < S; ++s) {
             cur[q][s] *= inv;
             if (node_distn && site0 + q * kWalkBlock < n_sites)
-              node_distn[off_s[ip] + (int64_t)s * stride + site0 + q * kWalkBlock] = cur[q][s];
+              node_distn[off_s[ip] + (int64_t)(s ^ fx) * stride + site0 + q * kWalkBlock] = cur[q][s];
           }
         }
         if (root_post_sum) {
+          double ts[S];
 #pragma unroll
           for (int s = 0; s < S; ++s) {
-            double t = 0.0;
+            ts[s] = 0.0;
 #pragma unroll
-            for (int q = 0; q < NS; ++q) t += cur[q][s];
-            t = rt_warp_sum(t);
+            for (int q = 0; q < NS; ++q) ts[s] += cur[q][s];
+          }
+          if constexpr (kFramed) xor_permute4(ts, fx);     // back to the natural state order
+#pragma unroll
+          for (int s = 0; s < S; ++s) {
+            const double t = rt_warp_sum(ts[s]);
             if (lane == 0 && t != 0.0) atomicAdd(&rp_s[s], t);
           }
         }
@@ -543,7 +555,7 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
           // ---- internal child: its marginal D_c = L o (P^T G) is parked (or kept) ----
           double Pr[S * S];
 #pragma unroll
-          for (int i = 0; i < S * S; ++i) Pr[i] = P_s[c * S * S + i];
+          for (int i = 0; i < S * S; ++i) Pr[i] = tab(P_s, c, i);
           const bool fresh = (op.x & OP_FLAG_FRESH) != 0;   // next (reverse) op is the child's OP_STORE
 #pragma unroll
           for (int q = 0; q < NS; ++q) {
@@ -581,10 +593,16 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
             }
 #pragma unroll
             for (int b = 0; b < S; ++b) {
-              if (fresh) cur[q][b] = t[b];
-              else stk[((op.z * NS + q) * S + b) * kWalkBlock + tid] = t[b];
+              // framed: position b ^ x ^ y, as one XOR of the row index (S * kWalkBlock is a power of 2)
+              const int pos = kFramed ? ((((op.z * NS + q) * S * kWalkBlock) | (fd * kWalkBlock + tid)) ^ (b * kWalkBlock))
+                                      : ((op.z * NS + q) * S + b) * kWalkBlock + tid;
+              if (!fresh || kFramed) stk[pos] = t[b];
               if (node_distn && site0 + q * kWalkBlock < n_sites)
-                node_distn[off_s[ip] + (int64_t)b * stride + site0 + q * kWalkBlock] = t[b];
+                node_distn[off_s[ip] + (int64_t)(b ^ fy) * stride + site0 + q * kWalkBlock] = t[b];
+            }
+            if (fresh) {
+#pragma unroll
+              for (int b = 0; b < S; ++b) cur[q][b] = kFramed ? stk[((op.z * NS + q) * S + b) * kWalkBlock + tid] : t[b];
             }
           }
         } else if (code == OP_MSG_OBS && OBS == OBS_CODES) {
@@ -599,8 +617,8 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
             double G[S], L[S];
 #pragma unroll
             for (int a = 0; a < S; ++a) {
-              G[a] = cur[q][a] * Pl[a * SP1 + col];     // (a site that failed carries D = 0 from the root op)
-              L[a] = (k == RT_MISSING || k == a) ? 1.0 : 0.0;
+              G[a] = cur[q][a] * Pl[(a ^ fx) * SP1 + col];     // (a site that failed carries D = 0 from the root op)
+              L[a] = (k == RT_MISSING || (k ^ fy) == a) ? 1.0 : 0.0;
             }
 #pragma unroll
             for (int i = 0; i < S * S; ++i) w[i] = fma(G[i / S], L[i % S], w[i]);
@@ -620,7 +638,7 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
           // ---- leaf with a mask / dense emission row / no observation ----
           double Pr[S * S];
 #pragma unroll
-          for (int i = 0; i < S * S; ++i) Pr[i] = P_s[c * S * S + i];
+          for (int i = 0; i < S * S; ++i) Pr[i] = tab(P_s, c, i);
 #pragma unroll
           for (int q = 0; q < NS; ++q) {
             double L[S];
@@ -631,11 +649,11 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
               const unsigned long long mk = live[q]
                   ? reinterpret_cast<const unsigned long long*>(obs)[off_s[ip] + site0 + q * kWalkBlock] : 0ull;
 #pragma unroll
-              for (int s = 0; s < S; ++s) L[s] = ((mk >> s) & 1ull) ? 1.0 : 0.0;
+              for (int s = 0; s < S; ++s) L[s] = ((mk >> (s ^ fy)) & 1ull) ? 1.0 : 0.0;
             } else {
               const double* d = reinterpret_cast<const double*>(obs) + off_s[ip] + site0 + q * kWalkBlock;
 #pragma unroll
-              for (int s = 0; s < S; ++s) L[s] = live[q] ? d[(int64_t)s * stride] : 0.0;
+              for (int s = 0; s < S; ++s) L[s] = live[q] ? d[(int64_t)(s ^ fy) * stride] : 0.0;
             }
             double G[S];
 #pragma unroll
@@ -661,10 +679,7 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
           }
         }
         // W_c += sum over the warp's 32*NS sites of G (x) L
-        if (RT_WALK_DMMA_REDUCE) {
-          reduce_w_dmma<S, V>(w, sel, lane, W_s + c * S * S);
-        } else {
-        reduce_scatter_warp<V>(w, lane);
+        reduce_scatter_warp<V, kFramed>(w, lane);
         if (V == 16) {
           if ((lane & 1) == 0 && (lane >> 1) < S * S && w[0] != 0.0)
             atomicAdd(&W_s[c * S * S + (lane >> 1)], w[0]);
@@ -673,7 +688,6 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
         } else {
           if (2 * lane < S * S && w[0] != 0.0) atomicAdd(&W_s[c * S * S + 2 * lane], w[0]);
           if (2 * lane + 1 < S * S && w[1] != 0.0) atomicAdd(&W_s[c * S * S + 2 * lane + 1], w[1]);
-        }
         }
       }
     };
@@ -700,7 +714,11 @@ down_walk_kernel(int64_t n_sites, int64_t stride, const int4* __restrict__ progr
     const double v = W_s[i];
     if (v != 0.0 && P_s[i] > 0.0) atomicAdd(&W[i], v);
   }
-  if (root_post_sum && tid < S && rp_s[tid] != 0.0) atomicAdd(&root_post_sum[tid], rp_s[tid]);
+  if (root_post_sum) {
+    int t = tid;
+    if constexpr (kFramed) asm volatile("mov.u32 %0, %%tid.x;" : "=r"(t));
+    if (t < S && rp_s[t] != 0.0) atomicAdd(&root_post_sum[t], rp_s[t]);
+  }
 }
 
 template <int S, int OBS, bool BR, bool PACKED, bool WEIGHTED>
