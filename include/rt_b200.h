@@ -384,6 +384,37 @@ typedef struct rt_posterior_draw_args {
 int rt_posterior_draw(const rt_posterior_draw_args* args, void* stream);
 
 /*
+ * Exact posterior draws under a site-class mixture (+G rates, +I, per-class rate matrices): the
+ * joint draw of (class, history) given the site's observations.  Each trajectory first draws its
+ * site's class c from class_post[.][site] (the class posterior, e.g. w_k L_k / sum_j w_j L_j),
+ * then the history exactly as rt_posterior_draw does, on class c's inputs.  Every field of `base`
+ * means what it means for rt_posterior_draw, except:
+ *   Q          [K][S][S], the class generators r_k Q_k (a rate-0 class has Q = 0: no jumps);
+ *   P          [K][n_nodes][S][S], P_k = expm(t_b r_k Q_k) with t the tree lengths in `length`;
+ *   partials   class k's stored partials at partials + k * partials_class_stride (doubles), each
+ *              [n_store][S][site_stride];
+ *   dwell_sum  [K][S] and trans_sum [K][S*S] += the statistics of the histories of each class;
+ *              dwell and event times are in tree time;
+ *   site_status  the mixture's (0 where some class is feasible);
+ *   sweep_count  must be NULL (these draws are not a sweep of one MJP's chain).
+ * class_post [K][class_post_stride] fp64, class_post_stride >= n_sites; site_class [traj_stride]
+ * uint8: the class drawn for trajectory t (written where the site's status is 0).  1 <= K <= 255.
+ * Philox4x32-10 keyed by (seed; traj0 + t, k) as in rt_posterior_draw: the class is drawn by the
+ * rule of the node states (the first class of positive weight whose cumulative weight reaches
+ * x = (u + 1/2) 2^-32 sum_k class_post) from u = word 0 of (substream 2, block 0); the history
+ * uses substream 1 as in rt_posterior_draw, so with K = 1 it is bit for bit that draw.
+ */
+typedef struct rt_posterior_draw_mixture_args {
+  rt_posterior_draw_args base;
+  int32_t K, reserved;
+  int64_t partials_class_stride, class_post_stride;
+  const double* class_post;
+  uint8_t* site_class;
+} rt_posterior_draw_mixture_args;
+
+int rt_posterior_draw_mixture(const rt_posterior_draw_mixture_args* args, void* stream);
+
+/*
  * Warp-cooperative Rao-Teh kernels: one warp per (chain, site) trajectory.
  *
  * (1) Rao-Teh sweeps for S = 7 and 9 <= S <= 64 primary states (rt_raoteh_sweeps dispatches

@@ -127,6 +127,19 @@ class PosteriorDrawArgs(ctypes.Structure):
 EXPORTS['rt_posterior_draw'] = ([ctypes.POINTER(PosteriorDrawArgs), c_void_p], c_int)
 
 
+class PosteriorDrawMixtureArgs(ctypes.Structure):
+    """Mirror of `rt_posterior_draw_mixture_args` (include/rt_b200.h)."""
+    _fields_ = [
+        ('base', PosteriorDrawArgs),
+        ('K', ctypes.c_int32), ('reserved', ctypes.c_int32),
+        ('partials_class_stride', c_int64), ('class_post_stride', c_int64),
+        ('class_post', c_void_p), ('site_class', c_void_p),
+    ]
+
+
+EXPORTS['rt_posterior_draw_mixture'] = ([ctypes.POINTER(PosteriorDrawMixtureArgs), c_void_p], c_int)
+
+
 class NativeError(RuntimeError):
     pass
 

@@ -88,10 +88,11 @@ int rt_raoteh_dispatch(const rt_raoteh_args&, cudaStream_t);
 int rt_tmjp_dispatch(const rt_tmjp_args&, cudaStream_t);
 
 int rt_posterior_draw_dispatch(const rt_posterior_draw_args&, cudaStream_t);
+int rt_posterior_draw_mixture_dispatch(const rt_posterior_draw_mixture_args&, cudaStream_t);
 
 extern "C" {
 
-int rt_version(void) { return 203; }
+int rt_version(void) { return 204; }
 
 int rt_release_workspace(void) {
   int dev = 0;
@@ -338,9 +339,10 @@ int rt_raoteh_sweeps(int S, int n_nodes, int64_t n_traj, int64_t traj_stride, in
   return raoteh_run_impl(R, stream);
 }
 
-int rt_posterior_draw(const rt_posterior_draw_args* args, void* stream) {
-  if (!args) return arg_error("null pointer");
-  const rt_posterior_draw_args& R = *args;
+}  // extern "C"
+
+// the checks of rt_posterior_draw; RT_OK if the arguments are valid
+static int posterior_draw_check(const rt_posterior_draw_args& R) {
   if (!R.program || !R.parent || !R.length || !R.Q || !R.P || !R.obs || !R.partials ||
       !R.node_state || !R.ev_time || !R.ev_sb || !R.ev_count || !R.ev_total || !R.status)
     return arg_error("null pointer");
@@ -352,8 +354,34 @@ int rt_posterior_draw(const rt_posterior_draw_args* args, void* stream) {
   if (R.site_stride < R.n_sites) return arg_error("site_stride < n_sites");
   if (R.k < 0 || R.k >= INT32_MAX) return arg_error("draw index k out of range");
   if (R.n_ops <= 0 || R.n_nodes <= 1) return arg_error("empty program");
+  return RT_OK;
+}
+
+extern "C" {
+
+int rt_posterior_draw(const rt_posterior_draw_args* args, void* stream) {
+  if (!args) return arg_error("null pointer");
+  const rt_posterior_draw_args& R = *args;
+  int rc = posterior_draw_check(R);
+  if (rc != RT_OK) return rc;
   if (R.n_traj <= 0) return RT_OK;
-  int rc = rt_posterior_draw_dispatch(R, (cudaStream_t)stream);
+  rc = rt_posterior_draw_dispatch(R, (cudaStream_t)stream);
+  if (rc == RT_ERR_UNSUPPORTED) snprintf(g_err, sizeof(g_err), "unsupported: S or shared-memory budget");
+  return rc;
+}
+
+int rt_posterior_draw_mixture(const rt_posterior_draw_mixture_args* args, void* stream) {
+  if (!args) return arg_error("null pointer");
+  const rt_posterior_draw_mixture_args& M = *args;
+  int rc = posterior_draw_check(M.base);
+  if (rc != RT_OK) return rc;
+  if (M.K < 1 || M.K > 255) return arg_error("rt_posterior_draw_mixture needs 1 <= K <= 255");
+  if (!M.class_post || !M.site_class) return arg_error("null pointer");
+  if (M.class_post_stride < M.base.n_sites) return arg_error("class_post_stride < n_sites");
+  if (M.partials_class_stride < 0) return arg_error("partials_class_stride < 0");
+  if (M.base.sweep_count) return arg_error("rt_posterior_draw_mixture takes no sweep_count");
+  if (M.base.n_traj <= 0) return RT_OK;
+  rc = rt_posterior_draw_mixture_dispatch(M, (cudaStream_t)stream);
   if (rc == RT_ERR_UNSUPPORTED) snprintf(g_err, sizeof(g_err), "unsupported: S or shared-memory budget");
   return rc;
 }

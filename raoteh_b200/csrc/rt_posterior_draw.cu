@@ -78,8 +78,8 @@ template <> __device__ __forceinline__ double next_down(double x) { return nexta
 // One block: mu = max_s q_s (1 if Q is zero), n_pow from the Poisson tail at mu * max_b t_b
 // (capped at kMaxPow), then Bt[m] = (B^m)^T for m = 0..n_pow.
 template <int S>
-__global__ void power_table_kernel(const double* __restrict__ Q, const double* __restrict__ length,
-                                   int n_nodes, double* __restrict__ ws) {
+__device__ __forceinline__ void power_table(const double* __restrict__ Q, const double* __restrict__ length,
+                                            int n_nodes, double* __restrict__ ws) {
   __shared__ double B_s[S * S], cur[S * S];
   __shared__ int n_pow_s;
   __shared__ double mu_s;
@@ -132,6 +132,23 @@ __global__ void power_table_kernel(const double* __restrict__ Q, const double* _
   }
 }
 
+template <int S>
+__global__ void power_table_kernel(const double* __restrict__ Q, const double* __restrict__ length,
+                                   int n_nodes, double* __restrict__ ws) {
+  power_table<S>(Q, length, n_nodes, ws);
+}
+
+// doubles of one power table in the workspace
+template <int S>
+constexpr size_t table_size() { return kHeader + (size_t)(kMaxPow + 1) * S * S; }
+
+// block c: the table of class c, generator Q + c S^2, at ws + c * table_size
+template <int S>
+__global__ void power_table_classes_kernel(const double* __restrict__ Q, const double* __restrict__ length,
+                                           int n_nodes, double* __restrict__ ws) {
+  power_table<S>(Q + (size_t)blockIdx.x * S * S, length, n_nodes, ws + blockIdx.x * table_size<S>());
+}
+
 template <typename TT>
 struct DrawArgs {
   int n_nodes, n_ops, cap;
@@ -158,232 +175,82 @@ struct DrawArgs {
   int8_t* status;
 };
 
+// the site-class mixture's additions (posterior_draw_mixture_kernel): P, partials, power tables
+// and statistics are per class, the class drawn per trajectory from class_post [K][stride]
+struct MixArgs {
+  int K;
+  int64_t partials_class_stride, class_post_stride;
+  const double* class_post;
+  uint8_t* site_class;
+};
+
+// p + off for the mixture kernel's per-class inputs; the single-class kernel's pointer untouched
+template <bool MIX>
+__device__ __forceinline__ const double* at_class(const double* p, size_t off) {
+  if constexpr (MIX) return p + off;
+  else return p;
+}
+
+// class ~ w[k * stride], k < K: draw_categorical's rule; -1 if every weight is 0
+__device__ __forceinline__ int draw_class(const double* w, int64_t stride, int K, uint32_t u) {
+  double tot = 0.0;
+  for (int k = 0; k < K; ++k) tot += w[k * stride];
+  if (!(tot > 0.0)) return -1;
+  const double x = ((double)u + 0.5) * 2.3283064365386963e-10 * tot;
+  double cum = 0.0;
+  int last = -1;
+  for (int k = 0; k < K; ++k) {
+    const double wk = w[k * stride];
+    cum += wk;
+    if (wk > 0.0) {
+      last = k;
+      if (x <= cum) break;
+    }
+  }
+  return last;
+}
+
 template <int S, int OBS, bool STATS, typename TT>
 __global__ void __launch_bounds__(kBlock, 4)
 posterior_draw_kernel(DrawArgs<TT> A) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  int4* prog_s = reinterpret_cast<int4*>(smem_raw);
-  double* B_s = reinterpret_cast<double*>(prog_s + A.n_ops);          // [S][S]
-  double* pi_s = B_s + S * S;                                          // [S]
-  double* len_s = pi_s + S;                                            // [n_nodes]
-  double* dwell_s = len_s + A.n_nodes;                                 // [S][kBlock]
-  uint32_t* trans_s = reinterpret_cast<uint32_t*>(dwell_s + (STATS ? S * kBlock : 0));   // [S*S][kBlock]
-  int* par_s = reinterpret_cast<int*>(trans_s + (STATS ? S * S * kBlock : 0));           // [n_nodes]
-  __shared__ double red[kBlock / 32][S * S + S];
-
-  const int tid = threadIdx.x;
-  const double mu = A.ws[0];
-  const int n_pow = (int)A.ws[1];
-  const double* Bt = A.ws + kHeader;
-  for (int i = tid; i < A.n_ops; i += kBlock) prog_s[i] = A.program[i];
-  for (int i = tid; i < S * S; i += kBlock) B_s[i] = Bt[S * S + (i % S) * S + i / S];
-  if (tid < S) pi_s[tid] = A.root_distn ? A.root_distn[tid] : 1.0;
-  for (int i = tid; i < A.n_nodes; i += kBlock) { len_s[i] = A.length[i]; par_s[i] = A.parent[i]; }
-  if (STATS) {
-#pragma unroll
-    for (int s = 0; s < S; ++s) dwell_s[s * kBlock + tid] = 0.0;
-#pragma unroll
-    for (int q = 0; q < S * S; ++q) trans_s[q * kBlock + tid] = 0u;
-  }
-  __syncthreads();
-
-  const int64_t traj = (int64_t)blockIdx.x * kBlock + tid;
-  const int64_t site = traj < A.n_traj ? (A.traj0 + traj) % A.n_sites : 0;
-  bool active = traj < A.n_traj && A.status[traj] == RT_SITE_OK;
-  if (active && A.site_status && A.site_status[site] != RT_SITE_OK) {
-    A.status[traj] = A.site_status[site];
-    active = false;
-  }
-
-  if (active) {
-    const int64_t st = A.stride;
-    uint8_t* ns_p = A.node_state + traj;
-    uint8_t* cnt_p = A.ev_count + traj;
-    TT* evt_p = A.ev_time + (size_t)traj * A.cap;
-    uint8_t* evs_p = A.ev_sb + (size_t)traj * A.cap;
-    Philox rng;
-    rng.init(A.seed, (uint64_t)(A.traj0 + traj), (uint32_t)A.k);
-    // substream 1: the draw's own words (a sweep uses substream 0); word 0 draws the root, words
-    // 2 and 3 seed the PCG32 stream of everything else, as in the sweeps
-    rng.block(1u, 0u);
-    uint64_t pcg_state = ((uint64_t)rng.out[3] << 32) | (uint64_t)rng.out[2];
-    const uint64_t pcg_inc = ((uint64_t)(A.traj0 + traj) << 1) | 1ull;
-    auto pcg_next = [&]() -> uint32_t {
-      const uint64_t old = pcg_state;
-      pcg_state = old * 6364136223846793005ull + pcg_inc;
-      const uint32_t xs = (uint32_t)(((old >> 18) ^ old) >> 27);
-      const uint32_t rot = (uint32_t)(old >> 59);
-      return (xs >> rot) | (xs << ((32u - rot) & 31u));
-    };
-    pcg_next();
-    auto unit = [&]() -> double { return ((double)pcg_next() + 0.5) * 2.3283064365386963e-10; };
-
-    int8_t fail = RT_SITE_OK;
-    // ---- root ~ pi * L_root (store index of the OP_ROOT op) ----
-    {
-      const int4 op = prog_s[A.n_ops - 1];
-      const double* Lp = A.partials + (int64_t)op.w * S * A.site_stride + site;
-      double w[S], tot = 0.0;
-#pragma unroll
-      for (int s = 0; s < S; ++s) { w[s] = pi_s[s] * Lp[(int64_t)s * A.site_stride]; tot += w[s]; }
-      if (!(tot > 0.0)) fail = RT_SITE_STRUCTURAL_ZERO;
-      else ns_p[(int64_t)op.y * st] = (uint8_t)draw_categorical<S>(w, tot, rng.out[0]);
-    }
-    int wr = A.cap;
-    for (int ip = A.n_ops - 1; ip >= 0 && fail == RT_SITE_OK; --ip) {
-      const int4 op = prog_s[ip];
-      const int code = op.x & 0xff;
-      if (code > OP_MSG_ONES) continue;
-      const int c = op.y;
-      const int xa = ns_p[(int64_t)par_s[c] * st];
-      // ---- node state: x_c ~ P_c[x_a, :] * L_c ----
-      double L[S];
-      if (code == OP_MSG_SLOT) {
-        const double* Lp = A.partials + (int64_t)op.w * S * A.site_stride + site;
-#pragma unroll
-        for (int s = 0; s < S; ++s) L[s] = Lp[(int64_t)s * A.site_stride];
-      } else if (code == OP_MSG_OBS) {
-        load_obs_vec<S, OBS>(A.obs, op.z, A.obs_stride, site, L);
-      } else {
-#pragma unroll
-        for (int s = 0; s < S; ++s) L[s] = 1.0;
-      }
-      const double* Prow = A.P + ((size_t)c * S + xa) * S;
-      double w[S], tot = 0.0;
-#pragma unroll
-      for (int s = 0; s < S; ++s) { w[s] = __ldg(Prow + s) * L[s]; tot += w[s]; }
-      if (!(tot > 0.0)) { fail = RT_SITE_STRUCTURAL_ZERO; break; }
-      const int xc = draw_categorical<S>(w, tot, pcg_next());
-      ns_p[(int64_t)c * st] = (uint8_t)xc;
-
-      // ---- path on the branch given (x_a, x_c, t_c) ----
-      const double tc = len_s[c];
-      int kept = 0;
-      int x = xa;
-      TT prev = (TT)0;
-      if (tc > 0.0) {
-        // largest stored time: the largest TT value below t_c
-        TT hi = (TT)tc;
-        if (!((double)hi < tc)) hi = next_down(hi);
-        const double lam = mu * tc;
-        const double* Btc = Bt + (size_t)xc * S;          // Bt[m][xc][s] = (B^m)[s][xc]
-        // Pr(N = n) ~ Pois(n; lam) (B^n)[xa, xc]: sum of the series up to n_pow, or until the
-        // Poisson tail cannot move it (for n > lam the tail is below p_n r / (1 - r))
-        double p = exp(-lam), tot_n = 0.0;
-        int n_end = n_pow;
-        for (int n = 0; n <= n_pow; ++n) {
-          tot_n = fma(p, __ldg(Btc + (size_t)n * S * S + xa), tot_n);
-          const double r = lam / (n + 1);
-          if (r < 0.5 && tot_n > 0.0 && p * 2.0 * r < kTailEps * tot_n) { n_end = n; break; }
-          p *= r;
-        }
-        const double pac = __ldg(Prow + xc);
-        // truncation guard: the series must reach P_c[xa, xc] (1e-14 absolute: the accuracy of
-        // the smallest entries of expm)
-        if (!(tot_n > 0.0) || tot_n < pac * (1.0 - 1e-12) - 1e-14) { fail = 3; break; }
-        const double xu = unit() * tot_n;
-        int N = -1;
-        {
-          double q = exp(-lam), cum = 0.0;
-          int last = 0;            // rounding past the end: the last n of positive weight
-          for (int n = 0; n <= n_end; ++n) {
-            const double wn = q * __ldg(Btc + (size_t)n * S * S + xa);
-            cum += wn;
-            if (wn > 0.0) {
-              last = n;
-              if (xu <= cum) { N = n; break; }
-            }
-            q *= lam / (n + 1);
-          }
-          if (N < 0) N = last;
-        }
-        // events 1..N: state given the previous one and the end state, time as the next order
-        // statistic of N uniforms on (0, 1): U_(i) = 1 - (1 - U_(i-1)) V^(1 / (N - i + 1))
-        double u_prev = 0.0;
-        for (int i = 1; i <= N; ++i) {
-          const double v = unit();
-          const double u_i = 1.0 - (1.0 - u_prev) * exp(log(v) / (double)(N - i + 1));
-          u_prev = u_i;
-          int nx = xc;
-          if (i < N) {
-            const double* Bm = Btc + (size_t)(N - i) * S * S;
-            double ws[S], tw = 0.0;
-#pragma unroll
-            for (int s = 0; s < S; ++s) { ws[s] = B_s[x * S + s] * __ldg(Bm + s); tw += ws[s]; }
-            nx = tw > 0.0 ? draw_categorical<S>(ws, tw, pcg_next()) : -1;
-            if (nx < 0) { fail = 3; break; }
-          }
-          if (nx == x) continue;
-          // a real jump: stored strictly inside (0, t_c) and after the previous one in TT
-          TT tau = (TT)(u_i * tc);
-          if (tau > hi) tau = hi;
-          if (!(tau > prev)) tau = next_up(prev);
-          if (tau > hi) { fail = 3; break; }
-          if (STATS) {
-            dwell_s[x * kBlock + tid] += (double)(tau - prev);
-            trans_s[(x * S + nx) * kBlock + tid] += 1u;
-          }
-          --wr;
-          if (wr >= 0) { evt_p[wr] = tau; evs_p[wr] = (uint8_t)x; }
-          prev = tau;
-          ++kept;
-          x = nx;
-        }
-        if (fail != RT_SITE_OK) break;
-        if (kept > 255) { fail = 3; break; }
-      }
-      if (STATS) dwell_s[x * kBlock + tid] += tc - (double)prev;
-      cnt_p[(int64_t)c * st] = (uint8_t)kept;
-    }
-    if (fail == RT_SITE_OK && wr < 0) fail = 4;
-    if (fail != RT_SITE_OK) {
-      A.status[traj] = fail;
-      A.ev_total[traj] = 0;
-    } else {
-      A.ev_total[traj] = A.cap - wr;
-      if (A.sweep_count) A.sweep_count[traj] = (int32_t)(A.k + 1);
-    }
-  }
-
-  if (STATS && A.dwell_sum) {
-#pragma unroll
-    for (int q = 0; q < S + S * S; ++q) {
-      const double mine = q < S ? dwell_s[(q < S ? q : 0) * kBlock + tid]
-                                : (double)trans_s[(q >= S ? q - S : 0) * kBlock + tid];
-      const double v = rt_warp_sum(mine);
-      if ((tid & 31) == 0) red[tid >> 5][q] = v;
-    }
-    __syncthreads();
-    if (tid < S + S * S) {
-      double t = 0.0;
-      for (int i = 0; i < kBlock / 32; ++i) t += red[i][tid];
-      if (t != 0.0) atomicAdd(tid < S ? &A.dwell_sum[tid] : &A.trans_sum[tid - S], t);
-    }
-  }
+  constexpr bool MIX = false;
+  [[maybe_unused]] const MixArgs X{};
+#include "rt_posterior_draw_walk.cuh"
 }
 
-template <int S, int OBS, typename TT>
-int launch(const DrawArgs<TT>& A, bool stats, cudaStream_t stream) {
+template <int S, int OBS, bool STATS, typename TT>
+__global__ void __launch_bounds__(kBlock, 4)
+posterior_draw_mixture_kernel(DrawArgs<TT> A, MixArgs X) {
+  constexpr bool MIX = true;
+#include "rt_posterior_draw_walk.cuh"
+}
+
+template <int S, int OBS, bool MIX, typename TT>
+int launch(const DrawArgs<TT>& A, const MixArgs& X, bool stats, cudaStream_t stream) {
   const size_t smem = sizeof(int4) * A.n_ops + sizeof(double) * (S * S + S + A.n_nodes) +
                       (stats ? sizeof(double) * S * kBlock + sizeof(uint32_t) * S * S * kBlock : 0) +
-                      sizeof(int) * A.n_nodes + 16;
+                      sizeof(int) * A.n_nodes + (MIX ? sizeof(uint32_t) * 8 + kBlock : 0) + 16;
   if (smem > 200 * 1024) return RT_ERR_UNSUPPORTED;
   const unsigned grid = (unsigned)((A.n_traj + kBlock - 1) / kBlock);
-  if (stats) {
-    auto kern = posterior_draw_kernel<S, OBS, true, TT>;
+  auto go = [&](auto kern, auto... extra) -> int {
     RT_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, kBlock, smem, stream>>>(A);
-  } else {
-    auto kern = posterior_draw_kernel<S, OBS, false, TT>;
-    RT_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, kBlock, smem, stream>>>(A);
-  }
+    kern<<<grid, kBlock, smem, stream>>>(A, extra...);
+    return RT_OK;
+  };
+  int rc;
+  if constexpr (MIX)
+    rc = stats ? go(posterior_draw_mixture_kernel<S, OBS, true, TT>, X)
+               : go(posterior_draw_mixture_kernel<S, OBS, false, TT>, X);
+  else
+    rc = stats ? go(posterior_draw_kernel<S, OBS, true, TT>) : go(posterior_draw_kernel<S, OBS, false, TT>);
+  if (rc != RT_OK) return rc;
   RT_CUDA_CHECK(cudaGetLastError());
   return RT_OK;
 }
 
+// K = 0: rt_posterior_draw (one power table from Q); K >= 1: the mixture (K tables, one block each)
 template <int S, typename TT>
-int launch_s(const rt_posterior_draw_args& R, const double* ws, cudaStream_t stream) {
+int launch_s(const rt_posterior_draw_args& R, const MixArgs& X, const double* ws, cudaStream_t stream) {
   DrawArgs<TT> A;
   A.n_nodes = R.n_nodes; A.n_ops = R.n_ops; A.cap = R.cap;
   A.n_traj = R.n_traj; A.stride = R.traj_stride; A.n_sites = R.n_sites; A.traj0 = R.traj0;
@@ -396,39 +263,59 @@ int launch_s(const rt_posterior_draw_args& R, const double* ws, cudaStream_t str
   A.ev_count = R.ev_count; A.ev_total = R.ev_total; A.sweep_count = R.sweep_count;
   A.dwell_sum = R.dwell_sum; A.trans_sum = R.trans_sum; A.status = R.status;
   const bool stats = R.dwell_sum != nullptr && R.trans_sum != nullptr;
-  power_table_kernel<S><<<1, 64, 0, stream>>>(R.Q, R.length, R.n_nodes, const_cast<double*>(ws));
+  if (X.K == 0) {
+    power_table_kernel<S><<<1, 64, 0, stream>>>(R.Q, R.length, R.n_nodes, const_cast<double*>(ws));
+    RT_CUDA_CHECK(cudaGetLastError());
+    if (R.obs_kind == OBS_CODES) return launch<S, OBS_CODES, false, TT>(A, X, stats, stream);
+    return launch<S, OBS_MASK, false, TT>(A, X, stats, stream);
+  }
+  power_table_classes_kernel<S><<<X.K, 64, 0, stream>>>(R.Q, R.length, R.n_nodes, const_cast<double*>(ws));
   RT_CUDA_CHECK(cudaGetLastError());
-  if (R.obs_kind == OBS_CODES) return launch<S, OBS_CODES, TT>(A, stats, stream);
-  return launch<S, OBS_MASK, TT>(A, stats, stream);
+  if (R.obs_kind == OBS_CODES) return launch<S, OBS_CODES, true, TT>(A, X, stats, stream);
+  return launch<S, OBS_MASK, true, TT>(A, X, stats, stream);
 }
 
 template <int S>
-int dispatch_s(const rt_posterior_draw_args& R, const double* ws, cudaStream_t stream) {
+int dispatch_s(const rt_posterior_draw_args& R, const MixArgs& X, const double* ws, cudaStream_t stream) {
   if (R.time_f64) {
     if constexpr (S == 7) return RT_ERR_UNSUPPORTED;
-    else return launch_s<S, double>(R, ws, stream);
+    else return launch_s<S, double>(R, X, ws, stream);
   }
-  return launch_s<S, float>(R, ws, stream);
+  return launch_s<S, float>(R, X, ws, stream);
+}
+
+int draw_dispatch(const rt_posterior_draw_args& R, const MixArgs& X, cudaStream_t stream) {
+  const int S = R.S;
+  double* ws = nullptr;
+  const size_t bytes = sizeof(double) * (X.K > 0 ? X.K : 1) * (kHeader + (size_t)(kMaxPow + 1) * S * S);
+  RT_CUDA_CHECK(rt_ws_alloc((void**)&ws, bytes, stream));
+  int rc;
+  switch (S) {
+    case 2: rc = dispatch_s<2>(R, X, ws, stream); break;
+    case 3: rc = dispatch_s<3>(R, X, ws, stream); break;
+    case 4: rc = dispatch_s<4>(R, X, ws, stream); break;
+    case 5: rc = dispatch_s<5>(R, X, ws, stream); break;
+    case 6: rc = dispatch_s<6>(R, X, ws, stream); break;
+    case 7: rc = dispatch_s<7>(R, X, ws, stream); break;
+    case 8: rc = dispatch_s<8>(R, X, ws, stream); break;
+    default: rc = RT_ERR_UNSUPPORTED;
+  }
+  rt_ws_free(ws, stream);
+  return rc;
 }
 
 }  // namespace
 
 int rt_posterior_draw_dispatch(const rt_posterior_draw_args& R, cudaStream_t stream) {
-  const int S = R.S;
-  double* ws = nullptr;
-  const size_t bytes = sizeof(double) * (kHeader + (size_t)(kMaxPow + 1) * S * S);
-  RT_CUDA_CHECK(rt_ws_alloc((void**)&ws, bytes, stream));
-  int rc;
-  switch (S) {
-    case 2: rc = dispatch_s<2>(R, ws, stream); break;
-    case 3: rc = dispatch_s<3>(R, ws, stream); break;
-    case 4: rc = dispatch_s<4>(R, ws, stream); break;
-    case 5: rc = dispatch_s<5>(R, ws, stream); break;
-    case 6: rc = dispatch_s<6>(R, ws, stream); break;
-    case 7: rc = dispatch_s<7>(R, ws, stream); break;
-    case 8: rc = dispatch_s<8>(R, ws, stream); break;
-    default: rc = RT_ERR_UNSUPPORTED;
-  }
-  rt_ws_free(ws, stream);
-  return rc;
+  return draw_dispatch(R, MixArgs{}, stream);
+}
+
+int rt_posterior_draw_mixture_dispatch(const rt_posterior_draw_mixture_args& M, cudaStream_t stream) {
+  MixArgs X;
+  X.K = M.K;
+  X.partials_class_stride = M.partials_class_stride;
+  X.class_post_stride = M.class_post_stride;
+  X.class_post = M.class_post;
+  X.site_class = M.site_class;
+  return draw_dispatch(M.base, X, stream);
 }

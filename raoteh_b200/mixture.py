@@ -178,3 +178,144 @@ class SiteMixtureMJP(object):
             b = m.branch_expectations(obs, E=E)['branch'] * cp[k][None, :]
             branch = b if branch is None else branch.add_(b)
         return dict(branch=branch, loglik=mix['loglik'], status=mix['status'], class_post=cp)
+
+    def history_draws(self, obs, n_chains=1, seed=0, cap=96, time_dtype='float32', traj0=0,
+                      n_traj=None):
+        """Exact posterior draws of (class, history) per site under the mixture (stochastic mapping
+        under +G, +I or omega classes): see MixtureHistoryDraws.  2..8 states, hard codes or
+        allowed-state masks."""
+        return MixtureHistoryDraws(self, obs, n_chains=n_chains, seed=seed, cap=cap,
+                                   time_dtype=time_dtype, traj0=traj0, n_traj=n_traj)
+
+
+class MixtureHistoryDraws(object):
+    """n_chains x n_sites iid exact draws from p(class, history | data) of a SiteMixtureMJP
+    (rt_posterior_draw_mixture): each trajectory draws its site's class from the class posterior,
+    then the whole history from that class's P, pruning partials and uniformization (the
+    single-class draw of RaoTehChains.draw_posterior).  A fast site gets the jumps of its rate class
+    and a site drawn into the +I class none.
+
+    Trajectory arrays as RaoTehChains (trajectory t = chain * n_sites + site; this object may own
+    the shard [traj0, traj0 + n_traj)): node_state, ev_count, ev_total, ev_time, ev_sb, status,
+    plus site_class [n_traj] (uint8); draw(stats=True) accumulates dwell_class [K, S] (tree time)
+    and trans_class [K, S, S].  Draw k is keyed by (seed; traj0 + t, k), so shards and repeats
+    reproduce it bit for bit.
+
+    There is no sweep(): the draws are iid, so Rao-Teh sweeps are not needed, and a sweep under a
+    mixture would have to update the class inside the sweep, which is not implemented.
+
+    Memory: every class's up-pass partials are kept, K x n_store x S x 8 bytes per site (about
+    100 MB for K = 5 at 4 states, 63 stored nodes and 1e4 sites; about 10 GB at 1e6 sites), plus
+    the class P and the per-site class posteriors."""
+
+    def __init__(self, mix, obs, n_chains=1, seed=0, cap=96, time_dtype='float32', traj0=0,
+                 n_traj=None):
+        from . import raoteh
+        from .engine import OBS_CODES, OBS_MASK
+        S, K = mix.S, mix.K
+        if not 2 <= S <= 8:
+            raise ValueError('exact history draws support 2..8 states')
+        if obs.kind not in (OBS_CODES, OBS_MASK):
+            raise ValueError('exact history draws take hard codes or allowed-state masks')
+        if time_dtype not in ('float32', 'float64'):
+            raise ValueError("time_dtype must be 'float32' or 'float64'")
+        if time_dtype == 'float64' and S == 7:
+            raise ValueError('fp64 event times are implemented for 2, 3, 4, 5, 6 or 8 states')
+        length = np.asarray(mix.sched.length, dtype=np.float64)
+        gens = [float(mix.rates[k]) * mix.classes[k].Q_host[0] for k in range(K)]
+        for k, G in enumerate(gens):
+            n_pow = raoteh.draw_power_table_length(G, length)
+            if n_pow > raoteh.DRAW_MAX_POW:
+                raise ValueError(
+                    'class %d (rate %g) has a branch too long for the exact draw: max_s q_s * rate * '
+                    'length = %.0f needs B^n up to n = %d, more than %d; subdivide long branches '
+                    'with degree-two nodes (lowering.subdivide_long_branches)'
+                    % (k, mix.rates[k], float(-np.diag(G).min()) * float(length.max()), n_pow,
+                       raoteh.DRAW_MAX_POW))
+        self.mix, self.obs, self.S, self.K = mix, obs, S, K
+        self.sched, self.device = mix.sched, mix.device
+        dev = self.device
+        self.n_sites, self.n_chains = obs.n_sites, int(n_chains)
+        self.traj0 = int(traj0)
+        self.n_traj = T = self.n_chains * self.n_sites if n_traj is None else int(n_traj)
+        self.cap, self.seed, self.time_dtype = int(cap), int(seed), time_dtype
+        self._tt = torch.float64 if time_dtype == 'float64' else torch.float32
+        self._max_rate_length = max(float(-np.diag(G).min()) for G in gens) * float(length.max())
+        # inputs, built once: class generators r_k Q_k, class P on lengths r_k t, every class's
+        # up-pass partials in its own slice (the classes share one workspace), class posteriors
+        self.Q = torch.from_numpy(np.ascontiguousarray(np.stack(gens))).to(dev)
+        n, ns, stride = self.sched.n, self.sched.n_store, obs.stride
+        self.P = torch.empty((K, n, S, S), dtype=torch.float64, device=dev)
+        self.partials = torch.empty((K, ns, S, stride), dtype=torch.float64, device=dev)
+        lik = mix.log_likelihood(obs)
+        self.class_post = lik['class_post'].contiguous()
+        self.site_status = lik['status'].contiguous()
+        for k, m in enumerate(mix.classes):
+            self.P[k].copy_(m.transition_matrices())
+            self.partials[k].copy_(m.log_likelihood(obs, keep_partials=True)['partials'])
+        ops, _ = self.sched.up_program(obs.obs_slot)
+        self.ops, self.n_ops = torch.from_numpy(ops).to(dev), len(ops)
+        self.parent = torch.from_numpy(self.sched.parent.copy()).to(dev)
+        self.stride = T
+        self.node_state = torch.zeros((n, T), dtype=torch.uint8, device=dev)
+        self.ev_count = torch.zeros((n, T), dtype=torch.uint8, device=dev)
+        self.ev_total = torch.zeros(T, dtype=torch.int32, device=dev)
+        self.ev_time = torch.zeros((T, self.cap), dtype=self._tt, device=dev)
+        self.ev_sb = torch.zeros((T, self.cap), dtype=torch.uint8, device=dev)
+        self.status = torch.zeros(T, dtype=torch.int8, device=dev)
+        self.site_class = torch.zeros(T, dtype=torch.uint8, device=dev)
+        self.dwell_class = torch.zeros((K, S), dtype=torch.float64, device=dev)
+        self.trans_class = torch.zeros((K, S, S), dtype=torch.float64, device=dev)
+        self.draws_done = 0
+
+    def _args(self, stats):
+        from . import _native
+        from .engine import _ptr
+        A = _native.PosteriorDrawMixtureArgs()
+        B = A.base
+        B.S, B.n_nodes, B.n_ops, B.cap = self.S, self.sched.n, self.n_ops, self.cap
+        B.obs_kind, B.time_f64 = self.obs.kind, 1 if self.time_dtype == 'float64' else 0
+        B.n_traj, B.traj_stride, B.n_sites, B.traj0 = self.n_traj, self.stride, self.n_sites, self.traj0
+        B.obs_stride, B.site_stride = self.obs.stride, self.obs.stride
+        B.seed, B.k = self.seed, self.draws_done
+        B.program, B.parent, B.length = _ptr(self.ops), _ptr(self.parent), _ptr(self.mix.length)
+        B.Q, B.P, B.root_distn = _ptr(self.Q), _ptr(self.P), _ptr(self.mix.classes[0].root_distn)
+        B.obs, B.partials, B.site_status = _ptr(self.obs.data), _ptr(self.partials), _ptr(self.site_status)
+        B.node_state, B.ev_time, B.ev_sb = _ptr(self.node_state), _ptr(self.ev_time), _ptr(self.ev_sb)
+        B.ev_count, B.ev_total, B.sweep_count = _ptr(self.ev_count), _ptr(self.ev_total), None
+        B.dwell_sum = _ptr(self.dwell_class) if stats else None
+        B.trans_sum = _ptr(self.trans_class) if stats else None
+        B.status = _ptr(self.status)
+        A.K = self.K
+        A.partials_class_stride = self.partials[0].numel()
+        A.class_post_stride = self.class_post.shape[1]
+        A.class_post, A.site_class = _ptr(self.class_post), _ptr(self.site_class)
+        return A
+
+    def draw(self, stats=True):
+        """Replace every trajectory with a new iid draw (index k = draws_done); stats=True adds the
+        drawn histories' statistics to dwell_class / trans_class."""
+        import ctypes
+        from . import _native
+        from .engine import _stream
+        self.status.zero_()
+        A = self._args(stats)
+        rc = _native.lib().rt_posterior_draw_mixture(ctypes.byref(A), _stream())
+        _native.check(rc, 'rt_posterior_draw_mixture')
+        self.draws_done += 1
+        self.check()
+
+    def trajectory(self, t):
+        """Trajectory t as (node states, dict child node -> (times, segment states)), as
+        RaoTehChains.trajectory."""
+        from .raoteh import trajectory_edges
+        return trajectory_edges(self.ops, self.node_state, self.ev_count, self.ev_total, self.ev_time,
+                                self.ev_sb, self.cap, t)
+
+    def check(self):
+        from .raoteh import check_status
+        check_status(self.status, self.cap, self._max_rate_length)
+
+    def reset_statistics(self):
+        self.dwell_class.zero_()
+        self.trans_class.zero_()

@@ -39,6 +39,47 @@ def draw_power_table_length(Q, length, eps=1e-17):
     return max(n, 2 * Q.shape[0] + 8)
 
 
+def check_status(status, cap, max_rate_length):
+    """Raise NativeError for trajectories with status != 0 (1: no feasible history, 4: more than
+    `cap` real jumps, else out of event capacity); max_rate_length = the largest expected number of
+    events on one branch, for the message."""
+    bad = int((status != 0).sum())
+    if bad and int((status == 1).sum()):
+        raise _native.NativeError('no feasible history (structural zero) for %d trajectories'
+                                  % int((status == 1).sum()))
+    if bad and int((status == 4).sum()):
+        raise _native.NativeError('initial history has more than cap=%d real jumps' % cap)
+    if bad:
+        raise _native.NativeError(
+            '%d trajectories exceeded the event capacity in one sweep (status 3): more than '
+            'cap=%d candidate events in the trajectory, or more than 255 on one branch '
+            '(expected per branch: omega * length, here up to %.0f); re-create the sampler '
+            'with a larger cap, or subdivide long branches with degree-two nodes'
+            % (bad, cap, max_rate_length))
+
+
+def trajectory_edges(ops, node_state, ev_count, ev_total, ev_time, ev_sb, cap, t):
+    """Trajectory t of the trajectory arrays as per-edge arrays: (node states, dict child node ->
+    (times from the parent end, ascending; states of the k+1 segments, parent side first))."""
+    cnt = ev_count[:, t].cpu().numpy().astype(int)
+    tot = int(ev_total[t])
+    times = ev_time[t, cap - tot:].cpu().numpy()
+    sbs = ev_sb[t, cap - tot:].cpu().numpy().astype(int)
+    ns = node_state[:, t].cpu().numpy().astype(int)
+    out = {}
+    pos = 0
+    for code, c, a, b in ops.cpu().numpy():
+        if (code & 0xff) > 2:
+            continue
+        k = cnt[c]
+        tt = times[pos:pos + k][::-1]          # stored child end first
+        sb = sbs[pos:pos + k][::-1]
+        pos += k
+        states = np.concatenate([sb, [ns[c]]]) if k else np.array([ns[c]])
+        out[int(c)] = (tt.astype(float), states)
+    return ns, out
+
+
 class RaoTehChains(object):
     """n_chains x n_sites trajectories of one MJP on one tree.
 
@@ -257,19 +298,7 @@ class RaoTehChains(object):
         self.status[self.status == 3] = 0
 
     def check(self):
-        bad = int((self.status != 0).sum())
-        if bad and int((self.status == 1).sum()):
-            raise _native.NativeError('no feasible history (structural zero) for %d trajectories'
-                                      % int((self.status == 1).sum()))
-        if bad and int((self.status == 4).sum()):
-            raise _native.NativeError('initial history has more than cap=%d real jumps' % self.cap)
-        if bad:
-            raise _native.NativeError(
-                '%d trajectories exceeded the event capacity in one sweep (status 3): more than '
-                'cap=%d candidate events in the trajectory, or more than 255 on one branch '
-                '(expected per branch: omega * length, here up to %.0f); re-create the sampler '
-                'with a larger cap, or subdivide long branches with degree-two nodes'
-                % (bad, self.cap, self.omega * float(self.sched.length.max())))
+        check_status(self.status, self.cap, self.omega * float(self.sched.length.max()))
 
     def reset_statistics(self):
         self.dwell_sum.zero_()
@@ -359,22 +388,5 @@ class RaoTehChains(object):
     def trajectory(self, t):
         """Trajectory t as per-edge arrays: dict child node -> (times from the parent
         end, ascending; states of the k+1 segments, parent side first)."""
-        n = self.sched.n
-        cnt = self.ev_count[:, t].cpu().numpy().astype(int)
-        tot = int(self.ev_total[t])
-        times = self.ev_time[t, self.cap - tot:].cpu().numpy()
-        sbs = self.ev_sb[t, self.cap - tot:].cpu().numpy().astype(int)
-        ns = self.node_state[:, t].cpu().numpy().astype(int)
-        out = {}
-        pos = 0
-        ops = self.ops.cpu().numpy()
-        for code, c, a, b in ops:
-            if (code & 0xff) > 2:
-                continue
-            k = cnt[c]
-            tt = times[pos:pos + k][::-1]          # stored child end first
-            sb = sbs[pos:pos + k][::-1]
-            pos += k
-            states = np.concatenate([sb, [ns[c]]]) if k else np.array([ns[c]])
-            out[int(c)] = (tt.astype(float), states)
-        return ns, out
+        return trajectory_edges(self.ops, self.node_state, self.ev_count, self.ev_total, self.ev_time,
+                                self.ev_sb, self.cap, t)
