@@ -415,6 +415,77 @@ typedef struct rt_posterior_draw_mixture_args {
 int rt_posterior_draw_mixture(const rt_posterior_draw_mixture_args* args, void* stream);
 
 /*
+ * Forward (prior) simulation of n_traj independent sites: the batched replacement of the
+ * reference's jump-by-jump simulator _sampler.get_forward_sample / gen_forward_samples
+ * (raoteh/sampler/_sampler.py:67-235), one history per call there.  Trajectory t (0 <= t < n_traj)
+ * is the global index traj0 + t; every output is written at t.
+ *
+ * Classes (site-class mixtures: +G rates, +I, per-class rate matrices), 1 <= K <= 255: the class c of
+ * a site is drawn first from class_weight [K] (nullable when K = 1) and written to site_class
+ * [traj_stride] (nullable).  Q [K][S][S] holds the class generators r_k Q_k (rate 0: Q = 0, an +I
+ * class), P [K][n_nodes][S][S] their transition matrices expm(t_b r_k Q_k).  root_distn [S] is
+ * nullable, and NULL means UNIFORM here (the pruning calls read NULL as weights of one); it is
+ * normalised, as is every sampled row.  Both modes walk the upward program backwards (parents first):
+ *   RT_SIM_NODES   x_root ~ pi, x_c ~ P_c[x_a, :] with negative round-off clamped to 0 and the row
+ *                  renormalised (as synth.simulate_leaf_codes); P is read, Q and length are not.
+ *   RT_SIM_HISTORY jump by jump on every branch as get_forward_sample: dwell ~ Exp(q_s) with
+ *                  q_s = sum_{s' != s} Q[s][s'], next state ~ Q[s, :] / q_s.  The history is written
+ *                  in the trajectory layout of rt_raoteh_run (node_state, ev_count, ev_total, ev_time,
+ *                  ev_sb; jumps right-aligned at `cap`, upward-program order, child end first, times
+ *                  strictly inside (0, t_b) and strictly increasing in the stored precision), so
+ *                  rt_raoteh_run and rt_tmjp_run (RT_TMJP_TRAJ_LOGLIK) read it unchanged.  ev_time is
+ *                  float, or double with time_f64.  dwell_sum [K][S] / trans_sum [K][S*S] (nullable,
+ *                  together) += the statistics of the simulated histories; they are accumulated in
+ *                  shared memory, K S (8 + 4 S) bytes, which must stay within 160 KiB.  Q and length
+ *                  are read, P is not.
+ *                  status [traj_stride] (required): 0, 3 = more than 255 jumps on one branch (the
+ *                  uint8 counts; subdivide it with degree-two nodes) or a jump time that cannot be
+ *                  stored, 4 = more than `cap` jumps in the trajectory (ev_total is then 0).  The node
+ *                  states and leaf codes of such a site are still a draw from the prior.
+ * node_state [n_nodes][traj_stride]: nullable in RT_SIM_NODES.
+ * Leaf codes: obs (nullable) uint8 [n_slots][obs_stride] in the RT_OBS_CODES layout, obs_stride >=
+ * n_traj; node v with obs_slot[v] >= 0 (obs_slot int32 [n_nodes]) writes its state to row obs_slot[v].
+ * tmpl (nullable) uint8 [n_slots][tmpl_stride], the codes of a real alignment of tmpl_n_sites sites:
+ * where tmpl[obs_slot[v]][(traj0 + t) % tmpl_n_sites] is RT_MISSING (255) the written code is too.
+ * Randomness: Philox4x32-10 keyed by (seed; traj0 + t, k), k the replicate index, on its own
+ * substream 0xffff (the sweeps use 0 and the warp kernel 0 .. (n_parts+2)(n_ops+1)-1 < 65535, the
+ * exact draws 1 and 2): words 0 and 1 draw the class, words 2 and 3 seed the PCG32 stream of every
+ * other draw.  Results do not depend on how sites are split over calls or GPUs.
+ * Every draw reads one entry of a Walker alias table built per call (one per sampled row), so it is
+ * O(1) for every S in 2..64; the tables take 4 bytes per entry: 4 K n_nodes S^2 (NODES) or 4 K S^2.
+ */
+#define RT_SIM_NODES 0
+#define RT_SIM_HISTORY 1
+
+typedef struct rt_forward_args {
+  int32_t S, n_nodes, n_ops, K, mode, cap, time_f64, reserved;
+  int64_t n_traj, traj_stride, traj0, obs_stride, tmpl_stride, tmpl_n_sites;
+  uint64_t seed;
+  int64_t k;
+  const int32_t* program;      /* [n_ops][4] upward program (raoteh_b200/lowering.py) */
+  const int32_t* parent;       /* [n_nodes] */
+  const double* length;        /* [n_nodes] (HISTORY) */
+  const int32_t* obs_slot;     /* [n_nodes], -1 = no leaf row (required with obs) */
+  const double* class_weight;  /* [K] */
+  const double* Q;             /* [K][S][S] (HISTORY) */
+  const double* P;             /* [K][n_nodes][S][S] (NODES) */
+  const double* root_distn;    /* [S], NULL = uniform */
+  const uint8_t* tmpl;
+  uint8_t* obs;
+  uint8_t* site_class;
+  uint8_t* node_state;
+  void* ev_time;
+  uint8_t* ev_sb;
+  uint8_t* ev_count;
+  int32_t* ev_total;
+  double* dwell_sum;
+  double* trans_sum;
+  int8_t* status;
+} rt_forward_args;
+
+int rt_forward_simulate(const rt_forward_args* args, void* stream);
+
+/*
  * Warp-cooperative Rao-Teh kernels: one warp per (chain, site) trajectory.
  *
  * (1) Rao-Teh sweeps for S = 7 and 9 <= S <= 64 primary states (rt_raoteh_sweeps dispatches

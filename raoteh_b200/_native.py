@@ -139,6 +139,28 @@ class PosteriorDrawMixtureArgs(ctypes.Structure):
 
 EXPORTS['rt_posterior_draw_mixture'] = ([ctypes.POINTER(PosteriorDrawMixtureArgs), c_void_p], c_int)
 
+SIM_NODES, SIM_HISTORY = 0, 1
+
+
+class ForwardArgs(ctypes.Structure):
+    """Mirror of `rt_forward_args` (include/rt_b200.h)."""
+    _fields_ = [
+        ('S', ctypes.c_int32), ('n_nodes', ctypes.c_int32), ('n_ops', ctypes.c_int32),
+        ('K', ctypes.c_int32), ('mode', ctypes.c_int32), ('cap', ctypes.c_int32),
+        ('time_f64', ctypes.c_int32), ('reserved', ctypes.c_int32),
+        ('n_traj', c_int64), ('traj_stride', c_int64), ('traj0', c_int64), ('obs_stride', c_int64),
+        ('tmpl_stride', c_int64), ('tmpl_n_sites', c_int64),
+        ('seed', ctypes.c_uint64), ('k', c_int64),
+        ('program', c_void_p), ('parent', c_void_p), ('length', c_void_p), ('obs_slot', c_void_p),
+        ('class_weight', c_void_p), ('Q', c_void_p), ('P', c_void_p), ('root_distn', c_void_p),
+        ('tmpl', c_void_p), ('obs', c_void_p), ('site_class', c_void_p), ('node_state', c_void_p),
+        ('ev_time', c_void_p), ('ev_sb', c_void_p), ('ev_count', c_void_p), ('ev_total', c_void_p),
+        ('dwell_sum', c_void_p), ('trans_sum', c_void_p), ('status', c_void_p),
+    ]
+
+
+EXPORTS['rt_forward_simulate'] = ([ctypes.POINTER(ForwardArgs), c_void_p], c_int)
+
 
 class NativeError(RuntimeError):
     pass

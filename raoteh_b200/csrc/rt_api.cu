@@ -92,7 +92,7 @@ int rt_posterior_draw_mixture_dispatch(const rt_posterior_draw_mixture_args&, cu
 
 extern "C" {
 
-int rt_version(void) { return 204; }
+int rt_version(void) { return 205; }
 
 int rt_release_workspace(void) {
   int dev = 0;
@@ -383,6 +383,44 @@ int rt_posterior_draw_mixture(const rt_posterior_draw_mixture_args* args, void* 
   if (M.base.n_traj <= 0) return RT_OK;
   rc = rt_posterior_draw_mixture_dispatch(M, (cudaStream_t)stream);
   if (rc == RT_ERR_UNSUPPORTED) snprintf(g_err, sizeof(g_err), "unsupported: S or shared-memory budget");
+  return rc;
+}
+
+}  // extern "C"
+
+int rt_forward_simulate_dispatch(const rt_forward_args&, cudaStream_t);
+
+extern "C" {
+
+int rt_forward_simulate(const rt_forward_args* args, void* stream) {
+  if (!args) return arg_error("null pointer");
+  const rt_forward_args& R = *args;
+  if (R.S < 2 || R.S > 64) return unsupported("rt_forward_simulate needs 2 <= S <= 64");
+  if (R.K < 1 || R.K > 255) return arg_error("rt_forward_simulate needs 1 <= K <= 255");
+  if (R.mode != RT_SIM_NODES && R.mode != RT_SIM_HISTORY) return arg_error("mode");
+  if (!R.program || !R.parent) return arg_error("null pointer");
+  if (R.K > 1 && !R.class_weight) return arg_error("class_weight is required when K > 1");
+  if (R.obs && !R.obs_slot) return arg_error("obs needs obs_slot");
+  if (R.tmpl && !R.obs) return arg_error("tmpl without obs");
+  if (R.n_ops <= 0 || R.n_nodes <= 1) return arg_error("empty program");
+  if (R.n_traj < 0 || R.traj0 < 0 || R.traj_stride < R.n_traj) return arg_error("traj_stride < n_traj");
+  if (R.obs && R.obs_stride < R.n_traj) return arg_error("obs_stride < n_traj");
+  if (R.tmpl && (R.tmpl_n_sites <= 0 || R.tmpl_stride < R.tmpl_n_sites)) return arg_error("tmpl_stride / tmpl_n_sites");
+  if (R.k < 0 || R.k >= INT32_MAX) return arg_error("replicate index k out of range");
+  if (R.mode == RT_SIM_NODES) {
+    if (!R.P) return arg_error("null pointer");
+  } else {
+    if (!R.Q || !R.length || !R.node_state || !R.ev_time || !R.ev_sb || !R.ev_count || !R.ev_total ||
+        !R.status)
+      return arg_error("null pointer");
+    if ((R.dwell_sum == nullptr) != (R.trans_sum == nullptr)) return arg_error("dwell_sum and trans_sum go together");
+    if (R.cap <= 0) return arg_error("cap");
+    if (R.time_f64 && (R.S == 7 || R.S > 8)) return unsupported("fp64 event times: S in {2,3,4,5,6,8} only");
+  }
+  if (R.n_traj == 0) return RT_OK;
+  int rc = rt_forward_simulate_dispatch(R, (cudaStream_t)stream);
+  if (rc == RT_ERR_UNSUPPORTED)
+    snprintf(g_err, sizeof(g_err), "unsupported: shared-memory budget (tree size, or K S (8 + 4 S) bytes of statistics)");
   return rc;
 }
 

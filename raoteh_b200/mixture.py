@@ -179,6 +179,23 @@ class SiteMixtureMJP(object):
             branch = b if branch is None else branch.add_(b)
         return dict(branch=branch, loglik=mix['loglik'], status=mix['status'], class_post=cp)
 
+    def simulate(self, n_sites, seed=0, k=0, leaf_nodes=None, missing_like=None, keep_node_states=False,
+                 traj0=0, n_traj=None):
+        """Leaf codes of n_sites sites simulated from the mixture (rt_forward_simulate, RT_SIM_NODES):
+        each site draws its class from the weights, then its node states from that class's P (on
+        lengths r_k t; the +I class keeps the root state everywhere).  The root distribution is the
+        mixture's (None: uniform).  Arguments as simulate.simulate_sites.  Returns (Observations,
+        site_class uint8 [n_traj]), plus the node states [n_nodes, n_traj] with keep_node_states.
+        With K = 1 the codes are bit for bit those of simulate_sites."""
+        from .simulate import _simulate_nodes
+        P = torch.stack([m.transition_matrices() for m in self.classes])
+        w = torch.from_numpy(self.weights.copy()).to(self.device)
+        obs, ns, cls = _simulate_nodes(self.sched, P, w, self.classes[0].root_distn_host, n_sites, seed, k,
+                                       leaf_nodes, missing_like, keep_node_states, traj0, n_traj, self.device)
+        if cls is None:
+            cls = torch.zeros(obs.n_sites, dtype=torch.uint8, device=self.device)
+        return (obs, cls, ns) if keep_node_states else (obs, cls)
+
     def history_draws(self, obs, n_chains=1, seed=0, cap=96, time_dtype='float32', traj0=0,
                       n_traj=None):
         """Exact posterior draws of (class, history) per site under the mixture (stochastic mapping

@@ -365,6 +365,31 @@ class RaoTehChains(object):
             self.sweep_count.fill_(self.sweeps_done)
         self.initialized = True
 
+    def load_trajectories(self, node_state, ev_count, ev_total, ev_time, ev_sb):
+        """Copy in a whole trajectory state in this object's layout (for instance the histories of
+        simulate.ForwardHistories, whose leaves are these observations): node_state / ev_count
+        [n_nodes, n_traj], ev_total [n_traj], ev_time / ev_sb [n_traj, c] with c <= cap (jumps
+        right-aligned; ev_time of this object's time dtype).  The chains are then initialized and
+        the next sweep takes index sweeps_done (sweep_count is set to it where the kernel keeps one)."""
+        n, T = self.sched.n, self.n_traj
+        c = int(ev_time.shape[-1])
+        if tuple(node_state.shape) != (n, T) or tuple(ev_count.shape) != (n, T) or \
+                tuple(ev_total.shape) != (T,) or tuple(ev_time.shape) != (T, c) or tuple(ev_sb.shape) != (T, c):
+            raise ValueError('trajectory arrays must be [n_nodes, n_traj] / [n_traj] / [n_traj, c]')
+        if c > self.cap:
+            raise ValueError('the jump lists hold %d entries, more than cap=%d' % (c, self.cap))
+        if ev_time.dtype != self._tt:
+            raise ValueError('ev_time must be %s like this object (time_dtype)' % self._tt)
+        self.node_state.copy_(node_state)
+        self.ev_count.copy_(ev_count)
+        self.ev_total.copy_(ev_total)
+        self.ev_time[:, self.cap - c:].copy_(ev_time)
+        self.ev_sb[:, self.cap - c:].copy_(ev_sb)
+        self.status.zero_()
+        if self.sweep_count is not None:
+            self.sweep_count.fill_(self.sweeps_done)
+        self.initialized = True
+
     _STATE = ('node_state', 'ev_count', 'ev_total', 'ev_time', 'ev_sb')
 
     def snapshot(self):
